@@ -4,7 +4,7 @@ executor on B200, with the roofline of the dominant kernel and the reference run
 cores in the same run.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c5|c3]
-                  [--streams S] [--frames T]
+                  [--streams S] [--frames T] [--dump-outputs DIR]
 
 Workload at N=1 (config.workload): BASELINE.json configs[1] -- "DAC8PRO-style 8-ch 3-way crossover,
 fixed-point int64 format, 192 kHz, 4096 independent streams batched on 1xB200" = program
@@ -29,6 +29,8 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: no __pycache__ written into it
+DUMP_BYTES = 64 * 10**6             # cap of --dump-outputs
 
 WORKLOADS = {
     # name: (program, DSP_FORMAT, fs, default streams, default frames, MACs/frame, description)
@@ -55,6 +57,22 @@ def workload_config(desc, prog, S, T, fs, n_in, n_out):
 
 def prog_file(name):
     return os.path.join(ROOT, "tests", "golden", "programs", name + ".bin")
+
+
+def dump_outputs(d, y, first):
+    """--dump-outputs: what the last timed step returned (int32 PCM [S, T, n_out] on the device) as float64, which holds every
+    int32 exactly.  Every stream when that fits DUMP_BYTES, else a fixed seeded sample of streams (and only the leading frames
+    when one stream alone is larger): outputs.npy [k, t, n_out] and outputs_streams.npy [k], the job's stream numbers."""
+    import numpy as np
+    import torch
+    S, T, n_out = y.shape
+    room = DUMP_BYTES - 1024                                  # two .npy headers
+    t = min(T, (room - 8) // (n_out * 8))
+    k = min(S, room // (t * n_out * 8 + 8))
+    idx = np.arange(S) if k == S else np.sort(np.random.default_rng(0).choice(S, k, replace=False))
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "outputs.npy"), y[torch.from_numpy(idx).to(y.device), :t].cpu().numpy().astype(np.float64))
+    np.save(os.path.join(d, "outputs_streams.npy"), (idx + first).astype(np.float64))
 
 
 def measured_peaks():
@@ -168,7 +186,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--kernel", default="auto", choices=["auto", "generic", "chain", "chain_v2", "chain_v3", "mix", "fir", "fir_tc", "dag"],
                     help="force a kernel (diagnostics; the default is what the product picks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one to DIR/*.npy (float64, at most 64 MB: a fixed "
+                         "sample of streams when larger; rank 0's streams when N > 1), to compare builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
@@ -246,6 +271,8 @@ def main():
     kernel_ms = sum(a.elapsed_time(b) for a, b in evs) / max(args.steps, 1)      # all launches of one step (1 for the chain kernel, 3 for the mix path)
     timed_kernel, timed_variant = ex.last_kernel, ex.last_chain_variant            # of the device-resident step (the e2e leg runs other sizes)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, y, first)
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

@@ -9,6 +9,8 @@
   vectors/*.npz     : input PCM + output PCM + final data area produced by the reference runtime itself
                       (oracle/_ref/libavdspruntime<fmt>_strict.so through oracle/refdriver.py), canonical
                       order (frame-major, cores ascending).
+  reference_digests.json : not written here; AVDSP_RECORD_REFERENCE_DIGESTS=1 python -m pytest
+                      tests/test_oracle_golden.py -k compiled_reference  rewrites it (see AgainstReference there).
 
 Nothing here runs on the GPU box: /root/reference does not exist there; the committed files do.
 Usage:  python tests/golden/make_golden.py         (from the repo root, after `make -C oracle`)

@@ -1,11 +1,70 @@
 """Pins the CPU oracle (oracle/avdsp_oracle.c) against the golden vectors produced by the real
-reference runtime (tests/golden/make_golden.py) and, when it was built here, against the compiled
-reference itself (oracle/_ref)."""
+reference runtime (tests/golden/make_golden.py), against the stored record of what the compiled
+reference returned on the runs below (tests/golden/reference_digests.json) and, when it was built
+here, against the compiled reference itself (oracle/_ref)."""
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 
-from conftest import CASES, load_program, load_vector, vector_names
+from conftest import CASES, GOLDEN, load_program, load_vector, vector_names
 from avdsp_b200 import synth
+from test_gpu_fuzz import nan_aware_equal
+
+REFERENCE_DIGESTS = os.path.join(GOLDEN, "reference_digests.json")
+# AVDSP_RECORD_REFERENCE_DIGESTS=1 rewrites the record from the oracle's results; run it where oracle/_ref is built, so that the
+# same run holds every recorded result against the compiled reference
+RECORD = os.environ.get("AVDSP_RECORD_REFERENCE_DIGESTS") == "1"
+
+
+def _digest(words, nan_aware):
+    """First 64 bits of the SHA-256 of int32 words; with nan_aware, every float NaN pattern is hashed as one (nan_aware_equal)"""
+    u = np.ascontiguousarray(words, dtype=np.int32).view(np.uint32)
+    if nan_aware:
+        u = np.where(((u & 0x7F800000) == 0x7F800000) & ((u & 0x007FFFFF) != 0), np.uint32(0x7FC00000), u)
+    return hashlib.sha256(u.tobytes()).hexdigest()[:16]
+
+
+class AgainstReference:
+    """The runs of one test, oracle against compiled reference.  Each run is held against the stored record of the reference's
+    return code, outputs and data area (digests: the full arrays of ~1000 runs would not fit the repository), and against the
+    compiled reference itself where oracle/_ref is built.  The record was taken from the oracle at a commit where every one of
+    these runs matched the compiled reference, NaN payloads aside."""
+
+    def __init__(self, oracle_lib, request):
+        from oracle import refdriver
+        self.oracle_lib, self.refdriver, self.key, self.got = oracle_lib, refdriver, request.node.name, []
+        with open(REFERENCE_DIGESTS) as f:
+            self.want = json.load(f).get(self.key)
+        assert RECORD or self.want is not None, f"{self.key}: no record in {REFERENCE_DIGESTS}"
+
+    def run(self, w, fmt, fs, x, seed, dither, nan_y, nan_data, tag):
+        o = self.oracle_lib.Oracle(w, fmt, fs, seed=seed, dither=dither)
+        assert o.rc > 0, tag
+        y = o.process(x)
+        if self.refdriver.available(fmt):
+            r = self.refdriver.RefProgram(w, fmt, fs, seed=seed, dither=dither)
+            assert r.rc == o.rc, tag
+            assert nan_aware_equal(r.process(x), y, nan_y), tag
+            assert nan_aware_equal(r.data, o.data, nan_data), tag
+        got = [int(o.rc), _digest(y, nan_y), _digest(o.data, nan_data)]
+        if not RECORD:
+            i = len(self.got)
+            assert i < len(self.want) and got == self.want[i], (tag, "[rc, outputs, data area] differ from the reference's record")
+        self.got.append(got)
+
+    def finish(self):
+        if RECORD:
+            with open(REFERENCE_DIGESTS) as f:
+                rec = json.load(f)
+            rec[self.key] = self.got
+            with open(REFERENCE_DIGESTS, "w") as f:
+                f.write("{\n" + ",\n".join(f"{json.dumps(k)}: [\n" + ",\n".join(json.dumps(g) for g in v) + "\n]"
+                                           for k, v in sorted(rec.items())) + "\n}\n")
+        else:
+            assert len(self.got) == len(self.want), self.key
 
 
 @pytest.mark.parametrize("name", vector_names())
@@ -29,24 +88,21 @@ def test_golden_inputs_are_the_documented_synthetic_pcm():
 
 
 @pytest.mark.parametrize("prog,fmt,fs", CASES)
-def test_oracle_matches_compiled_reference(oracle_lib, prog, fmt, fs):
-    from oracle import refdriver
-    if not refdriver.available(fmt):
-        pytest.skip("oracle/_ref not built here (it needs /root/reference)")
+def test_oracle_matches_compiled_reference(oracle_lib, request, prog, fmt, fs):
     if fmt == 2 and "fir" in prog and fs == 48000:
         # the one UNPINNED corner (DESIGN.md 2): the reference's fixed-point dsp_calc_fir_int (dsp_firSTD.h:8-35) is
         # provably not a convolution (SURVEY.md App. C #3); the oracle defines the intended semantics there instead.
         # test_fixed_point_fir_is_the_float_kernels_structure below ties it to the pinned float kernel.
         pytest.skip("fixed-point DSP_FIR: reference kernel is broken; oracle-defined semantics")
+    from oracle import wire
+    ref = AgainstReference(oracle_lib, request)
     w = load_program(prog)
+    ins, _ = wire.io_maps(w)
     gen = synth.pcm_float if fmt >= 5 else synth.pcm
     for kind, seed, dither in (("full", 9, 24), ("sine", 0, 31)):
-        o = oracle_lib.Oracle(w, fmt, fs, seed=seed, dither=dither)
-        x = gen(kind, 1, 700, len(o.ins), fs)[0]
-        r = refdriver.RefProgram(w, fmt, fs, seed=seed, dither=dither)
-        assert r.rc == o.rc > 0
-        assert np.array_equal(r.process(x), o.process(x))
-        assert np.array_equal(r.data, o.data)
+        x = gen(kind, 1, 700, len(ins), fs)[0]
+        ref.run(w, fmt, fs, x, seed, dither, False, False, kind)
+    ref.finish()
 
 
 def test_fixed_point_fir_is_the_float_kernels_structure(oracle_lib):
@@ -103,34 +159,29 @@ def test_oracle_chunking_is_invisible(oracle_lib):
     assert np.array_equal(a, b)
 
 
-def test_oracle_matches_compiled_reference_on_random_xy_programs(oracle_lib):
+def test_oracle_matches_compiled_reference_on_random_xy_programs(oracle_lib, request):
     """144 randomised X/Y-dataflow programs (the generator of tests/test_gpu_fuzz.py): the restatement against the compiled
-    reference, outputs and data area.  Needs oracle/_ref (built where /root/reference exists)."""
-    from oracle import refdriver, wire
-    if not refdriver.available(2):
-        pytest.skip("oracle/_ref not built here (it needs /root/reference)")
+    reference, outputs and data area."""
+    from oracle import wire
     from test_gpu_fuzz import random_program
+    ref = AgainstReference(oracle_lib, request)
     for seed in range(24):
         rng = np.random.default_rng(1000 + seed)
         for k in range(6):
             w = random_program(rng)
             ins, _ = wire.io_maps(w)
             x = synth.pcm("full" if k & 1 else "noise", 1, 150, len(ins), 48000)[0]
-            r = refdriver.RefProgram(w, 2, 48000, seed=seed, dither=24)
-            o = oracle_lib.Oracle(w, 2, 48000, seed=seed, dither=24)
-            assert r.rc == o.rc > 0
-            assert np.array_equal(r.process(x), o.process(x)), (seed, k)
-            assert np.array_equal(r.data, o.data), (seed, k)
+            ref.run(w, 2, 48000, x, seed, 24, False, False, (seed, k))
+    ref.finish()
 
 
 @pytest.mark.parametrize("fmt", [3, 4, 5, 6])
-def test_oracle_matches_compiled_reference_on_random_xy_programs_float_formats(oracle_lib, fmt):
+def test_oracle_matches_compiled_reference_on_random_xy_programs_float_formats(oracle_lib, request, fmt):
     """72 programs of the same generator per float format (5/6: float samples): outputs and data area bit for bit, two NaNs
     equal whatever their payload (see tests/test_gpu_fuzz.nan_aware_equal)."""
-    from oracle import refdriver, wire
-    if not refdriver.available(fmt):
-        pytest.skip("oracle/_ref not built here (it needs /root/reference)")
-    from test_gpu_fuzz import random_program, nan_aware_equal
+    from oracle import wire
+    from test_gpu_fuzz import random_program
+    ref = AgainstReference(oracle_lib, request)
     gen = synth.pcm_float if fmt >= 5 else synth.pcm
     for seed in range(12):
         rng = np.random.default_rng(2000 + seed)
@@ -138,21 +189,17 @@ def test_oracle_matches_compiled_reference_on_random_xy_programs_float_formats(o
             w = random_program(rng, 48000, fmt)
             ins, _ = wire.io_maps(w)
             x = gen("full" if k & 1 else "noise", 1, 150, len(ins), 48000)[0]
-            r = refdriver.RefProgram(w, fmt, 48000, seed=seed, dither=24)
-            o = oracle_lib.Oracle(w, fmt, 48000, seed=seed, dither=24)
-            assert r.rc == o.rc > 0
-            assert nan_aware_equal(r.process(x), o.process(x), fmt >= 5), (fmt, seed, k)
-            assert nan_aware_equal(r.data, o.data), (fmt, seed, k)
+            ref.run(w, fmt, 48000, x, seed, 24, fmt >= 5, True, (fmt, seed, k))
+    ref.finish()
 
 
 @pytest.mark.parametrize("fmt", [2, 3, 4, 5, 6])
-def test_oracle_matches_compiled_reference_on_random_misc_programs(oracle_lib, fmt):
+def test_oracle_matches_compiled_reference_on_random_misc_programs(oracle_lib, request, fmt):
     """60 programs per format of tests/test_gpu_fuzz.random_misc_program (immediates, register products and quotients, LOAD_MUX,
     LOAD_STORE, core-local TPDF, WHITE, DITHER, DITHER_NS2, DCBLOCK, CLIP, DIRAC / SQUAREWAVE, DELAY_1, fixed delays)."""
-    from oracle import refdriver, wire
-    if not refdriver.available(fmt):
-        pytest.skip("oracle/_ref not built here (it needs /root/reference)")
-    from test_gpu_fuzz import random_misc_program, nan_aware_equal
+    from oracle import wire
+    from test_gpu_fuzz import random_misc_program
+    ref = AgainstReference(oracle_lib, request)
     gen = synth.pcm_float if fmt >= 5 else synth.pcm
     for seed in range(10):
         rng = np.random.default_rng(3000 + seed)
@@ -160,28 +207,23 @@ def test_oracle_matches_compiled_reference_on_random_misc_programs(oracle_lib, f
             w = random_misc_program(rng, 48000, fmt)
             ins, _ = wire.io_maps(w)
             x = gen("full" if k & 1 else "noise", 1, 150, max(len(ins), 1), 48000)[0][:, : len(ins)]
-            r = refdriver.RefProgram(w, fmt, 48000, seed=seed, dither=24)
-            o = oracle_lib.Oracle(w, fmt, 48000, seed=seed, dither=24)
-            assert r.rc == o.rc > 0
-            assert nan_aware_equal(r.process(x), o.process(x), fmt >= 5), (fmt, seed, k)
-            assert nan_aware_equal(r.data, o.data, fmt != 2), (fmt, seed, k)
+            ref.run(w, fmt, 48000, x, seed, 24, fmt >= 5, fmt != 2, (fmt, seed, k))
+    ref.finish()
 
 
 @pytest.mark.parametrize("family,fmt", [("chain", 2), ("chain", 3), ("chain", 5), ("mix", 2), ("mix", 3), ("fir", 3)])
-def test_oracle_matches_compiled_reference_on_random_kernel_shaped_programs(oracle_lib, family, fmt):
+def test_oracle_matches_compiled_reference_on_random_kernel_shaped_programs(oracle_lib, request, family, fmt):
     """The generators of tests/test_gpu_fuzz_chain.py / test_gpu_fuzz_mix.py (the programs the fused kernels are fuzzed with): the
     restatement against the compiled reference.  Unstable cascades only in fixed point (wrapping accumulators are defined); in the
     float formats a cascade that has blown up adds NaNs to NaNs, and which operand's sign and payload an x86 addss keeps is the
     reference COMPILER's choice of operand order -- visible as +-full scale after the saturation -- so there is no behaviour to pin
     there (the oracle and the GPU take the accumulator as first operand).  Fixed-point FIR is left out as well: the reference's
     own kernel is broken there, SURVEY App. C #4-5, and the oracle defines the intended convolution."""
-    from oracle import refdriver, wire
-    if not refdriver.available(fmt):
-        pytest.skip("oracle/_ref not built here (it needs /root/reference)")
+    from oracle import wire
     import importlib
-    from test_gpu_fuzz import nan_aware_equal
     chain = importlib.import_module("test_gpu_fuzz_chain")
     mix = importlib.import_module("test_gpu_fuzz_mix")
+    ref = AgainstReference(oracle_lib, request)
     gen = synth.pcm_float if fmt >= 5 else synth.pcm
     for seed in range(10):
         rng = np.random.default_rng(13000 + seed)
@@ -195,8 +237,5 @@ def test_oracle_matches_compiled_reference_on_random_kernel_shaped_programs(orac
             ins, _ = wire.io_maps(w)
             T = 1500 if family == "fir" else 400
             x = gen(("full", "noise", "impulse")[k % 3], 1, T, max(len(ins), 1), 48000)[0][:, : len(ins)]
-            r = refdriver.RefProgram(w, fmt, 48000, seed=seed, dither=24)
-            o = oracle_lib.Oracle(w, fmt, 48000, seed=seed, dither=24)
-            assert r.rc == o.rc > 0
-            assert nan_aware_equal(r.process(x), o.process(x), fmt >= 5), (family, fmt, seed, k)
-            assert nan_aware_equal(r.data, o.data, fmt != 2), (family, fmt, seed, k)
+            ref.run(w, fmt, 48000, x, seed, 24, fmt >= 5, fmt != 2, (family, fmt, seed, k))
+    ref.finish()
