@@ -129,6 +129,23 @@ __global__ void k_widen_pcm(const unsigned char* __restrict__ src, int fmt, int*
     dst[i] = v;
 }
 
+// Rows of the coefficient table, [n][nCoef] (row s = stream first + s, avdsp_b200_set_coefs), into the table, [nCoef][pitch]:
+// a transpose through 32 x 32 tiles so that both the row reads and the column writes coalesce.  block (32, 8), grid (stream
+// tiles, column tiles).
+__global__ void __launch_bounds__(256) k_coef_scatter(int* __restrict__ tab, int pitch, int first, int n, int nCoef, const int* __restrict__ rows) {
+    __shared__ int t[32][33];
+    const int s0 = blockIdx.x * 32, c0 = blockIdx.y * 32;
+    for (int j = threadIdx.y; j < 32; j += 8) {
+        const int s = s0 + j, c = c0 + threadIdx.x;
+        if (s < n && c < nCoef) t[j][threadIdx.x] = rows[(size_t)s * nCoef + c];
+    }
+    __syncthreads();
+    for (int j = threadIdx.y; j < 32; j += 8) {
+        const int c = c0 + j, s = s0 + threadIdx.x;
+        if (s < n && c < nCoef) tab[(size_t)c * pitch + first + s] = t[threadIdx.x][j];
+    }
+}
+
 #include "instance.h"
 
 static int quiesce(avdsp_b200* h);
@@ -269,6 +286,8 @@ static void freeAll(avdsp_b200* h) {
     if (h->dRedoCount) cudaFree(h->dRedoCount);
     if (h->dFirTaps) cudaFree(h->dFirTaps);
     if (h->dFirWs) cudaFree(h->dFirWs);
+    if (h->dCoef) cudaFree(h->dCoef);
+    if (h->dCoefStage) cudaFree(h->dCoefStage);
     if (h->pcmRaw) cudaFree(h->pcmRaw);
     if (h->pcmIn) cudaFree(h->pcmIn);
     if (h->pcmOut) cudaFree(h->pcmOut);
@@ -434,6 +453,7 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         outSS = (long long)cap * nOut; outFS = 1; outCS = cap;
     } else return setErr(AVDSP_B200_ERR_ARG, "unknown layout");
     int* st = h->dState + (size_t)first * P.stateWords;
+    const int* coefs = h->dCoef ? h->dCoef + first : nullptr;     // per-stream coefficient table, positioned like the state blocks
     if (ordered) CU(cudaStreamWaitEvent(stream, h->evLast, 0));          // stream-ordered after the instance's previous launch (see evLast)
     // the fused kernels run the canonical order; a plugin-order request may use them when the two orders provably agree
     const bool chainOrder = (h->period == 0 || pl->L.orderIndependent) && coreSel < 0 && !planOverride;
@@ -520,6 +540,7 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         A.nStreams = n; A.nFrames = nFrames;
         A.inStreamStride = inSS; A.outStreamStride = outSS;
         A.inFrameStride = inFS; A.inChStride = inCS; A.outFrameStride = outFS; A.outChStride = outCS;
+        A.coefs = coefs; A.coefPitch = h->nStreams;
         e = launchDag(*pl->L.dag, pl->geomDag, A, stream);
         h->lastKernel = AVDSP_B200_KERNEL_DAG;
     } else if (use == AVDSP_B200_KERNEL_CHAIN) {
@@ -528,6 +549,7 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         A.nStreams = n; A.nFrames = nFrames;
         A.inStreamStride = inSS; A.outStreamStride = outSS;
         A.inFrameStride = inFS; A.inChStride = inCS; A.outFrameStride = outFS; A.outChStride = outCS;
+        A.coefs = coefs; A.coefPitch = h->nStreams;
         // v3 (a cascade part per lane, lane = stream) wants full warps and several equal warps per sub-partition: AUTO takes it at
         // batch width (>= 16 streams per SM) when the cascades could be cut into parts of <= 4 sections (measured on C2: 9.06 ms
         // against v2's 9.50; with whole 6- and 8-section cascades per warp v3 is the slower one) and the call is long enough to
@@ -579,6 +601,7 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         A.inStreamStride = inSS; A.outStreamStride = outSS;
         A.inFrameStride = inFS; A.inChStride = inCS; A.outFrameStride = outFS; A.outChStride = outCS;
         A.coreSel = coreSel; A.period = coreSel >= 0 ? 0 : h->period;
+        A.coefs = planOverride ? nullptr : coefs; A.coefPitch = h->nStreams; A.coefStep = 5 * pl->L.nFreq;
         for (int c = 0; c < P.nCores && c < kMaxCores; c++) { A.coreInMask[c] = pl->L.cores[c].usedIn; A.coreOutMask[c] = pl->L.cores[c].usedOut; }
         e = launchGeneric(G, A, stream);
         h->lastKernel = AVDSP_B200_KERNEL_GENERIC;
@@ -1007,22 +1030,51 @@ int avdsp_b200_set_param(avdsp_b200_t* h, int firstStream, int nStreams, int wor
         return 0;
     }
     { const int q = quiesce(h); if (q < 0) return q; }
-    if (h->variantOf.empty()) h->variantOf.assign(h->nStreams, 0);
+    // while the instance has a coefficient table, coefficient words are written into the streams' rows; the other words make
+    // variants as without one.  Everything that can fail (lowering a variant) happens before anything changes.
+    const std::vector<int32_t>& cw = h->L.coefWords;
+    std::vector<int> colOf(nWords, -1);                  // table column of word k of the call, or -1
+    if (h->dCoef)
+        for (int k = 0; k < nWords; k++) {
+            const auto it = std::lower_bound(cw.begin(), cw.end(), wordIndex + k);
+            if (it != cw.end() && *it == wordIndex + k) colOf[k] = (int)(it - cw.begin());
+        }
+    const bool anyVariantWord = std::find(colOf.begin(), colOf.end(), -1) != colOf.end();
     // streams of the range may sit on different variants already: patch each of those once
     std::map<int, int> moved;                 // old variant -> new variant
-    for (int s = firstStream; s < firstStream + nStreams; s++) {
-        const int old = h->variantOf[s];
-        auto it = moved.find(old);
-        if (it == moved.end()) {
+    if (anyVariantWord) {
+        const size_t nBefore = h->variants.size();
+        auto undo = [&](int rc) {             // release the variants this call created; nothing else has changed yet
+            while (h->variants.size() > nBefore) { freeAll(h->variants.back()); h->variants.pop_back(); }
+            return rc;
+        };
+        for (int s = firstStream; s < firstStream + nStreams; s++) {
+            const int old = h->variantOf.empty() ? 0 : h->variantOf[s];
+            if (moved.count(old)) continue;
             std::vector<int32_t> words = old ? h->variants[old - 1]->L.words : h->L.words;
-            for (int k = 0; k < nWords; k++) words[wordIndex + k] = values[k];
+            for (int k = 0; k < nWords; k++) if (colOf[k] < 0) words[wordIndex + k] = values[k];
             int id = 0;
             const int r = variantFor(h, words, &id);
-            if (r < 0) return r;
-            it = moved.emplace(old, id).first;
+            if (r < 0) return undo(r);
+            if (h->dCoef && id > 0 && h->variants[id - 1]->L.coefWords != cw)
+                return undo(setErr(AVDSP_B200_ERR_UNSUPPORTED, "this change moves biquad coefficient words the coefficient table holds (section count)"));
+            moved.emplace(old, id);
         }
-        h->variantOf[s] = it->second;
     }
+    if (h->dCoef) {
+        std::vector<int32_t> col((size_t)nStreams);
+        for (int k = 0; k < nWords; k++) {
+            if (colOf[k] < 0) continue;
+            std::fill(col.begin(), col.end(), values[k]);
+            CU(cudaMemcpyAsync(h->dCoef + (size_t)colOf[k] * h->nStreams + firstStream, col.data(), col.size() * 4,
+                               cudaMemcpyHostToDevice, h->stream));
+            CU(cudaStreamSynchronize(h->stream));
+        }
+        CU(cudaEventRecord(h->evLast, h->stream));
+    }
+    if (!anyVariantWord) return 0;
+    if (h->variantOf.empty()) h->variantOf.assign(h->nStreams, 0);
+    for (int s = firstStream; s < firstStream + nStreams; s++) h->variantOf[s] = moved.at(h->variantOf[s]);
     // variants nobody runs any more are released (ids above shift down)
     std::vector<int> used(h->variants.size() + 1, 0);
     for (int v : h->variantOf) used[v] = 1;
@@ -1036,6 +1088,87 @@ int avdsp_b200_set_param(avdsp_b200_t* h, int firstStream, int nStreams, int wor
     bool any = false;
     for (int& v : h->variantOf) { v = remap[v]; any = any || v != 0; }
     if (!any) h->variantOf.clear();
+    return 0;
+}
+
+int avdsp_b200_coef_words(const int32_t* prog, int progWords, int format, int32_t* wordIndex, int maxOut) {
+    if (maxOut < 0 || (maxOut > 0 && !wordIndex)) return setErr(AVDSP_B200_ERR_ARG, "bad output buffer");
+    // the column list does not depend on the rate: lower at the lowest one the header admits (decodeProgram validates it)
+    const int fi = (prog && progWords > H_FREQMIN) ? prog[H_FREQMIN] : 0;
+    const int fs = (fi >= 0 && fi < kNumFreq) ? kFreqTable[fi] : 0;
+    std::unique_ptr<Lowered> L(new Lowered);
+    std::string err;
+    const int rc = decodeProgram(prog, progWords, 0x7FFFFFFF, format, fs, 31, L.get(), &err);
+    if (rc < 0) return setErr(rc, err);
+    const int n = (int)L->coefWords.size();
+    for (int k = 0; k < n && k < maxOut; k++) wordIndex[k] = L->coefWords[k];
+    return n;
+}
+
+// The instance's coefficient table, created on first use: every stream's row holds the words it runs with now (the program's, or
+// its variant's).  Synchronous: the table is not in use yet.
+static int ensureCoefTable(avdsp_b200* h) {
+    if (h->dCoef) return 0;
+    const std::vector<int32_t>& cw = h->L.coefWords;
+    const size_t N = (size_t)h->nStreams, nc = cw.size();
+    std::vector<int32_t> init(nc * N);
+    for (size_t s = 0; s < N; s++) {
+        const int v = h->variantOf.empty() ? 0 : h->variantOf[s];
+        const std::vector<int32_t>& w = v ? h->variants[v - 1]->L.words : h->L.words;
+        for (size_t c = 0; c < nc; c++) init[c * N + s] = w[cw[c]];
+    }
+    int* d = nullptr;
+    CU(cudaMalloc(&d, init.size() * 4));
+    const cudaError_t e = cudaMemcpyAsync(d, init.data(), init.size() * 4, cudaMemcpyHostToDevice, h->stream);
+    const cudaError_t e2 = e == cudaSuccess ? cudaStreamSynchronize(h->stream) : e;
+    if (e2 != cudaSuccess) { cudaFree(d); return cudaErr(e2, "coefficient table upload"); }
+    h->dCoef = d;
+    return 0;
+}
+
+int avdsp_b200_set_coefs(avdsp_b200_t* h, int firstStream, int nStreams, const int32_t* values, int memspace, void* cudaStream) {
+    if (!h || !values) return setErr(AVDSP_B200_ERR_ARG, "NULL argument");
+    if (firstStream < 0 || nStreams < 0 || (long long)firstStream + nStreams > h->nStreams) return setErr(AVDSP_B200_ERR_ARG, "bad stream range");
+    if (memspace != AVDSP_B200_HOST && memspace != AVDSP_B200_DEVICE) return setErr(AVDSP_B200_ERR_ARG, "unknown memspace");
+    const int nCoef = (int)h->L.coefWords.size();
+    if (nCoef == 0) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "the program has no biquad coefficients");
+    if (!h->L.coefTableOk) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "biquad parameter blocks of this program overlap: no coefficient table");
+    if (!h->shards.empty()) {
+        if (memspace != AVDSP_B200_HOST) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a multi-device instance takes HOST coefficient rows (device buffers belong to one GPU)");
+        for (const avdsp_b200* sh : h->shards)
+            for (const avdsp_b200* v : sh->variants)
+                if (v->L.coefWords != h->L.coefWords) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a parameter variant moved the biquad coefficient words (section count)");
+        return forShards(h, [&](int k, avdsp_b200* sh) {
+            const int a = std::max(firstStream, h->shardFirst[k]), b = std::min(firstStream + nStreams, h->shardFirst[k + 1]);
+            if (b <= a) return 0;
+            return avdsp_b200_set_coefs(sh, a - h->shardFirst[k], b - a, values + (size_t)(a - firstStream) * nCoef, AVDSP_B200_HOST, nullptr);
+        });
+    }
+    for (const avdsp_b200* v : h->variants)
+        if (v->L.coefWords != h->L.coefWords) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a parameter variant moved the biquad coefficient words (section count)");
+    if (nStreams == 0) return 0;
+    CU(cudaSetDevice(h->device));
+    { const int r = ensureCoefTable(h); if (r < 0) return r; }
+    const cudaStream_t s = memspace == AVDSP_B200_DEVICE ? (cudaStream_t)cudaStream : h->stream;
+    const size_t words = (size_t)nStreams * nCoef;
+    CU(cudaStreamWaitEvent(s, h->evLast, 0));                 // after every launch enqueued on the instance before this call
+    const int* rows = values;
+    if (memspace == AVDSP_B200_HOST) {
+        if (words > h->coefStageWords) {
+            CU(cudaStreamSynchronize(s));
+            if (h->dCoefStage) cudaFree(h->dCoefStage);
+            h->dCoefStage = nullptr; h->coefStageWords = 0;
+            CU(cudaMalloc(&h->dCoefStage, words * 4));
+            h->coefStageWords = words;
+        }
+        CU(cudaMemcpyAsync(h->dCoefStage, values, words * 4, cudaMemcpyHostToDevice, s));
+        rows = h->dCoefStage;
+    }
+    k_coef_scatter<<<dim3((unsigned)((nStreams + 31) / 32), (unsigned)((nCoef + 31) / 32)), dim3(32, 8), 0, s>>>(h->dCoef, h->nStreams, firstStream, nStreams, nCoef, rows);
+    CU(cudaGetLastError());
+    h->launches++;
+    CU(cudaEventRecord(h->evLast, s));
+    if (memspace == AVDSP_B200_HOST) CU(cudaStreamSynchronize(s));    // the caller's buffer (and the staging rows) are free again
     return 0;
 }
 
@@ -1057,6 +1190,7 @@ int avdsp_b200_reload_params(avdsp_b200_t* h, const int32_t* prog, int progWords
     }
     { const int q = quiesce(h); if (q < 0) return q; }
     dropVariants(h);                                          // a new program for everybody: per-stream overrides start over
+    if (h->dCoef) { cudaFree(h->dCoef); h->dCoef = nullptr; }   // ... the coefficient table too
     const int r = uploadPlanData(h);
     return r < 0 ? r : rc;
 }

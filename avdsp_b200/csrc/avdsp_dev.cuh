@@ -191,6 +191,29 @@ __device__ __forceinline__ void fltGuard(FltGuard& g, float v) {
     if (HUGE) g.mx = max(g.mx, b + b);
 }
 __device__ __forceinline__ bool fltGuardFired(const FltGuard& g) { return g.mn < kFltGuardTiny || g.mx >= kFltGuardHuge; }
+// A coefficient from the per-stream table is not checked on the host: one outside [2^-60, 2^7) (non-zero; what
+// chainFloatCoefsInRange admits) fires the lane's guard (mn = 0), so the stream is re-executed exactly like one that met a
+// tiny value.
+__device__ __forceinline__ bool fltCoefOutOfRange(int bits) {
+    const unsigned u = (unsigned)bits & 0x7FFFFFFFu, ex = u >> 23;
+    return u != 0u && (ex < 127u - 60u || ex > 127u + 6u);
+}
+
+// ---- per-stream coefficient table (avdsp_b200_set_coefs) ----------------------------------------------------------------
+// The five words b0 b1 b2 a1 a2 of one section: from the table ([column][stream], `col` = the section's b0 column, `pos` = the
+// stream's position in the call) when there is one, else from the plan.  Loaded once per launch, before the frame loop.
+// Two load paths on purpose: without a table the words stay constant-bank operands of the plan, as they were before tables
+// existed (one pointer for both would turn them into generic loads from parameter space).
+__device__ __forceinline__ void sectionCoefs(const int* planCf, const int* tab, int pitch, int col, int pos, int c[5]) {
+    if (tab) {
+        const int* t = tab + (size_t)col * pitch + pos;
+#pragma unroll
+        for (int q = 0; q < 5; q++) c[q] = __ldg(t + (size_t)q * pitch);
+    } else {
+#pragma unroll
+        for (int q = 0; q < 5; q++) c[q] = planCf[q];
+    }
+}
 
 // dspMulFloatDouble (:377-410): exact float x float product as a double (zero/denormal inputs -> +0)
 __device__ __forceinline__ double mulFD(float a, float b) {

@@ -26,6 +26,7 @@ struct Ctx {
     uint32_t delayFactor;
     int nMemSlots = 0;
     std::map<int, int> memSlotOfWord;
+    std::vector<std::pair<int, int>> biquadBlocks;      // (parameter block word, sections) of every DSP_BIQUADS, bypassed too
 
     [[noreturn]] void fail(int code, const char* fmt, int a = 0, int b = 0) {
         char buf[256]; snprintf(buf, sizeof buf, fmt, a, b);
@@ -142,13 +143,14 @@ void lowerCore(Ctx& cx, int begin) {
         case OP_BIQUADS: {                                  // :827-849
             int off = arg(0), h = p + arg(1);
             int num = (int16_t)(cx.code(h, p) & 0xFFFF);
+            if (num > 0) cx.biquadBlocks.emplace_back(h, num);
             if (cx.code(h + 1, p) == 0 || num <= 0) break;  // bypass flag: X untouched
             cx.checkData(off, 6 * num, p);
             int stride = 2 + 6 * L->nFreq, c0 = h + 5 + 6 * L->fsRel;
             int first = L->gen.h.nPool;
             for (int s = 0; s < num; s++)
                 for (int k = 0; k < 5; k++) cx.pool(cx.code(c0 + s * stride + k, p));
-            cx.emit(op, num, off, first, 0); break; }
+            cx.emit(op, num, off, first, h); break; }     // c: the block's word until lowerAll makes it a table column
         case OP_FIR: {                                      // :928-969
             int rel = arg(L->fsRel);
             if (rel == 0) break;
@@ -261,7 +263,7 @@ void buildChainPlan(Lowered* L) {
         c.h.chainOfOut[ch] = c.h.nChains;
         d.storeCh[d.nStores++] = (uint8_t)ch;
     };
-    struct MemProducer { int srcKind, srcCh, srcArg, consumers; std::vector<int> secOff; std::vector<int32_t> coefs; };
+    struct MemProducer { int srcKind, srcCh, srcArg, consumers; std::vector<int> secOff; std::vector<int32_t> coefs; std::vector<int> cols; };
     std::vector<std::pair<int, MemProducer>> producers;          // keyed by the MEM word's state offset
     auto findProducer = [&](int memOff) -> MemProducer* { for (auto& pr : producers) if (pr.first == memOff) return &pr.second; return nullptr; };
     for (int core = 0; core < g.h.nCores; core++) {
@@ -305,7 +307,7 @@ void buildChainPlan(Lowered* L) {
                 d.srcArg = c.h.nPool;
                 for (int k = 0; k < s.n; k++) { chainPool(c, inputCh(g.pool[s.a + 2 * k])); chainPool(c, g.pool[s.a + 2 * k + 1]); }
             }
-            std::vector<int> secOff;
+            std::vector<int> secOff, cols;
             std::vector<int32_t> coefs;
             if (s.op == OP_LOAD_MEM) {
                 // a cascade continued from an earlier core through a MEM word: inline the producer (same frame, canonical order:
@@ -313,13 +315,14 @@ void buildChainPlan(Lowered* L) {
                 MemProducer* pr = findProducer(s.a);
                 if (!pr) throw ChainFail{"LOAD_MEM of a word no earlier cascade of the frame stored"};
                 d.srcKind = (uint8_t)pr->srcKind; d.srcCh = (int16_t)pr->srcCh; d.srcArg = pr->srcArg;
-                secOff = pr->secOff; coefs = pr->coefs; pr->consumers++;
+                secOff = pr->secOff; coefs = pr->coefs; cols = pr->cols; pr->consumers++;
             } else if (s.op != OP_LOAD && s.op != OP_LOAD_GAIN && s.op != OP_LOAD_MUX)
                 throw ChainFail{"a signal path does not start with LOAD / LOAD_GAIN / LOAD_MUX"};
             i++;
             while (i < e && g.ops[i].op == OP_BIQUADS) {
                 for (int k = 0; k < g.ops[i].n; k++) {
                     secOff.push_back(g.ops[i].a + 6 * k);
+                    cols.push_back(g.ops[i].c + 5 * L->nFreq * k);
                     for (int q = 0; q < 5; q++) coefs.push_back(g.pool[g.ops[i].b + 5 * k + q]);
                 }
                 i++;
@@ -328,7 +331,7 @@ void buildChainPlan(Lowered* L) {
                 // producer half of such a cascade: no output of its own
                 if (g.h.aluClass != ALU_INT64 || secOff.empty() || d.srcKind == SRC_LOAD_MUX || findProducer(g.ops[i].a) || (int)producers.size() >= kMaxMemCopy)
                     throw ChainFail{"STORE_MEM the chain kernels cannot inline"};
-                MemProducer pr{d.srcKind, d.srcCh, d.srcArg, 0, secOff, coefs};
+                MemProducer pr{d.srcKind, d.srcCh, d.srcArg, 0, secOff, coefs, cols};
                 producers.emplace_back(g.ops[i].a, pr);
                 i++;
                 continue;
@@ -337,6 +340,8 @@ void buildChainPlan(Lowered* L) {
             for (int32_t v : coefs) chainPool(c, v);
             d.secStateOff = c.h.nPool;
             for (int v : secOff) chainPool(c, v);
+            d.coefColOff = c.h.nPool;
+            for (int v : cols) chainPool(c, v);
             d.nsec = (int16_t)secOff.size();
             if (i < e && g.ops[i].op == OP_GAIN) { d.hasGain = 1; d.gainBits = g.ops[i].a; i++; }
             if (i + 1 < e && g.ops[i].op == OP_DELAY && !d.hasGain && d.nsec > 0 && g.h.aluClass == ALU_INT64 &&
@@ -598,12 +603,19 @@ void buildDagPlan(Lowered* L) {
                     DagNode& n = d.nodes[id];
                     const int take = std::min(m.n - first, 8 - n.nsec);
                     // coefficients and state offsets of a node are contiguous in the pool: re-pack when sections are appended
-                    std::vector<int32_t> coefs, offs;
-                    for (int k = 0; k < n.nsec; k++) { for (int q = 0; q < 5; q++) coefs.push_back(d.pool[n.coefOff + 5 * k + q]); offs.push_back(d.pool[n.secStateOff + k]); }
-                    for (int k = first; k < first + take; k++) { for (int q = 0; q < 5; q++) coefs.push_back(g.pool[m.b + 5 * k + q]); offs.push_back(m.a + 6 * k); }
+                    std::vector<int32_t> coefs, offs, cols;
+                    for (int k = 0; k < n.nsec; k++) {
+                        for (int q = 0; q < 5; q++) coefs.push_back(d.pool[n.coefOff + 5 * k + q]);
+                        offs.push_back(d.pool[n.secStateOff + k]); cols.push_back(d.pool[n.coefColOff + k]);
+                    }
+                    for (int k = first; k < first + take; k++) {
+                        for (int q = 0; q < 5; q++) coefs.push_back(g.pool[m.b + 5 * k + q]);
+                        offs.push_back(m.a + 6 * k); cols.push_back(m.c + 5 * L->nFreq * k);
+                    }
                     n.nsec = (int)offs.size();
                     n.coefOff = d.nPool; for (int32_t v : coefs) dagPool(d, v);
                     n.secStateOff = d.nPool; for (int32_t v : offs) dagPool(d, v);
+                    n.coefColOff = d.nPool; for (int32_t v : cols) dagPool(d, v);
                     d.maxSec = std::max(d.maxSec, n.nsec);
                     X = exprOfNode(id);
                     first += take;
@@ -774,6 +786,41 @@ void analyseOrder(Lowered* L) {
         }
 }
 
+// The coefficient-table columns (Lowered::coefWords) and the column of every lowered BIQUADS micro-op.  Section s, fs column f,
+// coefficient q of the block at word h is word h + 5 + 6f + s * (2 + 6 * nFreq) + q (dsp_runtime.c:827-849), so within a block
+// the columns of a section's fs column are consecutive and sections step by 5 * nFreq.
+void buildCoefColumns(Ctx& cx) {
+    Lowered* L = cx.L;
+    const int stride = 2 + 6 * L->nFreq;
+    std::vector<int32_t> cw;
+    for (const auto& b : cx.biquadBlocks)
+        for (int s = 0; s < b.second; s++)
+            for (int f = 0; f < L->nFreq; f++)
+                for (int q = 0; q < 5; q++) {
+                    const int64_t w = (int64_t)b.first + 5 + 6 * f + (int64_t)s * stride + q;
+                    if (w >= 0 && w < cx.total) cw.push_back((int32_t)w);
+                }
+    std::sort(cw.begin(), cw.end());
+    cw.erase(std::unique(cw.begin(), cw.end()), cw.end());
+    L->coefWords = cw;
+    auto colOf = [&](int64_t w) -> int64_t {
+        auto it = std::lower_bound(cw.begin(), cw.end(), (int32_t)std::min<int64_t>(w, INT32_MAX));
+        return (it != cw.end() && *it == w) ? (int64_t)(it - cw.begin()) : -1;
+    };
+    L->coefTableOk = true;
+    GenericPlan& g = L->gen;
+    for (int i = 0; i < g.h.nOps; i++) {
+        MicroOp& m = g.ops[i];
+        if (m.op != OP_BIQUADS) continue;
+        const int64_t c0 = (int64_t)m.c + 5 + 6 * L->fsRel;
+        const int64_t col0 = colOf(c0);
+        for (int s = 0; s < m.n; s++)
+            for (int q = 0; q < 5; q++)
+                if (col0 < 0 || colOf(c0 + (int64_t)s * stride + q) != col0 + 5 * L->nFreq * s + q) L->coefTableOk = false;
+        m.c = col0 < 0 ? 0 : (int32_t)col0;
+    }
+}
+
 void lowerAll(Lowered* L) {
     Ctx cx; cx.L = L; cx.w = L->words.data(); cx.total = L->totalLength;
     cx.delayFactor = (uint32_t)(4294.967296 * (double)L->fs);      // dsp_runtime.c:81-90
@@ -782,7 +829,7 @@ void lowerAll(Lowered* L) {
     L->memWord.clear();
     for (size_t k = 0; k < keepMem.size(); k++) cx.memSlot(keepMem[k], 0);
     g.h.nOps = 0; g.h.nPool = 0;
-    L->bigPool.clear(); L->firs.clear();
+    L->bigPool.clear(); L->firs.clear(); cx.biquadBlocks.clear();
 
     g.h.nCores = (int)L->cores.size();
     uint32_t usedIn = 0, usedOut = 0;
@@ -805,6 +852,7 @@ void lowerAll(Lowered* L) {
     g.h.stateWords = (g.h.memOff + 2 * g.h.nMem + 3) & ~3;
     for (int i = 0; i < g.h.nOps; i++)
         if (g.ops[i].op == OP_LOAD_MEM || g.ops[i].op == OP_STORE_MEM) g.ops[i].a = g.h.memOff + 2 * g.ops[i].a;
+    buildCoefColumns(cx);
 
     analyseOrder(L);
     try { buildChainPlan(L); L->chainOk = true; L->chainWhyNot.clear(); }

@@ -42,6 +42,11 @@ struct Lowered {
     std::string orderWhy;
     // MEM words (LOAD_MEM / STORE_MEM targets inside the code area)
     std::vector<int> memWord;            // code word index of each slot
+    // biquad coefficient words: b0 b1 b2 a1 a2 of every section of every DSP_BIQUADS parameter block, for every fs column,
+    // bypassed blocks included, ascending.  The columns of the per-stream coefficient table (avdsp_b200_set_coefs); a lowered
+    // BIQUADS micro-op's `c` is the column of its first section's b0 at the current fs, section k at c + 5 * nFreq * k.
+    std::vector<int32_t> coefWords;
+    bool coefTableOk = true;             // every lowered section follows that column pattern (blocks that overlap do not)
     // human readable trace of the lowering (replaces the reference's DSP_PRINTF=2 opcode trace)
     std::string trace;
 };

@@ -65,6 +65,10 @@ struct avdsp_b200 {
     cudaStream_t varStream[kVarStreams] = {};
     cudaEvent_t varEv[kVarStreams] = {};
     cudaEvent_t evFork = nullptr;
+    // per-stream coefficient table (avdsp_b200_set_coefs): [column][stream] int32, column = index into L.coefWords; nullptr: none.
+    // Variants (set_param on other words) keep their own plans and read the same table.
+    int* dCoef = nullptr;
+    int* dCoefStage = nullptr; size_t coefStageWords = 0;     // HOST rows on their way to the table
     int numaNode = -1;                 // host NUMA node next to `device` (-1: unknown)
     std::map<void*, size_t> hostAllocs;   // avdsp_b200_host_alloc: pointer -> bytes
 };

@@ -370,6 +370,7 @@ k_chain2(const __grid_constant__ ChainPlan P, const Chain2Args A, const __grid_c
         int* post_s = reinterpret_cast<int*>(smem_raw + G.postOff);
         Lane2F<K> L;
         FltGuard mn;                       // exactness guard (avdsp_dev.cuh): smallest guard word of every value seen
+        bool coefBad = false;              // a table coefficient outside what the guard can bound (fltCoefOutOfRange)
         const ChainLane e = A.lanes[tid];
         const bool live = e.slot >= 0 && e.slot / C < nsHere;
         const bool head = (e.flags & 1) != 0, tail = (e.flags & 2) != 0;
@@ -387,7 +388,10 @@ k_chain2(const __grid_constant__ ChainPlan P, const Chain2Args A, const __grid_c
 #pragma unroll
             for (int k = 0; k < K; k++) {
                 const int sec = g0 + k;
-                const int* cf = P.pool + d.coefOff + 5 * sec;
+                int cf[5];
+                const bool tab = A.coefs && sec < d.nsec;
+                sectionCoefs(P.pool + d.coefOff + 5 * sec, tab ? A.coefs : nullptr, A.coefPitch, tab ? P.pool[d.coefColOff + sec] : 0, SX(slot / C), cf);
+                if (tab) for (int q = 0; q < 5; q++) coefBad |= fltCoefOutOfRange(cf[q]);
                 L.b0[k] = __int_as_float(cf[0]); L.b1[k] = __int_as_float(cf[1]); L.b2[k] = __int_as_float(cf[2]);
                 L.a1[k] = __int_as_float(cf[3]); L.a2[k] = __int_as_float(cf[4]);
                 const int* q = stLane + P.pool[d.secStateOff + sec];        // [acc, -, x1, x2, y1, y2] (dsp_biquadSTD.h:84-119)
@@ -395,6 +399,7 @@ k_chain2(const __grid_constant__ ChainPlan P, const Chain2Args A, const __grid_c
                 L.x1[k] = __int_as_float(q[2]); L.x2[k] = __int_as_float(q[3]); L.y1[k] = __int_as_float(q[4]); L.y2[k] = __int_as_float(q[5]);
                 fltGuard(mn, L.acc[k]); fltGuard(mn, L.x1[k]); fltGuard(mn, L.x2[k]); fltGuard(mn, L.y1[k]); fltGuard(mn, L.y2[k]);
             }
+            if (coefBad) mn.mn = 0u;
         }
         const int* xrow = x_s + (size_t)((slot / C) * nSrc + max(d.srcId, 0)) * XP;
         int* prow = post_s + (size_t)slot * G.postPitch;
@@ -485,7 +490,9 @@ k_chain2(const __grid_constant__ ChainPlan P, const Chain2Args A, const __grid_c
 #pragma unroll
             for (int k = 0; k < K; k++) {
                 const int sec = g0 + k;
-                const int* cf = P.pool + d.coefOff + 5 * sec;
+                int cf[5];
+                const bool tab = A.coefs && sec < d.nsec;
+                sectionCoefs(P.pool + d.coefOff + 5 * sec, tab ? A.coefs : nullptr, A.coefPitch, tab ? P.pool[d.coefColOff + sec] : 0, SX(slot / C), cf);
                 L.b0[k] = cf[0]; L.b1[k] = cf[1]; L.b2[k] = cf[2]; L.a1[k] = cf[3]; L.a2[k] = cf[4];
                 const int* q = stLane + P.pool[d.secStateOff + sec];
                 L.acc[k] = (long long)(((unsigned long long)(unsigned)q[1] << 32) | (unsigned)q[0]);

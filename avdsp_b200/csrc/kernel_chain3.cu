@@ -203,7 +203,8 @@ __device__ __forceinline__ void cascadeWarp(const ChainPlan& P, const Chain2Args
     L.X1 = L.X2 = 0;
 #pragma unroll
     for (int k = 0; k < NSEC; k++) {
-        const int* cf = P.pool + d.coefOff + 5 * (sec0 + k);
+        int cf[5];
+        sectionCoefs(P.pool + d.coefOff + 5 * (sec0 + k), A.coefs, A.coefPitch, P.pool[d.coefColOff + sec0 + k], s0 + sl, cf);
         L.b0[k] = cf[0]; L.b1[k] = cf[1]; L.b2[k] = cf[2]; L.a1[k] = cf[3]; L.a2[k] = cf[4];
         L.y3[k] = 0;
         {
@@ -497,10 +498,13 @@ __device__ __forceinline__ void cascadeWarpF(const ChainPlan& P, const Chain2Arg
 
     CascF<NSEC> L;
     FltGuard mn;            // exactness guard (avdsp_dev.cuh fltGuard): smallest guard word of every value loaded or produced
+    bool coefBad = false;   // a table coefficient outside what the guard can bound (fltCoefOutOfRange)
     L.X1 = L.X2 = 0.0f;
 #pragma unroll
     for (int k = 0; k < NSEC; k++) {
-        const int* cf = P.pool + d.coefOff + 5 * (sec0 + k);
+        int cf[5];
+        sectionCoefs(P.pool + d.coefOff + 5 * (sec0 + k), A.coefs, A.coefPitch, P.pool[d.coefColOff + sec0 + k], s0 + sl, cf);
+        if (A.coefs) for (int q = 0; q < 5; q++) coefBad |= fltCoefOutOfRange(cf[q]);
         L.b0[k] = __int_as_float(cf[0]); L.b1[k] = __int_as_float(cf[1]); L.b2[k] = __int_as_float(cf[2]);
         L.a1[k] = __int_as_float(cf[3]); L.a2[k] = __int_as_float(cf[4]);
         L.y3[k] = 0.0f;
@@ -510,6 +514,7 @@ __device__ __forceinline__ void cascadeWarpF(const ChainPlan& P, const Chain2Arg
         if (k == 0) { L.X1 = L.rx1[0]; L.X2 = L.rx2[0]; }
         fltGuard(mn, L.acc[k]); fltGuard(mn, L.rx1[k]); fltGuard(mn, L.rx2[k]); fltGuard(mn, L.y1[k]); fltGuard(mn, L.y2[k]);
     }
+    if (coefBad) mn.mn = 0u;
     // the post ring is the delay line (ring of s.31 values behind the saturation), exactly as in the fixed-point form
     const int n = fin ? d.delayN : 0;
     int idx0 = 0, staleIdx = -1;

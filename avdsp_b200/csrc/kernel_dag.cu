@@ -141,8 +141,7 @@ __device__ __forceinline__ void dagNodeWarp(const DagPlan& P, const Chain2Args& 
             const int* q = C.st + P.pool[n.secStateOff + k];          // [acc_lo, acc_hi, x1, x2, y1, y2] (dsp_biquadSTD.h:45)
             sAcc[k] = (long long)(((unsigned long long)(unsigned)q[1] << 32) | (unsigned)q[0]);
             xa[k] = q[2]; xb[k] = q[3]; ya[k] = q[4]; yb[k] = q[5];
-#pragma unroll
-            for (int c = 0; c < 5; c++) cf[k][c] = P.pool[n.coefOff + 5 * k + c];
+            sectionCoefs(P.pool + n.coefOff + 5 * k, A.coefs, A.coefPitch, P.pool[n.coefColOff + k], s0 + lane, cf[k]);
         }
         if (n.a.delayKind == 1) delayPrime<1>(da, n.a.delayN, n.a.delayOff, C.st, C.blk + G.aDlyOff[w], nullptr, G.aDlyMask[w]);
         if (n.a.delayKind == 2) delayPrime<2>(da, n.a.delayN, n.a.delayOff, C.st, C.blk + G.aDlyOff[w], C.blk + G.aDlyOff[w] + G.aDlyMask[w] + 1, G.aDlyMask[w]);

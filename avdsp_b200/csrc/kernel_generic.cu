@@ -125,12 +125,14 @@ __device__ __forceinline__ typename AluT<CLS>::T saturate(typename AluT<CLS>::T 
 }
 
 struct StreamRegs { Prng g; int tpdfValue, tpdfRandom, dither; };
+// this stream's view of the per-stream coefficient table (GenericArgs::coefs): its word of column c is coefs[c * pitch]
+struct CoefRow { const int* coefs; int pitch, step; };
 
 // Execute ops[i0,i1) of one core for one frame.  `io` is this lane's 32-slot sample array in shared
 // memory (stride = blockDim.x), `st` its state block in HBM.
-template <int CLS>
+template <int CLS, bool TAB>
 __device__ __forceinline__ void runCore(const GenericPlan& P, int i0, int i1, int* __restrict__ io, const int ios,
-                                        const SPi st, const int* __restrict__ big, StreamRegs& R) {
+                                        const SPi st, const int* __restrict__ big, StreamRegs& R, const CoefRow crow) {
     typedef typename AluT<CLS>::T ALU;
     typedef typename AluT<CLS>::SP SPT;
     constexpr int AW = AluT<CLS>::W;
@@ -275,13 +277,15 @@ __device__ __forceinline__ void runCore(const GenericPlan& P, int i0, int i1, in
             break; }
         case OP_BIQUADS: {
             SPi s = st + m.a;
-            const int* cf = P.pool + m.b;
+            // the plan's coefficients, or this stream's row of the coefficient table: column m.c, then coefStep per section
+            const int* cf = TAB ? crow.coefs + (size_t)m.c * crow.pitch : P.pool + m.b;
+            const size_t cq = TAB ? (size_t)crow.pitch : 1, cs = TAB ? (size_t)crow.step * crow.pitch : 5;
             if constexpr (CLS == ALU_INT64) {
                 int xn = (int)(X >> kMantBQ);
                 long long acc = 0;
-                for (int k = 0; k < m.n; k++, s += 6, cf += 5) {
+                for (int k = 0; k < m.n; k++, s += 6, cf += cs) {
                     BqStateI q; q.acc = ldA<CLS>(s); q.x1 = s[2]; q.x2 = s[3]; q.y1 = s[4]; q.y2 = s[5];
-                    xn = biquadStepI(q, xn, cf[0], cf[1], cf[2], cf[3], cf[4]);
+                    xn = biquadStepI(q, xn, cf[0], cf[cq], cf[2 * cq], cf[3 * cq], cf[4 * cq]);
                     acc = q.acc;
                     stA<CLS>(s, q.acc); s[2] = q.x1; s[3] = q.x2; s[4] = q.y1; s[5] = q.y2;
                 }
@@ -289,15 +293,15 @@ __device__ __forceinline__ void runCore(const GenericPlan& P, int i0, int i1, in
             } else {
                 float xn = toF(X);
                 ALU acc = 0;
-                for (int k = 0; k < m.n; k++, s += 6, cf += 5) {
+                for (int k = 0; k < m.n; k++, s += 6, cf += cs) {
                     acc = ldA<CLS>(s);
                     const float x1 = __int_as_float(s[2]), x2 = __int_as_float(s[3]);
                     const float y1 = __int_as_float(s[4]), y2 = __int_as_float(s[5]);
                     macc<CLS>(acc, xn, __int_as_float(cf[0]));
-                    macc<CLS>(acc, x1, __int_as_float(cf[1]));
-                    macc<CLS>(acc, x2, __int_as_float(cf[2]));
-                    macc<CLS>(acc, y1, __int_as_float(cf[3]));
-                    macc<CLS>(acc, y2, __int_as_float(cf[4]));
+                    macc<CLS>(acc, x1, __int_as_float(cf[cq]));
+                    macc<CLS>(acc, x2, __int_as_float(cf[2 * cq]));
+                    macc<CLS>(acc, y1, __int_as_float(cf[3 * cq]));
+                    macc<CLS>(acc, y2, __int_as_float(cf[4 * cq]));
                     stA<CLS>(s, acc);
                     s[2] = __float_as_int(xn); s[3] = __float_as_int(x1); s[5] = __float_as_int(y1);
                     xn = toF(acc);
@@ -484,7 +488,9 @@ __device__ __forceinline__ void runCore(const GenericPlan& P, int i0, int i1, in
 #undef IO
 }
 
-template <int CLS>
+// TAB: the launch reads a per-stream coefficient table (GenericArgs::coefs).  A template argument rather than a test: the
+// interpreter reads coefficients every frame, and the plan-only instance stays exactly what it was without the table.
+template <int CLS, bool TAB>
 __global__ void __launch_bounds__(kGenericThreads)
 k_generic(const __grid_constant__ GenericPlan P, const GenericArgs A) {
     extern __shared__ int io_s[];                       // [kIoSlots][blockDim.x], then (staged) [stateWords][blockDim.x]
@@ -506,6 +512,7 @@ k_generic(const __grid_constant__ GenericPlan P, const GenericArgs A) {
     R.tpdfValue = aux[AUX_TPDF_VALUE]; R.tpdfRandom = aux[AUX_TPDF_RANDOM]; R.dither = aux[AUX_DITHER];
     const int* in = A.in + (size_t)s * A.inStreamStride;
     int* out = A.out + (size_t)s * A.outStreamStride;
+    const CoefRow crow{TAB ? A.coefs + s : nullptr, A.coefPitch, A.coefStep};
     const int c0 = A.coreSel >= 0 ? A.coreSel : 0;
     const int c1 = A.coreSel >= 0 ? A.coreSel + 1 : P.h.nCores;
 
@@ -515,7 +522,7 @@ k_generic(const __grid_constant__ GenericPlan P, const GenericArgs A) {
 #pragma unroll
             for (int k = 0; k < kIoSlots; k++) io[k * ios] = 0;
             for (int k = 0; k < P.h.nIn; k++) io[P.h.inIdx[k] * ios] = in[(size_t)f * A.inFrameStride + (size_t)k * A.inChStride];
-            for (int c = c0; c < c1; c++) runCore<CLS>(P, P.h.coreStart[c], P.h.coreStart[c + 1], io, ios, st, A.bigPool, R);
+            for (int c = c0; c < c1; c++) runCore<CLS, TAB>(P, P.h.coreStart[c], P.h.coreStart[c + 1], io, ios, st, A.bigPool, R, crow);
             for (int k = 0; k < P.h.nOut; k++) out[(size_t)f * A.outFrameStride + (size_t)k * A.outChStride] = io[P.h.outIdx[k] * ios];
         }
     } else {
@@ -529,7 +536,7 @@ k_generic(const __grid_constant__ GenericPlan P, const GenericArgs A) {
                     for (int k = 0; k < kIoSlots; k++) io[k * ios] = 0;
                     for (int k = 0; k < P.h.nIn; k++)
                         if ((A.coreInMask[c] >> P.h.inIdx[k]) & 1u) io[P.h.inIdx[k] * ios] = in[(size_t)f * A.inFrameStride + (size_t)k * A.inChStride];
-                    runCore<CLS>(P, P.h.coreStart[c], P.h.coreStart[c + 1], io, ios, st, A.bigPool, R);
+                    runCore<CLS, TAB>(P, P.h.coreStart[c], P.h.coreStart[c + 1], io, ios, st, A.bigPool, R, crow);
                     for (int k = 0; k < P.h.nOut; k++)
                         if ((A.coreOutMask[c] >> P.h.outIdx[k]) & 1u) out[(size_t)f * A.outFrameStride + (size_t)k * A.outChStride] = io[P.h.outIdx[k] * ios];
                 }
@@ -556,16 +563,18 @@ cudaError_t launchGeneric(const GenericPlan& plan, const GenericArgs& args, cuda
     const int blocks = (A.nStreams + threads - 1) / threads;
     const size_t smem = (size_t)threads * (A.stageState ? perLane : kIoSlots * sizeof(int));
     cudaError_t e = cudaSuccess;
-#define LAUNCH_G(CLS) do { \
-        e = cudaFuncSetAttribute(k_generic<CLS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)); \
+#define LAUNCH_G1(CLS, TAB) do { \
+        e = cudaFuncSetAttribute(k_generic<CLS, TAB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)); \
         if (e != cudaSuccess) return e; \
-        k_generic<CLS><<<blocks, threads, smem, stream>>>(plan, A); } while (0)
+        k_generic<CLS, TAB><<<blocks, threads, smem, stream>>>(plan, A); } while (0)
+#define LAUNCH_G(CLS) do { if (A.coefs) LAUNCH_G1(CLS, true); else LAUNCH_G1(CLS, false); } while (0)
     switch (plan.h.aluClass) {
     case ALU_INT64: LAUNCH_G(ALU_INT64); break;
     case ALU_F32:   LAUNCH_G(ALU_F32); break;
     default:        LAUNCH_G(ALU_F64); break;
     }
 #undef LAUNCH_G
+#undef LAUNCH_G1
     return cudaGetLastError();
 }
 

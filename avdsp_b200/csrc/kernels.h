@@ -25,6 +25,10 @@ struct GenericArgs {
     // block the snapshot holds (what the stream's state was before the chain kernel touched it)
     const int* redo;            // [nStreams] or nullptr
     const int* snapshot;        // [nStreams][stateWords]
+    // per-stream coefficient table (avdsp_b200_set_coefs) or nullptr: word [column][stream] at coefs[column * coefPitch + s]; a
+    // BIQUADS micro-op's c is its first column, its sections step by coefStep (5 * the program's fs columns)
+    const int* coefs;
+    int coefPitch, coefStep;
     unsigned coreInMask[kMaxCores], coreOutMask[kMaxCores];
 };
 cudaError_t launchGeneric(const GenericPlan& plan, const GenericArgs& args, cudaStream_t stream);
@@ -77,6 +81,10 @@ struct Chain2Args {
     const int* map;
     const int* countPtr;
     int exact;
+    // per-stream coefficient table (avdsp_b200_set_coefs) or nullptr: [column][stream] words, coefs[column * coefPitch + p] for
+    // the stream at position p of the call; the cascades load their coefficients from it instead of the plan
+    const int* coefs;
+    int coefPitch;
 };
 // before a float-class chain kernel, one launch: state blocks of the range -> snapshot, flags and list counter cleared
 cudaError_t launchRedoPrepare(const int* state, int* snapshot, size_t words, int* flags, int nStreams, int* count, cudaStream_t stream);

@@ -102,6 +102,7 @@ struct ChainDesc {
     int32_t  muxStateOff;     // LOAD_MUX: data offset of the stored 64-bit result, else -1
     int32_t  coefOff;         // pool offset of 5*nsec coefficients (b0 b1 b2 a1-1 a2 per section)
     int32_t  secStateOff;     // pool offset of nsec data-area offsets (6 words each, dsp_biquadSTD.h:45)
+    int32_t  coefColOff;      // pool offset of nsec coefficient-table columns (Lowered::coefWords: the section's b0 at this fs)
     int32_t  gainBits;        // optional GAIN between cascade and saturation
     int32_t  satGainBits;     // SAT0DB_GAIN / SAT0DB_TPDF_GAIN
     int32_t  delayOff, delayN;// ring in the data area ([index][n samples]); delayN==0: none
@@ -172,7 +173,7 @@ struct DagNode {
     int32_t comb;                // 0: V = A;  +1: V = A + B;  -1: V = A - B
     int32_t postShift;           // > 0: V >>= postShift (DSP_SHIFT with a negative count) after the combination
     int32_t hasPostGain, postGain;   // then V *= gain (DSP_GAIN, 64 x 32 wrapping)
-    int32_t nsec, coefOff, secStateOff;      // cascade: x = V >> 28 (dsp_runtime.c:831); pool offsets as in ChainDesc
+    int32_t nsec, coefOff, secStateOff, coefColOff;   // cascade: x = V >> 28 (dsp_runtime.c:831); pool offsets as in ChainDesc
     int32_t exportAcc;           // a later node (or a MEM word) takes this node's 64-bit value
     int32_t memOff;              // DSP_STORE_MEM target (state offset) or -1
     int32_t finKind;             // DagFinish

@@ -72,6 +72,7 @@ class Executor:
         self.num_mem = L.avdsp_b200_num_mem(self._h)
         self.mem_words = [L.avdsp_b200_mem_word(self._h, k) for k in range(self.num_mem)]
         self.num_cores = L.avdsp_b200_num_cores(self._h)
+        self.n_coef = len(coef_words(self.words, fmt))   # columns of a set_coefs row
 
     def shards(self):
         """[(device, first_stream, n_streams, numa_node)] per GPU of the instance"""
@@ -124,6 +125,7 @@ class Executor:
         w = np.ascontiguousarray(words, dtype=np.int32)
         _check(self._L.avdsp_b200_reload_params(self._h, w.ctypes.data, len(w)))
         self.words = w
+        self.n_coef = len(coef_words(w, self.fmt))
 
     def param_index(self, offset: int, param_num: int = 0) -> int:
         """dump-file entry (offset, PARAM_NUM number) -> word index in the program (avdsp_b200_param_index)"""
@@ -133,6 +135,27 @@ class Executor:
         """streams [first_stream, first_stream + n_streams) run with program words [word_index, ...) replaced by `values`"""
         v = np.ascontiguousarray(values, dtype=np.int32).reshape(-1)
         _check(self._L.avdsp_b200_set_param(self._h, first_stream, n_streams, word_index, v.ctypes.data, len(v)))
+
+    def set_coefs(self, first: int, values):
+        """Per-stream biquad coefficients (avdsp_b200_set_coefs): row s of `values` ([n, nCoef], columns in the order of
+        coef_words(words, fmt)) holds the coefficient words of stream first + s.  A numpy array is copied from the host; a
+        contiguous int32 or float32 CUDA tensor on the instance's device is read on torch.cuda.current_stream() without a host
+        sync (a tensor on another device is refused).  Float arrays are bit patterns, never value-cast."""
+        if isinstance(values, np.ndarray):
+            v = self._as_words(values)
+            if v.ndim != 2 or v.shape[1] != self.n_coef:
+                raise ValueError(f"coefficient rows must be [n, {self.n_coef}], not {v.shape}")
+            _check(self._L.avdsp_b200_set_coefs(self._h, first, v.shape[0], v.ctypes.data, HOST, None))
+            return
+        import torch
+        if not (values.is_cuda and values.dtype in (torch.int32, torch.float32) and values.is_contiguous() and values.dim() == 2):
+            raise ValueError("device coefficient rows must be a contiguous 2-D int32 or float32 CUDA tensor")
+        if values.shape[1] != self.n_coef:
+            raise ValueError(f"coefficient rows must be [n, {self.n_coef}], not {tuple(values.shape)}")
+        if self.n_devices == 1 and values.device.index != self.device:
+            raise ValueError(f"device coefficient rows must be on cuda:{self.device}, not {values.device}")
+        stream = torch.cuda.current_stream(values.device).cuda_stream
+        _check(self._L.avdsp_b200_set_coefs(self._h, first, int(values.shape[0]), values.data_ptr(), DEVICE, stream))
 
     @property
     def num_variants(self) -> int:
@@ -257,6 +280,18 @@ def describe(words, fs: int, fmt: int = 2, n_streams: int = 1, dither: int = 31,
     buf = C.create_string_buffer(1 << 16)
     _check(_lib.lib().avdsp_b200_describe(w.ctypes.data, len(w), fs, fmt, dither, n_streams, num_sms, buf, len(buf)))
     return buf.value.decode()
+
+
+def coef_words(words, fmt: int = 2) -> np.ndarray:
+    """Word indices of the program's biquad coefficients (every section, every fs column, bypassed blocks too), ascending: the
+    column order of Executor.set_coefs.  Host-only (no CUDA device needed)."""
+    w = np.ascontiguousarray(words, dtype=np.int32)
+    L = _lib.lib()
+    n = _check(L.avdsp_b200_coef_words(w.ctypes.data, len(w), fmt, None, 0))
+    out = np.zeros(n, dtype=np.int32)
+    if n:
+        _check(L.avdsp_b200_coef_words(w.ctypes.data, len(w), fmt, out.ctypes.data, n))
+    return out
 
 
 def measure_int_peak(device: int = 0, iters: int = 4096) -> float:

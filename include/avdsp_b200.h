@@ -188,6 +188,36 @@ int  avdsp_b200_param_index(const avdsp_b200_t *, int offset, int paramNum);
 int  avdsp_b200_set_param(avdsp_b200_t *, int firstStream, int nStreams, int wordIndex, const int32_t *values, int nWords);
 int  avdsp_b200_num_variants(const avdsp_b200_t *);      /* distinct parameter sets alive (1 = no override) */
 
+/* Per-stream biquad coefficients in one launch: a room EQ or crossover per stream without a parameter variant per stream.
+ *
+ * Program words that are biquad coefficients: the b0 b1 b2 a1 a2 words of every section of every DSP_BIQUADS parameter block,
+ * for EVERY sampling-frequency column, bypassed blocks included.  Listed once each, in ascending word order (two BIQUADS opcodes
+ * that share a parameter block share its words).  The list is the column order of avdsp_b200_set_coefs.  Host-only: validates
+ * the program like avdsp_b200_describe (same error codes) and needs no instance and no CUDA device.  Writes at most maxOut
+ * indices and returns the count (0: no biquad in the program), or an error code. */
+int  avdsp_b200_coef_words(const int32_t *prog, int progWords, int format, int32_t *wordIndex, int maxOut);
+/* Per-stream coefficients at batch width.  values = nStreams rows of nCoef 32-bit words, nCoef = the count avdsp_b200_coef_words
+ * returns; row s holds the coefficient words of stream firstStream + s in that column order: Q4.28 integers for DSP_FORMAT 2,
+ * float bit patterns for the float formats.  memspace AVDSP_B200_HOST: the rows are copied before the call returns.
+ * AVDSP_B200_DEVICE: the buffer is read in order on cudaStream (a cudaStream_t), after every launch enqueued on the instance
+ * before this call, and the host is not blocked (the first call of an instance allocates the table and may wait).
+ * The effect is exactly avdsp_b200_set_param(firstStream + s, 1, w, &row[s][col], 1) for every stream s and column col with word
+ * index w, and outputs and state are bit-identical to that; but a call still costs the launches of one parameter set, however
+ * many distinct rows there are (the kernels load each stream's coefficients from the table once per launch).
+ *  - The first call creates the instance's coefficient table.  Every stream's row starts from the words the stream runs with at
+ *    that moment: the program's, or those of its set_param variant.  avdsp_b200_num_variants does not count the table.
+ *  - The latest call wins for a word.  While a table exists, set_param on coefficient words writes those streams' rows and
+ *    creates no variant; set_param on any other word (gains, delays, bypass flags) makes variants as before, and they combine
+ *    with the rows.  Runs of neighbouring streams that share a variant launch as before, every launch reading the table.
+ *  - reload_params drops the table (like every override).  reset keeps it: rows hold every fs column, so a reset to another
+ *    rate runs that rate's columns.
+ *  - Refusals change nothing: AVDSP_B200_ERR_UNSUPPORTED for a program without biquad coefficients, for DEVICE rows on a
+ *    multi-device instance (HOST rows are split over its shards), and for a program whose parameter blocks overlap or a variant
+ *    that changed a block's section count; AVDSP_B200_ERR_ARG for a bad stream range, NULL values or an unknown memspace.
+ *  - DSP_FORMAT 3 and 5 on the chain kernels: a row with a non-zero coefficient outside [2^-60, 2^7) sends its stream through the
+ *    exact re-execution of the float class inside the same call, so every stream stays bit-exact. */
+int  avdsp_b200_set_coefs(avdsp_b200_t *, int firstStream, int nStreams, const int32_t *values, int memspace, void *cudaStream);
+
 /* Per-stream state block, int32 words:  [0,dataSize) = the reference data area, same word offsets
  * (runtime/dsp_runtime.c:137-141);  then 8 aux words (xoshiro s0..s3, tpdfValue, tpdfRandom, current
  * global dither, pad -- the reference's process globals, runtime/dsp_tpdf.h:11-33);  then the 64-bit
