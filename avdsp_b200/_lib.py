@@ -25,7 +25,7 @@ SYMBOLS = [
     "avdsp_b200_last_error", "avdsp_b200_measure_int_peak", "avdsp_b200_measure_f32_peak",
     "avdsp_b200_create_multi", "avdsp_b200_num_devices", "avdsp_b200_shard_info", "avdsp_b200_host_alloc", "avdsp_b200_host_free",
     "avdsp_b200_copy_only", "avdsp_b200_param_index", "avdsp_b200_set_param", "avdsp_b200_num_variants",
-    "avdsp_b200_coef_words", "avdsp_b200_set_coefs",
+    "avdsp_b200_coef_words", "avdsp_b200_set_coefs", "avdsp_b200_fir_tap_words", "avdsp_b200_set_fir_taps",
 ]
 
 _lib = None
@@ -68,6 +68,8 @@ def lib():
     L.avdsp_b200_num_variants.argtypes = [vp]
     L.avdsp_b200_coef_words.argtypes = [vp, ci, ci, vp, ci]
     L.avdsp_b200_set_coefs.argtypes = [vp, ci, ci, vp, ci, vp]
+    L.avdsp_b200_fir_tap_words.argtypes = [vp, ci, ci, vp, ci]
+    L.avdsp_b200_set_fir_taps.argtypes = [vp, ci, ci, vp, ci, vp]
     L.avdsp_b200_destroy.argtypes = [vp]
     L.avdsp_b200_destroy.restype = None
     L.avdsp_b200_reset.argtypes = [vp, ci, vp, ci]

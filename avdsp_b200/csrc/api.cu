@@ -146,6 +146,22 @@ __global__ void __launch_bounds__(256) k_coef_scatter(int* __restrict__ tab, int
     }
 }
 
+// Exactness flags of the per-stream FIR table (float programs): flags[first + s] = 1 when row s holds a non-zero tap below
+// 2^-60, the bound under which the FIR kernels' products can come near 2^-126 and differ from dspMulFloatFloat (the rule
+// buildFirPlan applies to the program's own taps).  Every fs column counts.  One warp per stream.
+__global__ void __launch_bounds__(256) k_fir_tap_flags(const int* __restrict__ tab, int nCols, int first, int n, int* __restrict__ flags) {
+    const int s = (int)(blockIdx.x * (blockDim.x / 32) + threadIdx.x / 32), lane = (int)(threadIdx.x & 31);
+    if (s >= n) return;
+    const int* row = tab + (size_t)(first + s) * nCols;
+    bool tiny = false;
+    for (int c = lane; c < nCols; c += 32) {
+        const unsigned ex = ((unsigned)row[c] >> 23) & 255u;
+        tiny |= ex != 0u && ex < 127u - 60u;
+    }
+    tiny = __any_sync(0xFFFFFFFFu, tiny);
+    if (lane == 0) flags[first + s] = tiny ? 1 : 0;
+}
+
 #include "instance.h"
 
 static int quiesce(avdsp_b200* h);
@@ -219,6 +235,11 @@ static int uploadPlanData(avdsp_b200* h) {
         CU(cudaMalloc(&h->dBig, h->bigWords * 4));
         CU(cudaMemcpy(h->dBig, L.bigPool.data(), h->bigWords * 4, cudaMemcpyHostToDevice));
     }
+    if (h->dFirCol) { cudaFree(h->dFirCol); h->dFirCol = nullptr; }
+    if (!L.firColOfOp.empty()) {
+        CU(cudaMalloc(&h->dFirCol, L.firColOfOp.size() * 4));
+        CU(cudaMemcpy(h->dFirCol, L.firColOfOp.data(), L.firColOfOp.size() * 4, cudaMemcpyHostToDevice));
+    }
     std::vector<ChainLane> lanes2;
     planGeometries(h, &lanes2);
     if (h->chain2Usable) {
@@ -275,6 +296,7 @@ static void freeAll(avdsp_b200* h) {
     cudaSetDevice(h->device);
     if (h->dState) cudaFree(h->dState);
     if (h->dBig) cudaFree(h->dBig);
+    if (h->dFirCol) cudaFree(h->dFirCol);
     if (h->dMemInit) cudaFree(h->dMemInit);
     if (h->dSeeds) cudaFree(h->dSeeds);
     if (h->dLanes2) cudaFree(h->dLanes2);
@@ -288,6 +310,9 @@ static void freeAll(avdsp_b200* h) {
     if (h->dFirWs) cudaFree(h->dFirWs);
     if (h->dCoef) cudaFree(h->dCoef);
     if (h->dCoefStage) cudaFree(h->dCoefStage);
+    if (h->dFirTab) cudaFree(h->dFirTab);
+    if (h->dFirFlags) cudaFree(h->dFirFlags);
+    if (h->dFirTcPer) cudaFree(h->dFirTcPer);
     if (h->pcmRaw) cudaFree(h->pcmRaw);
     if (h->pcmIn) cudaFree(h->pcmIn);
     if (h->pcmOut) cudaFree(h->pcmOut);
@@ -376,6 +401,9 @@ int avdsp_b200_reset(avdsp_b200_t* h, int fs, const int32_t* seeds, int defaultD
         if (nl.gen.h.stateWords != h->L.gen.h.stateWords) return setErr(AVDSP_B200_ERR_ARG, "state layout changed on reset");
         h->L = nl;
         const int r = uploadPlanData(h); if (r < 0) return r;
+        // the per-stream Toeplitz planes follow this rate's tap blocks (and their size its longest impulse)
+        if (h->dFirTcPer) { cudaFree(h->dFirTcPer); h->dFirTcPer = nullptr; }
+        h->firTcPerValid = h->firTcPerFailed = false;
         for (avdsp_b200* v : h->variants) {                   // the overrides stay; their plans follow the new rate / dither
             Lowered vl;
             const std::vector<int32_t> vw = v->L.words;
@@ -454,6 +482,8 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
     } else return setErr(AVDSP_B200_ERR_ARG, "unknown layout");
     int* st = h->dState + (size_t)first * P.stateWords;
     const int* coefs = h->dCoef ? h->dCoef + first : nullptr;     // per-stream coefficient table, positioned like the state blocks
+    const int nTapCols = (int)h->L.firTapWords.size();
+    const int* firTaps = h->dFirTab ? h->dFirTab + (size_t)first * nTapCols : nullptr;      // ... and the FIR table
     if (ordered) CU(cudaStreamWaitEvent(stream, h->evLast, 0));          // stream-ordered after the instance's previous launch (see evLast)
     // the fused kernels run the canonical order; a plugin-order request may use them when the two orders provably agree
     const bool chainOrder = (h->period == 0 || pl->L.orderIndependent) && coreSel < 0 && !planOverride;
@@ -471,11 +501,29 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
     if (chainOrder && pl->mixUsable && (h->kernelSel == AVDSP_B200_KERNEL_AUTO || h->kernelSel == AVDSP_B200_KERNEL_MIX)) use = AVDSP_B200_KERNEL_MIX;
     if (chainOrder && pl->firUsable && (h->kernelSel == AVDSP_B200_KERNEL_AUTO || h->kernelSel == AVDSP_B200_KERNEL_FIR)) use = AVDSP_B200_KERNEL_FIR;
     // tensor-core Toeplitz GEMM: the bit-exact int8-limb form is the default for fixed-point batches that fill a tile;
-    // the 3xTF32 form (stated tolerance) only on request
+    // the 3xTF32 form (stated tolerance) only on request.  With a per-stream FIR table the int8-limb form runs per stream (a
+    // CTA = 128 outputs x 64 output blocks of one stream), which AUTO takes when a call fills those 64 blocks (8192 frames);
+    // the 3xTF32 form takes shared taps only
+    const bool fixedTc = pl->L.fir.aluClass == ALU_INT64 && pl->L.fir.maxLen >= 256;
+    if (h->kernelSel == AVDSP_B200_KERNEL_FIR_TC && firTaps && pl->L.fir.aluClass != ALU_INT64)
+        return setErr(AVDSP_B200_ERR_UNSUPPORTED, "the 3xTF32 tensor-core FIR kernel takes taps every stream shares; this instance has a per-stream FIR table");
     if (chainOrder && pl->firUsable && (h->kernelSel == AVDSP_B200_KERNEL_FIR_TC ||
-        (h->kernelSel == AVDSP_B200_KERNEL_AUTO && pl->L.fir.aluClass == ALU_INT64 && n >= 32 && nFrames >= 128 && pl->L.fir.maxLen >= 256)))
+        (h->kernelSel == AVDSP_B200_KERNEL_AUTO && fixedTc && (firTaps ? nFrames >= 8192 && !h->firTcPerFailed : n >= 32 && nFrames >= 128))))
         use = AVDSP_B200_KERNEL_FIR_TC;
-    if (h->kernelSel == AVDSP_B200_KERNEL_FIR_TC && use != AVDSP_B200_KERNEL_FIR_TC)
+    if (use == AVDSP_B200_KERNEL_FIR_TC && firTaps && !h->dFirTcPer && !h->firTcPerFailed) {
+        // every stream's Toeplitz planes (C4: 4.3 MB per stream); when they do not fit, this instance runs k_fir with its table
+        const size_t bytes = firTcPerTapsBytes(h->L.fir, h->nStreams);
+        if (cudaMalloc(&h->dFirTcPer, bytes) != cudaSuccess) {
+            cudaGetLastError();
+            h->dFirTcPer = nullptr; h->firTcPerFailed = true;
+            char line[160];
+            snprintf(line, sizeof line, "per-stream tensor-core FIR: %zu MB of Toeplitz planes could not be allocated, k_fir runs the FIR table\n", bytes >> 20);
+            h->trace += line;
+        }
+        h->firTcPerValid = false;
+    }
+    if (use == AVDSP_B200_KERNEL_FIR_TC && firTaps && h->firTcPerFailed) use = AVDSP_B200_KERNEL_FIR;
+    if (h->kernelSel == AVDSP_B200_KERNEL_FIR_TC && use != AVDSP_B200_KERNEL_FIR_TC && !(firTaps && h->firTcPerFailed))
         return setErr(AVDSP_B200_ERR_UNSUPPORTED, "tensor-core FIR kernel requested but this program/order does not map to it: " + pl->L.firWhyNot);
     if (h->kernelSel == AVDSP_B200_KERNEL_FIR && use != AVDSP_B200_KERNEL_FIR)
         return setErr(AVDSP_B200_ERR_UNSUPPORTED, "FIR kernel requested but this program/order does not map to it: " + pl->L.firWhyNot);
@@ -492,7 +540,24 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         A.inStreamStride = inSS; A.outStreamStride = outSS;
         A.inFrameStride = inFS; A.inChStride = inCS; A.outFrameStride = outFS; A.outChStride = outCS;
         int nl = 0;
-        if (use == AVDSP_B200_KERNEL_FIR_TC) {
+        if (use == AVDSP_B200_KERNEL_FIR_TC && firTaps) {
+            if (!h->firTcPerValid) {                              // rows changed since the planes were built: all streams again
+                e = launchFirTcBuildTaps(h->L.fir, h->dFirTab, nTapCols, h->nStreams, h->dFirTcPer, stream);
+                if (e != cudaSuccess) return cudaErr(e, "kernel launch");
+                h->firTcPerValid = true;
+                h->launches++;
+            }
+            const size_t need = firTcPerWorkspaceBytes(pl->L.fir, n, nFrames);
+            if (need > h->firWsBytes) {
+                CU(cudaStreamSynchronize(stream));
+                if (h->dFirWs) cudaFree(h->dFirWs);
+                h->dFirWs = nullptr; h->firWsBytes = 0;
+                CU(cudaMalloc(&h->dFirWs, need));
+                h->firWsBytes = need;
+            }
+            A.taps = firTaps; A.tapPitch = nTapCols;
+            e = launchFirTcPer(pl->L.fir, A, h->dFirTcPer + (size_t)first * (firTcPerTapsBytes(h->L.fir, 1)), h->dFirWs, stream, &nl);
+        } else if (use == AVDSP_B200_KERNEL_FIR_TC) {
             const int kind = pl->L.fir.aluClass == ALU_INT64 ? FIRTC_I8 : FIRTC_TF32;
             const size_t need = firTcWorkspaceBytes(pl->L.fir, kind, n, nFrames);
             if (need > h->firWsBytes) {
@@ -503,7 +568,27 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
                 h->firWsBytes = need;
             }
             e = launchFirTc(pl->L.fir, kind, A, pl->dFirTaps, h->dFirWs, stream, &nl);
-        } else e = launchFir(pl->L.fir, A, h->numSMs, stream, &nl);
+        } else {
+            A.taps = firTaps; A.tapPitch = nTapCols;
+            A.skip = firTaps && pl->L.fir.aluClass == ALU_F32 ? h->dFirFlags + first : nullptr;
+            e = launchFir(pl->L.fir, A, h->numSMs, stream, &nl);
+            if (e == cudaSuccess && A.skip) {
+                // float rows with a tap the FIR kernels cannot multiply exactly: their CTAs did nothing, and the interpreter
+                // runs those streams now from their untouched state blocks (one launch; streams without the flag return at once)
+                GenericArgs X{};
+                X.in = in; X.out = out; X.state = st; X.bigPool = pl->dBig;
+                X.nStreams = n; X.nFrames = nFrames;
+                X.inStreamStride = inSS; X.outStreamStride = outSS;
+                X.inFrameStride = inFS; X.inChStride = inCS; X.outFrameStride = outFS; X.outChStride = outCS;
+                X.coreSel = -1; X.period = 0;
+                X.redo = A.skip; X.snapshot = st;
+                X.coefs = coefs; X.coefPitch = h->nStreams; X.coefStep = 5 * pl->L.nFreq;
+                X.firTaps = firTaps; X.firPitch = nTapCols; X.firCol = pl->dFirCol;
+                for (int c = 0; c < P.nCores && c < kMaxCores; c++) { X.coreInMask[c] = pl->L.cores[c].usedIn; X.coreOutMask[c] = pl->L.cores[c].usedOut; }
+                e = launchGeneric(G, X, stream);
+                nl++;
+            }
+        }
         h->lastKernel = use;
         h->launches += nl - 1;
     } else if (use == AVDSP_B200_KERNEL_MIX) {
@@ -602,6 +687,7 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         A.inFrameStride = inFS; A.inChStride = inCS; A.outFrameStride = outFS; A.outChStride = outCS;
         A.coreSel = coreSel; A.period = coreSel >= 0 ? 0 : h->period;
         A.coefs = planOverride ? nullptr : coefs; A.coefPitch = h->nStreams; A.coefStep = 5 * pl->L.nFreq;
+        A.firTaps = planOverride ? nullptr : firTaps; A.firPitch = nTapCols; A.firCol = pl->dFirCol;
         for (int c = 0; c < P.nCores && c < kMaxCores; c++) { A.coreInMask[c] = pl->L.cores[c].usedIn; A.coreOutMask[c] = pl->L.cores[c].usedOut; }
         e = launchGeneric(G, A, stream);
         h->lastKernel = AVDSP_B200_KERNEL_GENERIC;
@@ -661,6 +747,15 @@ static int launchRange(avdsp_b200* h, const int* in, int* out, int nFrames, int 
         }
         CU(cudaEventRecord(h->evLast, stream));
     }
+    return 0;
+}
+
+// the FIR table's exactness flags of streams [first, first+n), on `s` after the rows were written there (float programs only)
+static int firTapFlags(avdsp_b200* h, int first, int n, cudaStream_t s) {
+    if (!h->dFirFlags || n == 0) return 0;
+    k_fir_tap_flags<<<(unsigned)((n + 7) / 8), 256, 0, s>>>(h->dFirTab, (int)h->L.firTapWords.size(), first, n, h->dFirFlags);
+    CU(cudaGetLastError());
+    h->launches++;
     return 0;
 }
 
@@ -1030,16 +1125,22 @@ int avdsp_b200_set_param(avdsp_b200_t* h, int firstStream, int nStreams, int wor
         return 0;
     }
     { const int q = quiesce(h); if (q < 0) return q; }
-    // while the instance has a coefficient table, coefficient words are written into the streams' rows; the other words make
-    // variants as without one.  Everything that can fail (lowering a variant) happens before anything changes.
+    // while the instance has a coefficient table (a FIR table), coefficient words (tap words) are written into the streams' rows;
+    // the other words make variants as without one.  Everything that can fail (lowering a variant) happens before anything changes.
     const std::vector<int32_t>& cw = h->L.coefWords;
-    std::vector<int> colOf(nWords, -1);                  // table column of word k of the call, or -1
-    if (h->dCoef)
-        for (int k = 0; k < nWords; k++) {
-            const auto it = std::lower_bound(cw.begin(), cw.end(), wordIndex + k);
-            if (it != cw.end() && *it == wordIndex + k) colOf[k] = (int)(it - cw.begin());
-        }
-    const bool anyVariantWord = std::find(colOf.begin(), colOf.end(), -1) != colOf.end();
+    const std::vector<int32_t>& tw = h->L.firTapWords;
+    auto columns = [&](bool on, const std::vector<int32_t>& list) {      // table column of word k of the call, or -1
+        std::vector<int> col(nWords, -1);
+        if (on)
+            for (int k = 0; k < nWords; k++) {
+                const auto it = std::lower_bound(list.begin(), list.end(), wordIndex + k);
+                if (it != list.end() && *it == wordIndex + k) col[k] = (int)(it - list.begin());
+            }
+        return col;
+    };
+    const std::vector<int> colOf = columns(h->dCoef != nullptr, cw), tapColOf = columns(h->dFirTab != nullptr, tw);
+    bool anyVariantWord = false;
+    for (int k = 0; k < nWords; k++) anyVariantWord = anyVariantWord || (colOf[k] < 0 && tapColOf[k] < 0);
     // streams of the range may sit on different variants already: patch each of those once
     std::map<int, int> moved;                 // old variant -> new variant
     if (anyVariantWord) {
@@ -1052,12 +1153,14 @@ int avdsp_b200_set_param(avdsp_b200_t* h, int firstStream, int nStreams, int wor
             const int old = h->variantOf.empty() ? 0 : h->variantOf[s];
             if (moved.count(old)) continue;
             std::vector<int32_t> words = old ? h->variants[old - 1]->L.words : h->L.words;
-            for (int k = 0; k < nWords; k++) if (colOf[k] < 0) words[wordIndex + k] = values[k];
+            for (int k = 0; k < nWords; k++) if (colOf[k] < 0 && tapColOf[k] < 0) words[wordIndex + k] = values[k];
             int id = 0;
             const int r = variantFor(h, words, &id);
             if (r < 0) return undo(r);
             if (h->dCoef && id > 0 && h->variants[id - 1]->L.coefWords != cw)
                 return undo(setErr(AVDSP_B200_ERR_UNSUPPORTED, "this change moves biquad coefficient words the coefficient table holds (section count)"));
+            if (h->dFirTab && id > 0 && h->variants[id - 1]->L.firTapWords != tw)
+                return undo(setErr(AVDSP_B200_ERR_UNSUPPORTED, "this change moves FIR tap words the FIR table holds (tap block length)"));
             moved.emplace(old, id);
         }
     }
@@ -1070,6 +1173,20 @@ int avdsp_b200_set_param(avdsp_b200_t* h, int firstStream, int nStreams, int wor
                                cudaMemcpyHostToDevice, h->stream));
             CU(cudaStreamSynchronize(h->stream));
         }
+        CU(cudaEventRecord(h->evLast, h->stream));
+    }
+    if (h->dFirTab) {
+        bool any = false;
+        std::vector<int32_t> col((size_t)nStreams);
+        for (int k = 0; k < nWords; k++) {
+            if (tapColOf[k] < 0) continue;
+            std::fill(col.begin(), col.end(), values[k]);       // one word of every row of the range: a strided copy
+            CU(cudaMemcpy2DAsync(h->dFirTab + (size_t)firstStream * tw.size() + tapColOf[k], tw.size() * 4, col.data(), 4, 4, (size_t)nStreams,
+                                 cudaMemcpyHostToDevice, h->stream));
+            CU(cudaStreamSynchronize(h->stream));
+            any = true;
+        }
+        if (any) { const int r = firTapFlags(h, firstStream, nStreams, h->stream); if (r < 0) return r; h->firTcPerValid = false; }
         CU(cudaEventRecord(h->evLast, h->stream));
     }
     if (!anyVariantWord) return 0;
@@ -1172,6 +1289,90 @@ int avdsp_b200_set_coefs(avdsp_b200_t* h, int firstStream, int nStreams, const i
     return 0;
 }
 
+int avdsp_b200_fir_tap_words(const int32_t* prog, int progWords, int format, int32_t* wordIndex, int maxOut) {
+    if (maxOut < 0 || (maxOut > 0 && !wordIndex)) return setErr(AVDSP_B200_ERR_ARG, "bad output buffer");
+    // the column list does not depend on the rate: lower at the lowest one the header admits (decodeProgram validates it)
+    const int fi = (prog && progWords > H_FREQMIN) ? prog[H_FREQMIN] : 0;
+    const int fs = (fi >= 0 && fi < kNumFreq) ? kFreqTable[fi] : 0;
+    std::unique_ptr<Lowered> L(new Lowered);
+    std::string err;
+    int rc = decodeProgram(prog, progWords, 0x7FFFFFFF, format, fs, 31, L.get(), &err);
+    if (rc < 0) return setErr(rc, err);
+    // the list covers every fs column: the program must lower at every rate it admits, as describe would check each of them
+    std::unique_ptr<Lowered> Lr(new Lowered);
+    for (int f = fi + 1; f <= prog[H_FREQMAX] && f < kNumFreq; f++) {
+        rc = decodeProgram(prog, progWords, 0x7FFFFFFF, format, kFreqTable[f], 31, Lr.get(), &err);
+        if (rc < 0) return setErr(rc, err);
+    }
+    const int n = (int)L->firTapWords.size();
+    for (int k = 0; k < n && k < maxOut; k++) wordIndex[k] = L->firTapWords[k];
+    return n;
+}
+
+// The instance's FIR table, created on first use: every stream's row holds the tap words it runs with now (the program's, or
+// its variant's).  Float programs get the exactness flags with it.  Synchronous: the table is not in use yet.
+static int ensureFirTable(avdsp_b200* h) {
+    if (h->dFirTab) return 0;
+    const std::vector<int32_t>& tw = h->L.firTapWords;
+    const size_t N = (size_t)h->nStreams, nt = tw.size();
+    std::vector<int32_t> init(nt * N);
+    for (size_t s = 0; s < N; s++) {
+        const int v = h->variantOf.empty() ? 0 : h->variantOf[s];
+        const std::vector<int32_t>& w = v ? h->variants[v - 1]->L.words : h->L.words;
+        for (size_t c = 0; c < nt; c++) init[s * nt + c] = w[tw[c]];
+    }
+    int* d = nullptr;
+    int* f = nullptr;
+    auto fail = [&](cudaError_t e) { if (d) cudaFree(d); if (f) cudaFree(f); return cudaErr(e, "FIR table upload"); };
+    cudaError_t e = cudaMalloc(&d, init.size() * 4);
+    if (e != cudaSuccess) { d = nullptr; return fail(e); }
+    if (h->L.gen.h.aluClass == ALU_F32) {
+        e = cudaMalloc(&f, N * 4);
+        if (e != cudaSuccess) { f = nullptr; return fail(e); }
+    }
+    e = cudaMemcpyAsync(d, init.data(), init.size() * 4, cudaMemcpyHostToDevice, h->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    if (e != cudaSuccess) return fail(e);
+    h->dFirTab = d; h->dFirFlags = f;
+    { const int r = firTapFlags(h, 0, h->nStreams, h->stream); if (r < 0) return r; }
+    CU(cudaStreamSynchronize(h->stream));
+    return 0;
+}
+
+int avdsp_b200_set_fir_taps(avdsp_b200_t* h, int firstStream, int nStreams, const int32_t* values, int memspace, void* cudaStream) {
+    if (!h || !values) return setErr(AVDSP_B200_ERR_ARG, "NULL argument");
+    if (firstStream < 0 || nStreams < 0 || (long long)firstStream + nStreams > h->nStreams) return setErr(AVDSP_B200_ERR_ARG, "bad stream range");
+    if (memspace != AVDSP_B200_HOST && memspace != AVDSP_B200_DEVICE) return setErr(AVDSP_B200_ERR_ARG, "unknown memspace");
+    const int nTaps = (int)h->L.firTapWords.size();
+    if (nTaps == 0) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "the program has no FIR taps");
+    if (!h->shards.empty()) {
+        if (memspace != AVDSP_B200_HOST) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a multi-device instance takes HOST FIR rows (device buffers belong to one GPU)");
+        for (const avdsp_b200* sh : h->shards)
+            for (const avdsp_b200* v : sh->variants)
+                if (v->L.firTapWords != h->L.firTapWords) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a parameter variant moved the FIR tap words (tap block length)");
+        return forShards(h, [&](int k, avdsp_b200* sh) {
+            const int a = std::max(firstStream, h->shardFirst[k]), b = std::min(firstStream + nStreams, h->shardFirst[k + 1]);
+            if (b <= a) return 0;
+            return avdsp_b200_set_fir_taps(sh, a - h->shardFirst[k], b - a, values + (size_t)(a - firstStream) * nTaps, AVDSP_B200_HOST, nullptr);
+        });
+    }
+    for (const avdsp_b200* v : h->variants)
+        if (v->L.firTapWords != h->L.firTapWords) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a parameter variant moved the FIR tap words (tap block length)");
+    if (nStreams == 0) return 0;
+    CU(cudaSetDevice(h->device));
+    { const int r = ensureFirTable(h); if (r < 0) return r; }
+    const cudaStream_t s = memspace == AVDSP_B200_DEVICE ? (cudaStream_t)cudaStream : h->stream;
+    CU(cudaStreamWaitEvent(s, h->evLast, 0));                 // after every launch enqueued on the instance before this call
+    // rows arrive [stream][column], the table's own layout: one copy
+    CU(cudaMemcpyAsync(h->dFirTab + (size_t)firstStream * nTaps, values, (size_t)nStreams * nTaps * 4,
+                       memspace == AVDSP_B200_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, s));
+    { const int r = firTapFlags(h, firstStream, nStreams, s); if (r < 0) return r; }
+    h->firTcPerValid = false;
+    CU(cudaEventRecord(h->evLast, s));
+    if (memspace == AVDSP_B200_HOST) CU(cudaStreamSynchronize(s));    // the caller's buffer is free again
+    return 0;
+}
+
 int avdsp_b200_num_variants(const avdsp_b200_t* h) {
     if (!h) return 0;
     int n = h->shards.empty() ? 1 + (int)h->variants.size() : 0;
@@ -1191,6 +1392,10 @@ int avdsp_b200_reload_params(avdsp_b200_t* h, const int32_t* prog, int progWords
     { const int q = quiesce(h); if (q < 0) return q; }
     dropVariants(h);                                          // a new program for everybody: per-stream overrides start over
     if (h->dCoef) { cudaFree(h->dCoef); h->dCoef = nullptr; }   // ... the coefficient table too
+    if (h->dFirTab) { cudaFree(h->dFirTab); h->dFirTab = nullptr; }      // ... and the FIR table
+    if (h->dFirFlags) { cudaFree(h->dFirFlags); h->dFirFlags = nullptr; }
+    if (h->dFirTcPer) { cudaFree(h->dFirTcPer); h->dFirTcPer = nullptr; }
+    h->firTcPerValid = h->firTcPerFailed = false;
     const int r = uploadPlanData(h);
     return r < 0 ? r : rc;
 }

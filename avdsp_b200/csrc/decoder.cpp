@@ -27,6 +27,8 @@ struct Ctx {
     int nMemSlots = 0;
     std::map<int, int> memSlotOfWord;
     std::vector<std::pair<int, int>> biquadBlocks;      // (parameter block word, sections) of every DSP_BIQUADS, bypassed too
+    std::vector<std::pair<int, int>> firBlocks;         // (first tap word, taps) of every DSP_FIR convolution entry, every fs column
+    std::vector<std::pair<int, int>> firConvs;          // (micro-op index, first tap word) of every lowered FIR convolution
 
     [[noreturn]] void fail(int code, const char* fmt, int a = 0, int b = 0) {
         char buf[256]; snprintf(buf, sizeof buf, fmt, a, b);
@@ -152,6 +154,13 @@ void lowerCore(Ctx& cx, int begin) {
                 for (int k = 0; k < 5; k++) cx.pool(cx.code(c0 + s * stride + k, p));
             cx.emit(op, num, off, first, h); break; }     // c: the block's word until lowerAll makes it a table column
         case OP_FIR: {                                      // :928-969
+            // the tap blocks of every fs column are columns of the per-stream FIR table; only this rate's entry is lowered
+            for (int f = 0; f < L->nFreq && f + 1 < skip; f++) {
+                const int32_t r = w[p + 1 + f];
+                const int64_t t = (int64_t)p + r;
+                if (r == 0 || t < 0 || t >= cx.total) continue;
+                if (w[t] > 0 && (w[t] >> 16) == 0) cx.firBlocks.emplace_back((int)t + 1, w[t]);
+            }
             int rel = arg(L->fsRel);
             if (rel == 0) break;
             int off = arg(L->nFreq);
@@ -167,6 +176,7 @@ void lowerCore(Ctx& cx, int begin) {
                 FirDesc fd; fd.tapsOff = (int)L->bigPool.size(); fd.length = lw; fd.stateOff = off;
                 for (int k = 0; k < lw; k++) L->bigPool.push_back(w[t + 1 + k]);
                 L->firs.push_back(fd);
+                cx.firConvs.emplace_back(L->gen.h.nOps, t + 1);
                 cx.emit(OP_FIR, 1, off, fd.tapsOff, lw);    // n==1: convolution, b=taps offset, c=length
             }
             break; }
@@ -694,7 +704,7 @@ void buildFirPlan(Lowered* L) {
             d.srcKind = s.op == OP_LOAD ? SRC_LOAD : SRC_LOAD_GAIN; d.srcCh = inChOfSlot[s.a]; d.srcArg = s.b;
             i++;
             if (i >= e || g.ops[i].op != OP_FIR || g.ops[i].n != 1) throw ChainFail{"a path has no FIR convolution right after its load"};
-            d.stateOff = g.ops[i].a; d.tapsOff = g.ops[i].b; d.length = g.ops[i].c;
+            d.stateOff = g.ops[i].a; d.tapsOff = g.ops[i].b; d.length = g.ops[i].c; d.tapCol = L->firColOfOp[i];
             if (d.length > kMaxFirTaps) throw ChainFail{"impulse longer than kMaxFirTaps"};
             if (g.h.aluClass == ALU_F32) {
                 // the float kernels multiply with mul.rz.ftz.f32, which equals the reference's dspMulFloatFloat (dsp_ieee754.h:336-375)
@@ -821,6 +831,21 @@ void buildCoefColumns(Ctx& cx) {
     }
 }
 
+// The FIR-table columns (Lowered::firTapWords) and the column of every lowered FIR convolution.  A tap block is a run of
+// consecutive words, all of them listed, so its taps sit in consecutive columns whatever other blocks overlap it.
+void buildFirColumns(Ctx& cx) {
+    Lowered* L = cx.L;
+    std::vector<int32_t> tw;
+    for (const auto& b : cx.firBlocks)
+        for (int k = 0; k < b.second && (int64_t)b.first + k < cx.total; k++) tw.push_back(b.first + k);
+    std::sort(tw.begin(), tw.end());
+    tw.erase(std::unique(tw.begin(), tw.end()), tw.end());
+    L->firTapWords = tw;
+    L->firColOfOp.assign(cx.firConvs.empty() ? 0 : (size_t)L->gen.h.nOps, -1);
+    for (const auto& c : cx.firConvs)
+        L->firColOfOp[c.first] = (int32_t)(std::lower_bound(tw.begin(), tw.end(), c.second) - tw.begin());
+}
+
 void lowerAll(Lowered* L) {
     Ctx cx; cx.L = L; cx.w = L->words.data(); cx.total = L->totalLength;
     cx.delayFactor = (uint32_t)(4294.967296 * (double)L->fs);      // dsp_runtime.c:81-90
@@ -829,7 +854,7 @@ void lowerAll(Lowered* L) {
     L->memWord.clear();
     for (size_t k = 0; k < keepMem.size(); k++) cx.memSlot(keepMem[k], 0);
     g.h.nOps = 0; g.h.nPool = 0;
-    L->bigPool.clear(); L->firs.clear(); cx.biquadBlocks.clear();
+    L->bigPool.clear(); L->firs.clear(); cx.biquadBlocks.clear(); cx.firBlocks.clear(); cx.firConvs.clear();
 
     g.h.nCores = (int)L->cores.size();
     uint32_t usedIn = 0, usedOut = 0;
@@ -853,6 +878,7 @@ void lowerAll(Lowered* L) {
     for (int i = 0; i < g.h.nOps; i++)
         if (g.ops[i].op == OP_LOAD_MEM || g.ops[i].op == OP_STORE_MEM) g.ops[i].a = g.h.memOff + 2 * g.ops[i].a;
     buildCoefColumns(cx);
+    buildFirColumns(cx);
 
     analyseOrder(L);
     try { buildChainPlan(L); L->chainOk = true; L->chainWhyNot.clear(); }

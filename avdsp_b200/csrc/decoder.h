@@ -47,6 +47,12 @@ struct Lowered {
     // BIQUADS micro-op's `c` is the column of its first section's b0 at the current fs, section k at c + 5 * nFreq * k.
     std::vector<int32_t> coefWords;
     bool coefTableOk = true;             // every lowered section follows that column pattern (blocks that overlap do not)
+    // FIR tap words: t + 1 .. t + lw of every DSP_FIR entry that is a convolution (length word lw > 0, lw >> 16 == 0), for every
+    // fs column, ascending, each word once.  The columns of the per-stream FIR table (avdsp_b200_set_fir_taps); a lowered FIR
+    // convolution's column (firColOfOp[its micro-op index], FirPath::tapCol) is that of its first tap at the current fs, tap k at
+    // that + k.  Kept beside the plan, not in it: the plan-only kernels never see it.
+    std::vector<int32_t> firTapWords;
+    std::vector<int32_t> firColOfOp;     // [nOps]: column of a FIR convolution micro-op, -1 for every other micro-op
     // human readable trace of the lowering (replaces the reference's DSP_PRINTF=2 opcode trace)
     std::string trace;
 };

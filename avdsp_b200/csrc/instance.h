@@ -15,6 +15,7 @@ struct avdsp_b200 {
     std::vector<int32_t> seeds;
     int* dState = nullptr;
     int* dBig = nullptr; size_t bigWords = 0;
+    int* dFirCol = nullptr;         // L.firColOfOp on the device: the FIR-table column of each micro-op (k_generic with a FIR table)
     int* dMemInit = nullptr;
     int* dSeeds = nullptr;
     avdsp::ChainLane* dLanes2 = nullptr;
@@ -69,6 +70,15 @@ struct avdsp_b200 {
     // Variants (set_param on other words) keep their own plans and read the same table.
     int* dCoef = nullptr;
     int* dCoefStage = nullptr; size_t coefStageWords = 0;     // HOST rows on their way to the table
+    // per-stream FIR table (avdsp_b200_set_fir_taps): [stream][column] int32, column = index into L.firTapWords, so that a k_fir CTA
+    // stages its stream's taps as one coalesced run; nullptr: none.  Float programs (ALU_F32) also keep one flag word per stream:
+    // set when the stream's row holds a non-zero tap below 2^-60, which the FIR kernels cannot multiply exactly (launchRun).
+    int* dFirTab = nullptr;
+    int* dFirFlags = nullptr;
+    // DSP_FORMAT 2 with a FIR table: every stream's Toeplitz limb planes for the per-stream tensor-core form (kernel_fir_tc.cu),
+    // built on the device before the first such launch after the rows changed (valid = false)
+    unsigned char* dFirTcPer = nullptr; bool firTcPerValid = false;
+    bool firTcPerFailed = false;       // their allocation failed once: this instance runs k_fir with its table
     int numaNode = -1;                 // host NUMA node next to `device` (-1: unknown)
     std::map<void*, size_t> hostAllocs;   // avdsp_b200_host_alloc: pointer -> bytes
 };

@@ -79,7 +79,10 @@ __device__ __forceinline__ void ld8(int (&v)[kFirR], const int* p) {
     v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
 }
 
-template <int CLS>
+// TAB: the taps come from the stream's row of the per-stream FIR table (FirArgs::taps), and a stream whose flag word is set
+// (FirArgs::skip, float rows with a tap the kernel cannot multiply exactly) is left to the interpreter.  A separate instance, so
+// that the shared-taps kernel stays what it was.
+template <int CLS, bool TAB>
 __global__ void __launch_bounds__(256)
 k_fir(const __grid_constant__ FirPlan P, const FirArgs A, const int nTiles, const int H) {
     extern __shared__ __align__(16) int fir_sm[];
@@ -89,12 +92,14 @@ k_fir(const __grid_constant__ FirPlan P, const FirArgs A, const int nTiles, cons
     const int tile = b % nTiles; b /= nTiles;
     const int path = b % P.nPaths;
     const int stream = b / P.nPaths;
+    if (TAB && A.skip && A.skip[stream]) return;
     const FirPath& d = P.paths[path];
     int* cs = fir_sm;                              // [H] taps, zero-padded to a multiple of 16
     int* xs = fir_sm + H + kFirPad;                // [H + TT] x window: xs[jp] = x[o0 - H + jp]
     const int N = d.length;
     const int tid = (int)threadIdx.x;
-    for (int k = tid; k < H; k += (int)blockDim.x) cs[k] = k < N ? A.bigPool[d.tapsOff + k] : 0;
+    const int* taps = TAB ? A.taps + (size_t)stream * A.tapPitch + d.tapCol : A.bigPool + d.tapsOff;
+    for (int k = tid; k < H; k += (int)blockDim.x) cs[k] = k < N ? taps[k] : 0;
     const int o0 = tile * TT;
     const int* in = A.in + (size_t)stream * A.inStreamStride + (size_t)(d.srcCh >= 0 ? d.srcCh : 0) * A.inChStride;
     const int* st = A.state + (size_t)stream * P.stateWords + d.stateOff;
@@ -137,11 +142,12 @@ k_fir(const __grid_constant__ FirPlan P, const FirArgs A, const int nTiles, cons
 }
 
 // delay line after T frames: st[i] = x[T-1-i] for i < T, the older entries move up by T (dsp_firSTD.h:43-47 applied T times)
-template <int CLS>
+template <int CLS, bool TAB>
 __global__ void __launch_bounds__(256)
 k_fir_state(const __grid_constant__ FirPlan P, const FirArgs A) {
     extern __shared__ __align__(16) int fir_sm[];
     const int path = (int)blockIdx.x % P.nPaths, stream = (int)blockIdx.x / P.nPaths;
+    if (TAB && A.skip && A.skip[stream]) return;
     const FirPath& d = P.paths[path];
     const int N = d.length, T = A.nFrames;
     const int* in = A.in + (size_t)stream * A.inStreamStride + (size_t)(d.srcCh >= 0 ? d.srcCh : 0) * A.inChStride;
@@ -152,7 +158,7 @@ k_fir_state(const __grid_constant__ FirPlan P, const FirArgs A) {
     for (int i = (int)threadIdx.x; i < N; i += (int)blockDim.x) st[i] = fir_sm[i];
 }
 
-template <int CLS>
+template <int CLS, bool TAB>
 static cudaError_t launchFirT(const FirPlan& P, const FirArgs& A, cudaStream_t stream, int* launches) {
     const int H = (P.maxLen + 15) & ~15;
     int threads = (A.nFrames + kFirR - 1) / kFirR;
@@ -160,11 +166,11 @@ static cudaError_t launchFirT(const FirPlan& P, const FirArgs& A, cudaStream_t s
     const int TT = threads * kFirR;
     const int nTiles = (A.nFrames + TT - 1) / TT;
     const size_t smem = (size_t)(2 * H + kFirPad + TT) * sizeof(int);
-    cudaError_t e = cudaFuncSetAttribute(k_fir<CLS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(k_fir<CLS, TAB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     const long long ctas = (long long)nTiles * P.nPaths * A.nStreams;
     if (ctas > 0x7FFFFFFFll) return cudaErrorInvalidConfiguration;
-    k_fir<CLS><<<(unsigned)ctas, threads, smem, stream>>>(P, A, nTiles, H);
+    k_fir<CLS, TAB><<<(unsigned)ctas, threads, smem, stream>>>(P, A, nTiles, H);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     if (launches) *launches = 2;
@@ -174,15 +180,24 @@ static cudaError_t launchFirT(const FirPlan& P, const FirArgs& A, cudaStream_t s
 cudaError_t launchFirState(const FirPlan& P, const FirArgs& A, cudaStream_t stream) {
     const unsigned grid = (unsigned)(P.nPaths * A.nStreams);
     const size_t smem = (size_t)P.maxLen * sizeof(int);
-    if (P.aluClass == ALU_INT64) k_fir_state<ALU_INT64><<<grid, 256, smem, stream>>>(P, A);
-    else k_fir_state<ALU_F32><<<grid, 256, smem, stream>>>(P, A);
+    if (A.taps) {
+        if (P.aluClass == ALU_INT64) k_fir_state<ALU_INT64, true><<<grid, 256, smem, stream>>>(P, A);
+        else k_fir_state<ALU_F32, true><<<grid, 256, smem, stream>>>(P, A);
+    } else {
+        if (P.aluClass == ALU_INT64) k_fir_state<ALU_INT64, false><<<grid, 256, smem, stream>>>(P, A);
+        else k_fir_state<ALU_F32, false><<<grid, 256, smem, stream>>>(P, A);
+    }
     return cudaGetLastError();
 }
 
 cudaError_t launchFir(const FirPlan& plan, const FirArgs& args, int numSMs, cudaStream_t stream, int* launches) {
     (void)numSMs;
-    if (plan.aluClass == ALU_INT64) return launchFirT<ALU_INT64>(plan, args, stream, launches);
-    return launchFirT<ALU_F32>(plan, args, stream, launches);
+    if (args.taps) {
+        if (plan.aluClass == ALU_INT64) return launchFirT<ALU_INT64, true>(plan, args, stream, launches);
+        return launchFirT<ALU_F32, true>(plan, args, stream, launches);
+    }
+    if (plan.aluClass == ALU_INT64) return launchFirT<ALU_INT64, false>(plan, args, stream, launches);
+    return launchFirT<ALU_F32, false>(plan, args, stream, launches);
 }
 
 } // namespace avdsp

@@ -49,12 +49,17 @@ template <> struct TcCfg<FIRTC_I8> {
 template <> struct TcCfg<FIRTC_TF32> {
     static constexpr int planes = 2, NS = 256, elemBytes = 4, nAcc = 1, tmemCols = 256, rowB = AVDSP_FIRTC_ROWB_TF32;
 };
-template <int KIND> struct TcGeo {
+// PER: the per-stream form (k_firtc<FIRTC_I8, true>): a B plane slot holds its NS rows at the swizzle phase of the first chunk,
+// so it is one 1 KB atom longer than the rows it holds, and the ring is two such stages
+constexpr int kTcSmemPer = 204800;
+template <int KIND, bool PER = false> struct TcGeo {
     typedef TcCfg<KIND> C;
     static constexpr int E = C::rowB / C::elemBytes;                       // samples of K per stage
     static constexpr int aBlob = kTcM * C::rowB, bBlob = C::NS * C::rowB;  // one plane of one stage
-    static constexpr int stageBytes = C::planes * (aBlob + bBlob);
-    static constexpr int stages = kTcSmem / stageBytes;
+    static constexpr int bSlot = PER ? bBlob + 1024 : bBlob;               // shared-memory slot of one B plane
+    static constexpr int stageBytes = C::planes * (aBlob + bSlot);
+    static constexpr int txBytes = C::planes * (aBlob + bBlob);            // bytes the bulk copies of one stage bring in
+    static constexpr int stages = (PER ? kTcSmemPer : kTcSmem) / stageBytes;
 };
 
 // byte offset of (row, byteInRow) inside a [rows][rowB] K-major tile in the canonical swizzled layout: 8-row atoms of
@@ -89,6 +94,7 @@ __device__ __forceinline__ unsigned long long smemDesc(unsigned addr) {
     constexpr unsigned long long sbo = (8ull * ROWB) >> 4, lt = ROWB == 128 ? 2ull : 4ull;
     return (unsigned long long)((addr >> 4) & 0x3FFFu) | (1ull << 16) | (sbo << 32) | (1ull << 46) | (lt << 61);
 }
+
 template <int KIND>
 __device__ __forceinline__ void mma(unsigned dTmem, unsigned long long aDesc, unsigned long long bDesc, unsigned idesc, unsigned accumulate) {
     if constexpr (KIND == FIRTC_I8)
@@ -189,12 +195,14 @@ k_firtc_pack(const __grid_constant__ FirPlan P, const FirArgs A, unsigned char* 
 }
 
 // ---- the GEMM ---------------------------------------------------------------------------------------------------
-template <int KIND>
+// PER (FIRTC_I8 only): taps of the stream's own (device-built) Toeplitz planes; the N index runs over NS consecutive 128-frame
+// output blocks of one stream instead of over streams.  blockIdx = (group of NS blocks, tile = the call's stream, path).
+template <int KIND, bool PER>
 __global__ void __launch_bounds__(kTcThreads, 1)
 k_firtc(const __grid_constant__ FirPlan P, const FirArgs A, const unsigned char* __restrict__ taps, const unsigned char* __restrict__ ws,
         const int Hc, const int Tpad, const int nStreamTiles) {
     typedef TcCfg<KIND> C;
-    typedef TcGeo<KIND> G;
+    typedef TcGeo<KIND, PER> G;
     constexpr int kTcStages = G::stages, kStageBytes = G::stageBytes;
     extern __shared__ __align__(1024) unsigned char tc_sm[];
     __shared__ __align__(8) unsigned long long bars[2 * kTcStages + 1];
@@ -205,7 +213,7 @@ k_firtc(const __grid_constant__ FirPlan P, const FirArgs A, const unsigned char*
     const int nTimeTiles = (Hc + Tpad) / G::E;
     const unsigned smBase = (smemAddr(tc_sm) + 1023u) & ~1023u;
     const unsigned barFull = smemAddr(&bars[0]), barEmpty = smemAddr(&bars[kTcStages]), barAcc = smemAddr(&bars[2 * kTcStages]);
-    constexpr unsigned aBlob = G::aBlob, bBlob = G::bBlob;
+    constexpr unsigned aBlob = G::aBlob, bBlob = G::bBlob, bSlot = G::bSlot;
 
     if (warp == 0 && lane == 0) {
         for (int s = 0; s < kTcStages; s++) { mbarInit(barFull + 8 * s, 1); mbarInit(barEmpty + 8 * s, 1); }
@@ -224,19 +232,24 @@ k_firtc(const __grid_constant__ FirPlan P, const FirArgs A, const unsigned char*
     if (warp == 0) {
         if (lane == 0) {
             // ===== producer: one bulk copy per operand plane and stage =====
-            const unsigned char* aSrc = taps + (size_t)path * C::planes * nStages * aBlob;
-            const unsigned char* bSrc = ws + (((size_t)path * C::planes) * nStreamTiles + tile) * nTimeTiles * (size_t)bBlob;
-            const size_t bPlaneStride = (size_t)nStreamTiles * nTimeTiles * bBlob;
-            const int tau0 = Q * (kTcM / G::E);
+            const unsigned char* aSrc = taps + ((PER ? (size_t)tile * P.nPaths : 0) + path) * C::planes * nStages * aBlob;
+            const unsigned char* bSrc = PER ? ws + (((size_t)path * C::planes) * nStreamTiles + tile) * (size_t)(Hc + Tpad)
+                                            : ws + (((size_t)path * C::planes) * nStreamTiles + tile) * nTimeTiles * (size_t)bBlob;
+            const size_t bPlaneStride = PER ? (size_t)nStreamTiles * (Hc + Tpad) : (size_t)nStreamTiles * nTimeTiles * bBlob;
+            const int tau0 = Q * (PER ? C::NS : kTcM / G::E);
             for (int st = 0; st < nStages; st++) {
                 const int slot = st % kTcStages;
                 mbarWait(barEmpty + 8 * slot, (((unsigned)st / kTcStages) & 1u) ^ 1u);
-                mbarExpectTx(barFull + 8 * slot, (unsigned)kStageBytes);
+                mbarExpectTx(barFull + 8 * slot, (unsigned)G::txBytes);
                 const unsigned dst = smBase + (unsigned)slot * kStageBytes;
 #pragma unroll
                 for (int pl = 0; pl < C::planes; pl++) {
                     tmaLoad1D(dst + pl * aBlob, aSrc + ((size_t)pl * nStages + st) * aBlob, aBlob, barFull + 8 * slot);
-                    tmaLoad1D(dst + C::planes * aBlob + pl * bBlob, bSrc + pl * bPlaneStride + (size_t)(tau0 + st) * bBlob, bBlob, barFull + 8 * slot);
+                    if constexpr (PER)      // NS consecutive chunks (rows) of the stream's chunk plane, from chunk tau0 + st, at its phase
+                        tmaLoad1D(dst + C::planes * aBlob + pl * bSlot + (unsigned)((tau0 + st) & 7) * C::rowB,
+                                  bSrc + pl * bPlaneStride + (size_t)(tau0 + st) * C::rowB, bBlob, barFull + 8 * slot);
+                    else
+                        tmaLoad1D(dst + C::planes * aBlob + pl * bBlob, bSrc + pl * bPlaneStride + (size_t)(tau0 + st) * bBlob, bBlob, barFull + 8 * slot);
                 }
             }
         }
@@ -248,7 +261,8 @@ k_firtc(const __grid_constant__ FirPlan P, const FirArgs A, const unsigned char*
             mbarWait(barFull + 8 * slot, ((unsigned)st / kTcStages) & 1u);
             tcFenceAfter();
             if (electOne()) {
-                const unsigned aBase = smBase + (unsigned)slot * kStageBytes, bBase = aBase + C::planes * aBlob;
+                const unsigned aBase = smBase + (unsigned)slot * kStageBytes;
+                const unsigned bBase = aBase + C::planes * aBlob + (PER ? (unsigned)(((Q * C::NS) + st) & 7) * C::rowB : 0u);
 #pragma unroll
                 for (int ks = 0; ks < C::rowB / 32; ks++) {                   // rowB bytes of K per stage = rowB/32 MMAs of 32 B
                     if constexpr (KIND == FIRTC_I8) {
@@ -258,7 +272,11 @@ k_firtc(const __grid_constant__ FirPlan P, const FirArgs A, const unsigned char*
                             for (int j = 0; j < 4; j++) {
                                 const int s = i + j;
                                 const bool first = st == 0 && ks == 0 && i == (s > 3 ? s - 3 : 0);
-                                mma<KIND>(tmem + (unsigned)(s * C::NS), smemDesc<C::rowB>(aBase + i * aBlob + ks * 32), smemDesc<C::rowB>(bBase + j * bBlob + ks * 32),
+                                // PER: the tile starts (st & 7) rows into a swizzle atom, its rows stored at their own phase; the
+                                // swizzle follows the address bits, so the descriptor needs no base offset (measured: setting
+                                // bits 49-51 to that phase gives wrong sums, leaving them 0 gives bit-exact ones)
+                                const unsigned long long bDesc = PER ? smemDesc<C::rowB>(bBase + j * bSlot + ks * 32) : smemDesc<C::rowB>(bBase + j * bBlob + ks * 32);
+                                mma<KIND>(tmem + (unsigned)(s * C::NS), smemDesc<C::rowB>(aBase + i * aBlob + ks * 32), bDesc,
                                           instrDesc<KIND>(i == 3, j == 3), first ? 0u : 1u);
                             }
                     } else {
@@ -278,14 +296,14 @@ k_firtc(const __grid_constant__ FirPlan P, const FirArgs A, const unsigned char*
         // ===== epilogue: warps 2..5 own TMEM lane quadrants (warp % 4) =====
         const int quad = warp & 3;
         const int m = quad * 32 + lane;
-        const int o = Q * kTcM + m;
+        const int o = Q * kTcM + m;                     // (shared taps; PER maps frames per column below)
         const FirPath& d = P.paths[path];
         mbarWait(barAcc, 0);
         tcFenceAfter();
         const unsigned trow = tmem + ((unsigned)(quad * 32) << 16);
         const int s0 = tile * C::NS;
         for (int n0 = 0; n0 < C::NS; n0 += 8) {
-            if (s0 + n0 >= A.nStreams) break;               // warp-uniform
+            if (PER ? (Q * C::NS + n0) * kTcM >= A.nFrames : s0 + n0 >= A.nStreams) break;      // warp-uniform
             int res[8];
             if constexpr (KIND == FIRTC_I8) {
                 unsigned long long y[8];
@@ -308,7 +326,17 @@ k_firtc(const __grid_constant__ FirPlan P, const FirArgs A, const unsigned char*
 #pragma unroll
                 for (int k = 0; k < 8; k++) res[k] = tcFinishF(d, __int_as_float(v[k]), P.storeMask);
             }
-            if (o < A.nFrames) {
+            if constexpr (PER) {                            // N = output blocks of stream `tile`: frame 128 * block + m
+#pragma unroll
+                for (int k = 0; k < 8; k++) {
+                    const int f = (Q * C::NS + n0 + k) * kTcM + m;
+                    if (f < A.nFrames) {
+                        int* out = A.out + (size_t)tile * A.outStreamStride + (size_t)f * A.outFrameStride;
+                        for (int q = 0; q < d.nStores; q++) out[(size_t)d.storeCh[q] * A.outChStride] = res[k];
+                        if (path == 0) for (int u = 0; u < P.nUnwritten; u++) out[(size_t)P.unwritten[u] * A.outChStride] = 0;
+                    }
+                }
+            } else if (o < A.nFrames) {
 #pragma unroll
                 for (int k = 0; k < 8; k++) {
                     const int stream = s0 + n0 + k;
@@ -324,6 +352,70 @@ k_firtc(const __grid_constant__ FirPlan P, const FirArgs A, const unsigned char*
     tcFenceBefore();
     __syncthreads();
     if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"((unsigned)C::tmemCols) : "memory");
+}
+
+// ---- per-stream form: operands ------------------------------------------------------------------------------------
+// B: one chunk plane per (path, limb plane, stream): rows = 128-sample chunks of the stream's input (element e = t + Hc, delay-line
+// history in front), chunk r at r * 128 bytes, swizzled at its own phase r & 7 -- so that any NS consecutive rows copied to the
+// matching phase of a shared-memory atom form a valid SWIZZLE_128B tile (swz(128, r, b) = r * 128 + the swizzled byte)
+__global__ void __launch_bounds__(256)
+k_firtc_pack_per(const __grid_constant__ FirPlan P, const FirArgs A, unsigned char* __restrict__ ws, const int Hc, const int Tpad) {
+    const int quadsPerRow = (Hc + Tpad) / 4;
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= (long long)P.nPaths * A.nStreams * quadsPerRow) return;
+    const int q = (int)(gid % quadsPerRow);
+    const long long r = gid / quadsPerRow;
+    const int stream = (int)(r % A.nStreams), path = (int)(r / A.nStreams);
+    const FirPath& d = P.paths[path];
+    const int* in = A.in + (size_t)stream * A.inStreamStride + (size_t)(d.srcCh >= 0 ? d.srcCh : 0) * A.inChStride;
+    const int* st = A.state + (size_t)stream * P.stateWords + d.stateOff;
+    int x[4];
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        const int t = 4 * q + k - Hc;
+        x[k] = 0;
+        if (t >= 0) { if (t < A.nFrames) x[k] = tcSource<FIRTC_I8>(d, d.srcCh >= 0 ? in[(size_t)t * A.inFrameStride] : 0); }
+        else { const int si = -1 - t; if (si < d.length) x[k] = st[si]; }
+    }
+    const int e = 4 * q;
+    const size_t planeBytes = (size_t)(Hc + Tpad);
+    const unsigned off = swz(128u, (unsigned)(e >> 7), (unsigned)(e & 127));
+#pragma unroll
+    for (int pl = 0; pl < 4; pl++) {
+        unsigned char* plane = ws + (((size_t)path * 4 + pl) * A.nStreams + stream) * planeBytes;
+        const unsigned w = ((unsigned)(x[0] >> (8 * pl)) & 255u) | (((unsigned)(x[1] >> (8 * pl)) & 255u) << 8) |
+                           (((unsigned)(x[2] >> (8 * pl)) & 255u) << 16) | (((unsigned)(x[3] >> (8 * pl)) & 255u) << 24);
+        *reinterpret_cast<unsigned*>(plane + off) = w;
+    }
+}
+
+// A: every stream's own Toeplitz limb planes from its row of the FIR table, the device counterpart of firTcBuildTaps:
+// blob (stream, path, plane, stage) = [128 rows m][128 B], A[m, k] = c[m + Hc - k].  One thread: 4 consecutive k of one row.
+__global__ void __launch_bounds__(256)
+k_firtc_build_taps(const __grid_constant__ FirPlan P, const int* __restrict__ tab, const int nCols, const int nStreams, const int Hc,
+                   unsigned char* __restrict__ out) {
+    const int nStages = (Hc + kTcM) / 128;
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= (long long)nStreams * P.nPaths * nStages * kTcM * 32) return;
+    const int w = (int)(gid & 31), m = (int)((gid >> 5) % kTcM);
+    long long r = gid / (32 * kTcM);
+    const int stg = (int)(r % nStages); r /= nStages;
+    const int path = (int)(r % P.nPaths), stream = (int)(r / P.nPaths);
+    const FirPath& d = P.paths[path];
+    const int* row = tab + (size_t)stream * nCols + d.tapCol;
+    int c[4];
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        const int idx = m + Hc - (stg * 128 + 4 * w + k);
+        c[k] = (idx >= 0 && idx < d.length) ? row[idx] : 0;
+    }
+    const unsigned off = swz(128u, (unsigned)m, (unsigned)(4 * w));
+#pragma unroll
+    for (int pl = 0; pl < 4; pl++) {
+        const unsigned v = ((unsigned)(c[0] >> (8 * pl)) & 255u) | (((unsigned)(c[1] >> (8 * pl)) & 255u) << 8) |
+                           (((unsigned)(c[2] >> (8 * pl)) & 255u) << 16) | (((unsigned)(c[3] >> (8 * pl)) & 255u) << 24);
+        *reinterpret_cast<unsigned*>(out + ((((size_t)stream * P.nPaths + path) * 4 + pl) * nStages + stg) * (size_t)(kTcM * 128) + off) = v;
+    }
 }
 
 } // namespace
@@ -372,7 +464,7 @@ size_t firTcWorkspaceBytes(const FirPlan& P, int kind, int nStreams, int nFrames
 }
 
 template <int KIND>
-static cudaError_t launchFirTcT(const FirPlan& P, const FirArgs& A, const unsigned char* dTaps, unsigned char* ws, cudaStream_t stream) {
+static cudaError_t launchFirTcT_(const FirPlan& P, const FirArgs& A, const unsigned char* dTaps, unsigned char* ws, cudaStream_t stream) {
     typedef TcCfg<KIND> C;
     const int Hc = firTcHistory(P), Tpad = (A.nFrames + kTcM - 1) / kTcM * kTcM;
     const int tiles = (A.nStreams + C::NS - 1) / C::NS;
@@ -381,19 +473,55 @@ static cudaError_t launchFirTcT(const FirPlan& P, const FirArgs& A, const unsign
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     const size_t smem = (size_t)TcGeo<KIND>::stages * TcGeo<KIND>::stageBytes + 1024;
-    e = cudaFuncSetAttribute(k_firtc<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    e = cudaFuncSetAttribute(k_firtc<KIND, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     if (tiles > 65535 || P.nPaths > 65535) return cudaErrorInvalidConfiguration;
-    k_firtc<KIND><<<dim3((unsigned)(Tpad / kTcM), (unsigned)tiles, (unsigned)P.nPaths), kTcThreads, smem, stream>>>(P, A, dTaps, ws, Hc, Tpad, tiles);
+    k_firtc<KIND, false><<<dim3((unsigned)(Tpad / kTcM), (unsigned)tiles, (unsigned)P.nPaths), kTcThreads, smem, stream>>>(P, A, dTaps, ws, Hc, Tpad, tiles);
     return cudaGetLastError();
 }
 
 cudaError_t launchFirTc(const FirPlan& plan, int kind, const FirArgs& args, const unsigned char* dTaps, unsigned char* workspace,
                         cudaStream_t stream, int* launches) {
-    cudaError_t e = kind == FIRTC_I8 ? launchFirTcT<FIRTC_I8>(plan, args, dTaps, workspace, stream)
-                                     : launchFirTcT<FIRTC_TF32>(plan, args, dTaps, workspace, stream);
+    cudaError_t e = kind == FIRTC_I8 ? launchFirTcT_<FIRTC_I8>(plan, args, dTaps, workspace, stream)
+                                     : launchFirTcT_<FIRTC_TF32>(plan, args, dTaps, workspace, stream);
     if (e != cudaSuccess) return e;
     e = launchFirState(plan, args, stream);
+    if (launches) *launches = 3;
+    return e;
+}
+
+// ---- per-stream form (DSP_FORMAT 2 with a per-stream FIR table) ------------------------------------------------------
+// frames are padded to whole groups of NS = 64 output blocks (8192 frames): one CTA = 128 outputs x 64 blocks of one stream
+static int firTcPerTpad(int nFrames) { const int g = TcCfg<FIRTC_I8>::NS * kTcM; return (nFrames + g - 1) / g * g; }
+
+size_t firTcPerTapsBytes(const FirPlan& P, int nStreams) {
+    return (size_t)nStreams * P.nPaths * 4 * ((firTcHistory(P) + kTcM) / 128) * (size_t)(kTcM * 128);
+}
+size_t firTcPerWorkspaceBytes(const FirPlan& P, int nStreams, int nFrames) {
+    return (size_t)P.nPaths * 4 * nStreams * (size_t)(firTcHistory(P) + firTcPerTpad(nFrames));
+}
+cudaError_t launchFirTcBuildTaps(const FirPlan& P, const int* tab, int nCols, int nStreams, unsigned char* out, cudaStream_t stream) {
+    const long long n = (long long)nStreams * P.nPaths * ((firTcHistory(P) + kTcM) / 128) * kTcM * 32;
+    k_firtc_build_taps<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(P, tab, nCols, nStreams, firTcHistory(P), out);
+    return cudaGetLastError();
+}
+cudaError_t launchFirTcPer(const FirPlan& P, const FirArgs& A, const unsigned char* dTaps, unsigned char* ws, cudaStream_t stream, int* launches) {
+    const int Hc = firTcHistory(P), Tpad = firTcPerTpad(A.nFrames);
+    const long long quads = (long long)P.nPaths * A.nStreams * ((Hc + Tpad) / 4);
+    k_firtc_pack_per<<<(unsigned)((quads + 255) / 256), 256, 0, stream>>>(P, A, ws, Hc, Tpad);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    typedef TcGeo<FIRTC_I8, true> G;
+    const size_t smem = (size_t)G::stages * G::stageBytes + 1024;
+    e = cudaFuncSetAttribute(k_firtc<FIRTC_I8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    if (A.nStreams > 65535 || P.nPaths > 65535) return cudaErrorInvalidConfiguration;
+    // blockIdx.x fastest: the CTAs of one stream run together and read its A planes from L2
+    k_firtc<FIRTC_I8, true><<<dim3((unsigned)(Tpad / (kTcM * TcCfg<FIRTC_I8>::NS)), (unsigned)A.nStreams, (unsigned)P.nPaths), kTcThreads, smem, stream>>>(
+        P, A, dTaps, ws, Hc, Tpad, A.nStreams);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    e = launchFirState(P, A, stream);
     if (launches) *launches = 3;
     return e;
 }

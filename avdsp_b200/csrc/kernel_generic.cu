@@ -125,8 +125,9 @@ __device__ __forceinline__ typename AluT<CLS>::T saturate(typename AluT<CLS>::T 
 }
 
 struct StreamRegs { Prng g; int tpdfValue, tpdfRandom, dither; };
-// this stream's view of the per-stream coefficient table (GenericArgs::coefs): its word of column c is coefs[c * pitch]
-struct CoefRow { const int* coefs; int pitch, step; };
+// this stream's view of the per-stream tables (GenericArgs::coefs, ::firTaps), nullptr where the instance has none: its word of
+// biquad column c is coefs[c * pitch], its tap of FIR column c is fir[c]; firCol: the column of micro-op i's first tap
+struct CoefRow { const int* coefs; int pitch, step; const int* fir; const int* firCol; };
 
 // Execute ops[i0,i1) of one core for one frame.  `io` is this lane's 32-slot sample array in shared
 // memory (stride = blockDim.x), `st` its state block in HBM.
@@ -278,8 +279,9 @@ __device__ __forceinline__ void runCore(const GenericPlan& P, int i0, int i1, in
         case OP_BIQUADS: {
             SPi s = st + m.a;
             // the plan's coefficients, or this stream's row of the coefficient table: column m.c, then coefStep per section
-            const int* cf = TAB ? crow.coefs + (size_t)m.c * crow.pitch : P.pool + m.b;
-            const size_t cq = TAB ? (size_t)crow.pitch : 1, cs = TAB ? (size_t)crow.step * crow.pitch : 5;
+            const bool tab = TAB && crow.coefs;
+            const int* cf = tab ? crow.coefs + (size_t)m.c * crow.pitch : P.pool + m.b;
+            const size_t cq = tab ? (size_t)crow.pitch : 1, cs = tab ? (size_t)crow.step * crow.pitch : 5;
             if constexpr (CLS == ALU_INT64) {
                 int xn = (int)(X >> kMantBQ);
                 long long acc = 0;
@@ -322,7 +324,8 @@ __device__ __forceinline__ void runCore(const GenericPlan& P, int i0, int i1, in
                 idx++; if (idx >= m.b) idx = 0;
                 if constexpr (CLS == ALU_INT64) s[0] = idx; else s[0] = __float_as_int((float)idx);
             } else {
-                const int* taps = big + m.b;
+                // the plan's taps, or this stream's row of the FIR table (from the column of this micro-op)
+                const int* taps = (TAB && crow.fir) ? crow.fir + __ldg(crow.firCol + i) : big + m.b;
                 if constexpr (CLS == ALU_INT64) {            // intended semantics, see DESIGN.md "FIR"
                     int xn = (int)(X >> kMantBQ);
                     long long acc = 0;
@@ -488,8 +491,9 @@ __device__ __forceinline__ void runCore(const GenericPlan& P, int i0, int i1, in
 #undef IO
 }
 
-// TAB: the launch reads a per-stream coefficient table (GenericArgs::coefs).  A template argument rather than a test: the
-// interpreter reads coefficients every frame, and the plan-only instance stays exactly what it was without the table.
+// TAB: the launch reads a per-stream biquad coefficient table (GenericArgs::coefs), a per-stream FIR table (::firTaps) or both.
+// A template argument rather than a test: the interpreter reads coefficients every frame, and the plan-only instance stays
+// what it was without the tables.
 template <int CLS, bool TAB>
 __global__ void __launch_bounds__(kGenericThreads)
 k_generic(const __grid_constant__ GenericPlan P, const GenericArgs A) {
@@ -512,7 +516,8 @@ k_generic(const __grid_constant__ GenericPlan P, const GenericArgs A) {
     R.tpdfValue = aux[AUX_TPDF_VALUE]; R.tpdfRandom = aux[AUX_TPDF_RANDOM]; R.dither = aux[AUX_DITHER];
     const int* in = A.in + (size_t)s * A.inStreamStride;
     int* out = A.out + (size_t)s * A.outStreamStride;
-    const CoefRow crow{TAB ? A.coefs + s : nullptr, A.coefPitch, A.coefStep};
+    const CoefRow crow{TAB && A.coefs ? A.coefs + s : nullptr, A.coefPitch, A.coefStep,
+                       TAB && A.firTaps ? A.firTaps + (size_t)s * A.firPitch : nullptr, A.firCol};
     const int c0 = A.coreSel >= 0 ? A.coreSel : 0;
     const int c1 = A.coreSel >= 0 ? A.coreSel + 1 : P.h.nCores;
 
@@ -567,7 +572,7 @@ cudaError_t launchGeneric(const GenericPlan& plan, const GenericArgs& args, cuda
         e = cudaFuncSetAttribute(k_generic<CLS, TAB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)); \
         if (e != cudaSuccess) return e; \
         k_generic<CLS, TAB><<<blocks, threads, smem, stream>>>(plan, A); } while (0)
-#define LAUNCH_G(CLS) do { if (A.coefs) LAUNCH_G1(CLS, true); else LAUNCH_G1(CLS, false); } while (0)
+#define LAUNCH_G(CLS) do { if (A.coefs || A.firTaps) LAUNCH_G1(CLS, true); else LAUNCH_G1(CLS, false); } while (0)
     switch (plan.h.aluClass) {
     case ALU_INT64: LAUNCH_G(ALU_INT64); break;
     case ALU_F32:   LAUNCH_G(ALU_F32); break;

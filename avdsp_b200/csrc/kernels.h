@@ -21,14 +21,19 @@ struct GenericArgs {
     int coreSel;                // -1: all cores; k: only core k (0-based)  -- dspRuntime_<fmt> compat path
     int period;                 // 0: canonical order; >0: ALSA plugin order with this period
     int stageState;             // filled by launchGeneric: the CTA works on a shared-memory copy of its streams' state blocks
-    // second pass behind a float-class chain kernel (api.cu): only the streams whose flag word is set run, from the state
-    // block the snapshot holds (what the stream's state was before the chain kernel touched it)
+    // second pass behind a fused kernel (api.cu): only the streams whose flag word is set run, from the state block the
+    // snapshot holds (the state block itself behind the FIR kernels, which leave flagged streams untouched)
     const int* redo;            // [nStreams] or nullptr
     const int* snapshot;        // [nStreams][stateWords]
     // per-stream coefficient table (avdsp_b200_set_coefs) or nullptr: word [column][stream] at coefs[column * coefPitch + s]; a
     // BIQUADS micro-op's c is its first column, its sections step by coefStep (5 * the program's fs columns)
     const int* coefs;
     int coefPitch, coefStep;
+    // per-stream FIR table (avdsp_b200_set_fir_taps) or nullptr: [stream][column], the stream at position s of the call reads
+    // firTaps[s * firPitch + column]; firCol ([nOps], device): the column of FIR micro-op i's first tap (Lowered::firColOfOp)
+    const int* firTaps;
+    int firPitch;
+    const int* firCol;
     unsigned coreInMask[kMaxCores], coreOutMask[kMaxCores];
 };
 cudaError_t launchGeneric(const GenericPlan& plan, const GenericArgs& args, cudaStream_t stream);
@@ -190,6 +195,12 @@ struct FirArgs {
     int nStreams, nFrames;
     long long inStreamStride, outStreamStride;
     int inFrameStride, inChStride, outFrameStride, outChStride;
+    // per-stream FIR table (avdsp_b200_set_fir_taps) or nullptr: the stream at position p of the call convolves with
+    // taps[p * tapPitch + FirPath::tapCol ...]; skip (or nullptr): [nStreams] flag words, set for a stream the FIR kernels leave
+    // alone (float rows with a tap below 2^-60: the interpreter runs it, see launchRun)
+    const int* taps;
+    int tapPitch;
+    const int* skip;
 };
 // exact kernels: int64 accumulation (any order is exact) / float in the reference's tap order
 cudaError_t launchFir(const FirPlan& plan, const FirArgs& args, int numSMs, cudaStream_t stream, int* launches);
@@ -202,5 +213,12 @@ void firTcBuildTaps(const FirPlan& plan, int kind, const int32_t* bigPool, std::
 size_t firTcWorkspaceBytes(const FirPlan& plan, int kind, int nStreams, int nFrames);
 cudaError_t launchFirTc(const FirPlan& plan, int kind, const FirArgs& args, const unsigned char* dTaps, unsigned char* workspace,
                         cudaStream_t stream, int* launches);
+// per-stream form (FIRTC_I8, a per-stream FIR table): Toeplitz planes of every stream built on the device from the table
+// ([stream][column], nCols columns), then pack + GEMM (128 outputs x 64 output blocks of one stream per CTA) + delay lines
+size_t firTcPerTapsBytes(const FirPlan& plan, int nStreams);
+size_t firTcPerWorkspaceBytes(const FirPlan& plan, int nStreams, int nFrames);
+cudaError_t launchFirTcBuildTaps(const FirPlan& plan, const int* table, int nCols, int nStreams, unsigned char* out, cudaStream_t stream);
+cudaError_t launchFirTcPer(const FirPlan& plan, const FirArgs& args, const unsigned char* dTaps, unsigned char* workspace,
+                           cudaStream_t stream, int* launches);
 
 } // namespace avdsp

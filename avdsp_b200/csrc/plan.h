@@ -214,6 +214,7 @@ struct FirPath {
     int32_t tapsOff, length, stateOff;   // FirDesc
     int32_t flags, gainBits, satGainBits;// PF_GAIN / PF_SAT_GAIN
     int32_t nStores, storeCh[kMaxChainStores];   // OUTPUT CHANNEL numbers
+    int32_t tapCol;                      // per-stream FIR table column of the first tap at this fs (Lowered::firTapWords)
 };
 struct FirPlan {
     int32_t aluClass, nPaths, nIn, nOut;

@@ -141,21 +141,34 @@ class Executor:
         coef_words(words, fmt)) holds the coefficient words of stream first + s.  A numpy array is copied from the host; a
         contiguous int32 or float32 CUDA tensor on the instance's device is read on torch.cuda.current_stream() without a host
         sync (a tensor on another device is refused).  Float arrays are bit patterns, never value-cast."""
+        self._set_rows(self._L.avdsp_b200_set_coefs, first, values, self.n_coef, "coefficient")
+
+    def set_fir_taps(self, first: int, values):
+        """Per-stream FIR taps (avdsp_b200_set_fir_taps): row s of `values` ([n, nTaps], columns in the order of
+        fir_tap_words(words, fmt)) holds the tap words of stream first + s.  Host and device rows as for set_coefs."""
+        self._set_rows(self._L.avdsp_b200_set_fir_taps, first, values, self.n_taps, "FIR tap")
+
+    @property
+    def n_taps(self) -> int:
+        """columns of a set_fir_taps row"""
+        return len(fir_tap_words(self.words, self.fmt))
+
+    def _set_rows(self, fn, first, values, ncol, what):
         if isinstance(values, np.ndarray):
             v = self._as_words(values)
-            if v.ndim != 2 or v.shape[1] != self.n_coef:
-                raise ValueError(f"coefficient rows must be [n, {self.n_coef}], not {v.shape}")
-            _check(self._L.avdsp_b200_set_coefs(self._h, first, v.shape[0], v.ctypes.data, HOST, None))
+            if v.ndim != 2 or v.shape[1] != ncol:
+                raise ValueError(f"{what} rows must be [n, {ncol}], not {v.shape}")
+            _check(fn(self._h, first, v.shape[0], v.ctypes.data, HOST, None))
             return
         import torch
         if not (values.is_cuda and values.dtype in (torch.int32, torch.float32) and values.is_contiguous() and values.dim() == 2):
-            raise ValueError("device coefficient rows must be a contiguous 2-D int32 or float32 CUDA tensor")
-        if values.shape[1] != self.n_coef:
-            raise ValueError(f"coefficient rows must be [n, {self.n_coef}], not {tuple(values.shape)}")
+            raise ValueError(f"device {what} rows must be a contiguous 2-D int32 or float32 CUDA tensor")
+        if values.shape[1] != ncol:
+            raise ValueError(f"{what} rows must be [n, {ncol}], not {tuple(values.shape)}")
         if self.n_devices == 1 and values.device.index != self.device:
-            raise ValueError(f"device coefficient rows must be on cuda:{self.device}, not {values.device}")
+            raise ValueError(f"device {what} rows must be on cuda:{self.device}, not {values.device}")
         stream = torch.cuda.current_stream(values.device).cuda_stream
-        _check(self._L.avdsp_b200_set_coefs(self._h, first, int(values.shape[0]), values.data_ptr(), DEVICE, stream))
+        _check(fn(self._h, first, int(values.shape[0]), values.data_ptr(), DEVICE, stream))
 
     @property
     def num_variants(self) -> int:
@@ -291,6 +304,18 @@ def coef_words(words, fmt: int = 2) -> np.ndarray:
     out = np.zeros(n, dtype=np.int32)
     if n:
         _check(L.avdsp_b200_coef_words(w.ctypes.data, len(w), fmt, out.ctypes.data, n))
+    return out
+
+
+def fir_tap_words(words, fmt: int = 2) -> np.ndarray:
+    """Word indices of the program's FIR taps (every convolution entry of every DSP_FIR, every fs column), ascending, each
+    word once: the column order of Executor.set_fir_taps.  Host-only (no CUDA device needed)."""
+    w = np.ascontiguousarray(words, dtype=np.int32)
+    L = _lib.lib()
+    n = _check(L.avdsp_b200_fir_tap_words(w.ctypes.data, len(w), fmt, None, 0))
+    out = np.zeros(n, dtype=np.int32)
+    if n:
+        _check(L.avdsp_b200_fir_tap_words(w.ctypes.data, len(w), fmt, out.ctypes.data, n))
     return out
 
 

@@ -218,6 +218,45 @@ int  avdsp_b200_coef_words(const int32_t *prog, int progWords, int format, int32
  *    exact re-execution of the float class inside the same call, so every stream stays bit-exact. */
 int  avdsp_b200_set_coefs(avdsp_b200_t *, int firstStream, int nStreams, const int32_t *values, int memspace, void *cudaStream);
 
+/* Per-stream FIR taps in one launch: a room-correction impulse response per stream without a parameter variant per stream.
+ * The rules are those of the biquad coefficient table above; the two tables are independent and may coexist.
+ *
+ * Program words that are FIR taps: for every DSP_FIR opcode and EVERY sampling-frequency column whose entry is a convolution
+ * (length word lw > 0 with lw >> 16 == 0), the words t + 1 .. t + lw after its length word t.  Plain-delay entries
+ * (lw >> 16 != 0) and skipped entries (relative pointer 0) contribute nothing.  Listed once each, in ascending word order (two
+ * opcodes that point at one tap block share its words).  The list is the column order of avdsp_b200_set_fir_taps.  Host-only:
+ * validates the program like avdsp_b200_describe at EVERY rate it admits (same error codes) and needs no instance and no CUDA
+ * device.  Writes at most
+ * maxOut indices and returns the count (0: no FIR convolution in the program), or an error code. */
+int  avdsp_b200_fir_tap_words(const int32_t *prog, int progWords, int format, int32_t *wordIndex, int maxOut);
+/* Per-stream taps at batch width.  values = nStreams rows of nTaps 32-bit words, nTaps = the count avdsp_b200_fir_tap_words
+ * returns; row s holds the tap words of stream firstStream + s in that column order: Q4.28 integers for DSP_FORMAT 2, float bit
+ * patterns for the float formats.  memspace AVDSP_B200_HOST: the rows are copied before the call returns.  AVDSP_B200_DEVICE:
+ * the buffer is read in order on cudaStream (a cudaStream_t), after every launch enqueued on the instance before this call, and
+ * the host is not blocked (the first call of an instance allocates the table and may wait).
+ * The effect is exactly avdsp_b200_set_param(firstStream + s, 1, w, &row[s][col], 1) for every stream s and column col with word
+ * index w, and outputs and state are bit-identical to that; but a call still costs the launches of one parameter set, however
+ * many distinct rows there are (the FIR kernels stage each stream's taps from its row).
+ *  - The table holds nStreams x nTaps words on the device (C4, 2 x 4096 taps at one rate: 32 KB per stream).
+ *  - The first call creates the instance's FIR table.  Every stream's row starts from the words the stream runs with at that
+ *    moment: the program's, or those of its set_param variant.  avdsp_b200_num_variants does not count the table.
+ *  - The latest call wins for a word.  While a FIR table exists, set_param on tap words writes those streams' rows and creates
+ *    no variant; set_param on any other word makes variants as before, and they combine with the rows.
+ *  - reload_params drops the table.  reset keeps it: rows hold every fs column, so a reset to another rate runs that rate's taps.
+ *  - Refusals change nothing: AVDSP_B200_ERR_UNSUPPORTED for a program without FIR taps, for DEVICE rows on a multi-device
+ *    instance (HOST rows are split over its shards), and for a variant that changed a tap block's length; AVDSP_B200_ERR_ARG for
+ *    a bad stream range, NULL values or an unknown memspace.
+ *  - Kernels, DSP_FORMAT 2: the tensor-core FIR kernel runs per stream (bit-exact, as with shared taps); AUTO takes it for calls
+ *    of at least 8192 frames, k_fir for shorter ones.  It keeps every stream's Toeplitz limb planes on the device, built from the
+ *    rows before its first launch after they change: nStreams x paths x 4 x ((longest impulse rounded up to 128) / 128 + 1) x
+ *    16 KB (C4, 2 x 4096 taps: 4.3 MB per stream, 4.4 GB for 1024 streams).  When they cannot be allocated the instance runs
+ *    k_fir with its table (and says so in avdsp_b200_trace).  DSP_FORMAT 3: k_fir; AVDSP_B200_KERNEL_FIR_TC (the 3xTF32 form
+ *    contracts with taps every stream shares) returns AVDSP_B200_ERR_UNSUPPORTED while a FIR table exists.
+ *  - DSP_FORMAT 3: a row with a non-zero tap below 2^-60 (any fs column) sends its stream through the interpreter inside the same
+ *    call, so every stream stays bit-exact (the FIR kernels' products could come near 2^-126, where they differ from the
+ *    reference's multiply). */
+int  avdsp_b200_set_fir_taps(avdsp_b200_t *, int firstStream, int nStreams, const int32_t *values, int memspace, void *cudaStream);
+
 /* Per-stream state block, int32 words:  [0,dataSize) = the reference data area, same word offsets
  * (runtime/dsp_runtime.c:137-141);  then 8 aux words (xoshiro s0..s3, tpdfValue, tpdfRandom, current
  * global dither, pad -- the reference's process globals, runtime/dsp_tpdf.h:11-33);  then the 64-bit
