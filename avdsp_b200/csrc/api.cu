@@ -281,6 +281,12 @@ static int initState(avdsp_b200* h) {
     return 0;
 }
 
+static void freeTable(StreamTable& t) {
+    if (t.d) cudaFree(t.d);
+    if (t.dStage) cudaFree(t.dStage);
+    t.d = t.dStage = nullptr; t.stageWords = 0;
+}
+
 static void freeAll(avdsp_b200* h) {
     if (!h) return;
     for (auto& kv : h->hostAllocs) { cudaHostUnregister(kv.first); hostFreePlaced(kv.first, kv.second); }
@@ -308,9 +314,8 @@ static void freeAll(avdsp_b200* h) {
     if (h->dRedoCount) cudaFree(h->dRedoCount);
     if (h->dFirTaps) cudaFree(h->dFirTaps);
     if (h->dFirWs) cudaFree(h->dFirWs);
-    if (h->dCoef) cudaFree(h->dCoef);
-    if (h->dCoefStage) cudaFree(h->dCoefStage);
-    if (h->dFirTab) cudaFree(h->dFirTab);
+    freeTable(h->coefTab);
+    freeTable(h->firTab);
     if (h->dFirFlags) cudaFree(h->dFirFlags);
     if (h->dFirTcPer) cudaFree(h->dFirTcPer);
     if (h->pcmRaw) cudaFree(h->pcmRaw);
@@ -481,9 +486,9 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         outSS = (long long)cap * nOut; outFS = 1; outCS = cap;
     } else return setErr(AVDSP_B200_ERR_ARG, "unknown layout");
     int* st = h->dState + (size_t)first * P.stateWords;
-    const int* coefs = h->dCoef ? h->dCoef + first : nullptr;     // per-stream coefficient table, positioned like the state blocks
+    const int* coefs = h->coefTab.d ? h->coefTab.d + first : nullptr;     // per-stream coefficient table, positioned like the state blocks
     const int nTapCols = (int)h->L.firTapWords.size();
-    const int* firTaps = h->dFirTab ? h->dFirTab + (size_t)first * nTapCols : nullptr;      // ... and the FIR table
+    const int* firTaps = h->firTab.d ? h->firTab.d + (size_t)first * nTapCols : nullptr;      // ... and the FIR table
     if (ordered) CU(cudaStreamWaitEvent(stream, h->evLast, 0));          // stream-ordered after the instance's previous launch (see evLast)
     // the fused kernels run the canonical order; a plugin-order request may use them when the two orders provably agree
     const bool chainOrder = (h->period == 0 || pl->L.orderIndependent) && coreSel < 0 && !planOverride;
@@ -542,7 +547,7 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         int nl = 0;
         if (use == AVDSP_B200_KERNEL_FIR_TC && firTaps) {
             if (!h->firTcPerValid) {                              // rows changed since the planes were built: all streams again
-                e = launchFirTcBuildTaps(h->L.fir, h->dFirTab, nTapCols, h->nStreams, h->dFirTcPer, stream);
+                e = launchFirTcBuildTaps(h->L.fir, h->firTab.d, nTapCols, h->nStreams, h->dFirTcPer, stream);
                 if (e != cudaSuccess) return cudaErr(e, "kernel launch");
                 h->firTcPerValid = true;
                 h->launches++;
@@ -750,10 +755,14 @@ static int launchRange(avdsp_b200* h, const int* in, int* out, int nFrames, int 
     return 0;
 }
 
-// the FIR table's exactness flags of streams [first, first+n), on `s` after the rows were written there (float programs only)
-static int firTapFlags(avdsp_b200* h, int first, int n, cudaStream_t s) {
-    if (!h->dFirFlags || n == 0) return 0;
-    k_fir_tap_flags<<<(unsigned)((n + 7) / 8), 256, 0, s>>>(h->dFirTab, (int)h->L.firTapWords.size(), first, n, h->dFirFlags);
+// What follows a write of rows [first, first + n) of a table, on `s` after the write.  Only the FIR table has data derived from
+// its rows: the per-stream Toeplitz planes are stale, and float programs recompute those streams' exactness flags.
+static int rowsChanged(avdsp_b200* h, StreamTable avdsp_b200::* tab, int first, int n, cudaStream_t s) {
+    if (tab != &avdsp_b200::firTab) return 0;
+    h->firTcPerValid = false;
+    if (h->L.gen.h.aluClass != ALU_F32) return 0;
+    if (!h->dFirFlags) CU(cudaMalloc(&h->dFirFlags, (size_t)h->nStreams * 4));
+    k_fir_tap_flags<<<(unsigned)((n + 7) / 8), 256, 0, s>>>(h->firTab.d, (int)h->L.firTapWords.size(), first, n, h->dFirFlags);
     CU(cudaGetLastError());
     h->launches++;
     return 0;
@@ -1090,6 +1099,110 @@ static int variantFor(avdsp_b200* h, const std::vector<int32_t>& words, int* id)
     return 0;
 }
 
+// ---- per-stream tables (StreamTable, instance.h): the biquad coefficient table and the FIR table ---------------------
+// A table's column list for a program.  The list does not depend on the rate: lower at the lowest one the header admits
+// (decodeProgram validates it).  allRates: the program must also lower at every other rate it admits, as describe would check
+// each of them.
+static int tableWords(std::vector<int32_t> Lowered::* list, bool allRates, const int32_t* prog, int progWords, int format,
+                      int32_t* wordIndex, int maxOut) {
+    if (maxOut < 0 || (maxOut > 0 && !wordIndex)) return setErr(AVDSP_B200_ERR_ARG, "bad output buffer");
+    const int fi = (prog && progWords > H_FREQMIN) ? prog[H_FREQMIN] : 0;
+    const int fs = (fi >= 0 && fi < kNumFreq) ? kFreqTable[fi] : 0;
+    std::unique_ptr<Lowered> L(new Lowered);
+    std::string err;
+    int rc = decodeProgram(prog, progWords, 0x7FFFFFFF, format, fs, 31, L.get(), &err);
+    if (rc < 0) return setErr(rc, err);
+    if (allRates) {
+        std::unique_ptr<Lowered> Lr(new Lowered);
+        for (int f = fi + 1; f <= prog[H_FREQMAX] && f < kNumFreq; f++) {
+            rc = decodeProgram(prog, progWords, 0x7FFFFFFF, format, kFreqTable[f], 31, Lr.get(), &err);
+            if (rc < 0) return setErr(rc, err);
+        }
+    }
+    const std::vector<int32_t>& w = (*L).*list;
+    const int n = (int)w.size();
+    for (int k = 0; k < n && k < maxOut; k++) wordIndex[k] = w[k];
+    return n;
+}
+
+// A table, created on first use: every stream's row holds the words it runs with now (the program's, or its variant's).
+// Synchronous: the table is not in use yet.
+static int ensureTable(avdsp_b200* h, StreamTable avdsp_b200::* tab) {
+    StreamTable& t = h->*tab;
+    if (t.d) return 0;
+    const std::vector<int32_t>& cols = h->L.*t.words;
+    const size_t N = (size_t)h->nStreams, nc = cols.size(), ss = t.streamStride(nc), cs = t.colStride(N);
+    std::vector<int32_t> init(nc * N);
+    for (size_t s = 0; s < N; s++) {
+        const int v = h->variantOf.empty() ? 0 : h->variantOf[s];
+        const std::vector<int32_t>& w = v ? h->variants[v - 1]->L.words : h->L.words;
+        for (size_t c = 0; c < nc; c++) init[s * ss + c * cs] = w[cols[c]];
+    }
+    int* d = nullptr;
+    CU(cudaMalloc(&d, init.size() * 4));
+    t.d = d;
+    cudaError_t e = cudaMemcpyAsync(d, init.data(), init.size() * 4, cudaMemcpyHostToDevice, h->stream);
+    int r = e == cudaSuccess ? rowsChanged(h, tab, 0, h->nStreams, h->stream) : cudaErr(e, "table upload");
+    if (r >= 0 && (e = cudaStreamSynchronize(h->stream)) != cudaSuccess) r = cudaErr(e, "table upload");
+    if (r < 0) { cudaFree(d); t.d = nullptr; }
+    return r;
+}
+
+// Rows [nStreams][columns] for streams [firstStream, firstStream + nStreams) of a table, from HOST or DEVICE memory, in the
+// instance's stream order.  refusal: why this program can have no such table (nullptr: it can).  A refused call changes nothing.
+static int setRows(avdsp_b200* h, StreamTable avdsp_b200::* tab, const char* refusal, int firstStream, int nStreams,
+                   const int32_t* values, int memspace, void* cudaStream) {
+    if (!h || !values) return setErr(AVDSP_B200_ERR_ARG, "NULL argument");
+    if (firstStream < 0 || nStreams < 0 || (long long)firstStream + nStreams > h->nStreams) return setErr(AVDSP_B200_ERR_ARG, "bad stream range");
+    if (memspace != AVDSP_B200_HOST && memspace != AVDSP_B200_DEVICE) return setErr(AVDSP_B200_ERR_ARG, "unknown memspace");
+    StreamTable& t = h->*tab;
+    const std::vector<int32_t>& cols = h->L.*t.words;
+    const int nCols = (int)cols.size();
+    if (nCols == 0) return setErr(AVDSP_B200_ERR_UNSUPPORTED, std::string("the program has no ") + t.noun + " words");
+    if (refusal) return setErr(AVDSP_B200_ERR_UNSUPPORTED, refusal);
+    if (!h->shards.empty() && memspace != AVDSP_B200_HOST)
+        return setErr(AVDSP_B200_ERR_UNSUPPORTED, std::string("a multi-device instance takes HOST ") + t.noun + " rows (device buffers belong to one GPU)");
+    for (const avdsp_b200* o : h->shards.empty() ? std::vector<avdsp_b200*>{h} : h->shards)
+        for (const avdsp_b200* v : o->variants)
+            if (v->L.*t.words != cols) return setErr(AVDSP_B200_ERR_UNSUPPORTED, std::string("a parameter variant moved the ") + t.noun + " words");
+    if (!h->shards.empty())
+        return forShards(h, [&](int k, avdsp_b200* sh) {
+            const int a = std::max(firstStream, h->shardFirst[k]), b = std::min(firstStream + nStreams, h->shardFirst[k + 1]);
+            if (b <= a) return 0;
+            return setRows(sh, tab, refusal, a - h->shardFirst[k], b - a, values + (size_t)(a - firstStream) * nCols, AVDSP_B200_HOST, nullptr);
+        });
+    if (nStreams == 0) return 0;
+    CU(cudaSetDevice(h->device));
+    { const int r = ensureTable(h, tab); if (r < 0) return r; }
+    const cudaStream_t s = memspace == AVDSP_B200_DEVICE ? (cudaStream_t)cudaStream : h->stream;
+    const size_t words = (size_t)nStreams * nCols;
+    CU(cudaStreamWaitEvent(s, h->evLast, 0));                 // after every launch enqueued on the instance before this call
+    if (t.streamMajor) {                                      // rows arrive in the table's own layout: one copy
+        CU(cudaMemcpyAsync(t.d + (size_t)firstStream * nCols, values, words * 4,
+                           memspace == AVDSP_B200_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, s));
+    } else {
+        const int* rows = values;
+        if (memspace == AVDSP_B200_HOST) {
+            if (words > t.stageWords) {
+                CU(cudaStreamSynchronize(s));
+                if (t.dStage) cudaFree(t.dStage);
+                t.dStage = nullptr; t.stageWords = 0;
+                CU(cudaMalloc(&t.dStage, words * 4));
+                t.stageWords = words;
+            }
+            CU(cudaMemcpyAsync(t.dStage, values, words * 4, cudaMemcpyHostToDevice, s));
+            rows = t.dStage;
+        }
+        k_coef_scatter<<<dim3((unsigned)((nStreams + 31) / 32), (unsigned)((nCols + 31) / 32)), dim3(32, 8), 0, s>>>(t.d, h->nStreams, firstStream, nStreams, nCols, rows);
+        CU(cudaGetLastError());
+        h->launches++;
+    }
+    { const int r = rowsChanged(h, tab, firstStream, nStreams, s); if (r < 0) return r; }
+    CU(cudaEventRecord(h->evLast, s));
+    if (memspace == AVDSP_B200_HOST) CU(cudaStreamSynchronize(s));    // the caller's buffer (and the staging rows) are free again
+    return 0;
+}
+
 extern "C" {
 
 int avdsp_b200_param_index(const avdsp_b200_t* h, int offset, int paramNum) {
@@ -1125,22 +1238,21 @@ int avdsp_b200_set_param(avdsp_b200_t* h, int firstStream, int nStreams, int wor
         return 0;
     }
     { const int q = quiesce(h); if (q < 0) return q; }
-    // while the instance has a coefficient table (a FIR table), coefficient words (tap words) are written into the streams' rows;
-    // the other words make variants as without one.  Everything that can fail (lowering a variant) happens before anything changes.
-    const std::vector<int32_t>& cw = h->L.coefWords;
-    const std::vector<int32_t>& tw = h->L.firTapWords;
-    auto columns = [&](bool on, const std::vector<int32_t>& list) {      // table column of word k of the call, or -1
-        std::vector<int> col(nWords, -1);
-        if (on)
-            for (int k = 0; k < nWords; k++) {
-                const auto it = std::lower_bound(list.begin(), list.end(), wordIndex + k);
-                if (it != list.end() && *it == wordIndex + k) col[k] = (int)(it - list.begin());
-            }
-        return col;
-    };
-    const std::vector<int> colOf = columns(h->dCoef != nullptr, cw), tapColOf = columns(h->dFirTab != nullptr, tw);
-    bool anyVariantWord = false;
-    for (int k = 0; k < nWords; k++) anyVariantWord = anyVariantWord || (colOf[k] < 0 && tapColOf[k] < 0);
+    // while the instance has a table, the words it holds are written into the streams' rows; the other words make variants as
+    // without one.  Everything that can fail (lowering a variant) happens before anything changes.
+    const decltype(&avdsp_b200::coefTab) tables[] = {&avdsp_b200::coefTab, &avdsp_b200::firTab};
+    std::vector<int> colOf[2];                // table column of word k of the call, or -1
+    std::vector<char> tableWord(nWords, 0);
+    for (int t = 0; t < 2; t++) {
+        colOf[t].assign(nWords, -1);
+        if (!(h->*tables[t]).d) continue;
+        const std::vector<int32_t>& list = h->L.*(h->*tables[t]).words;
+        for (int k = 0; k < nWords; k++) {
+            const auto it = std::lower_bound(list.begin(), list.end(), wordIndex + k);
+            if (it != list.end() && *it == wordIndex + k) { colOf[t][k] = (int)(it - list.begin()); tableWord[k] = 1; }
+        }
+    }
+    const bool anyVariantWord = std::count(tableWord.begin(), tableWord.end(), 0) > 0;
     // streams of the range may sit on different variants already: patch each of those once
     std::map<int, int> moved;                 // old variant -> new variant
     if (anyVariantWord) {
@@ -1153,40 +1265,33 @@ int avdsp_b200_set_param(avdsp_b200_t* h, int firstStream, int nStreams, int wor
             const int old = h->variantOf.empty() ? 0 : h->variantOf[s];
             if (moved.count(old)) continue;
             std::vector<int32_t> words = old ? h->variants[old - 1]->L.words : h->L.words;
-            for (int k = 0; k < nWords; k++) if (colOf[k] < 0 && tapColOf[k] < 0) words[wordIndex + k] = values[k];
+            for (int k = 0; k < nWords; k++) if (!tableWord[k]) words[wordIndex + k] = values[k];
             int id = 0;
             const int r = variantFor(h, words, &id);
             if (r < 0) return undo(r);
-            if (h->dCoef && id > 0 && h->variants[id - 1]->L.coefWords != cw)
-                return undo(setErr(AVDSP_B200_ERR_UNSUPPORTED, "this change moves biquad coefficient words the coefficient table holds (section count)"));
-            if (h->dFirTab && id > 0 && h->variants[id - 1]->L.firTapWords != tw)
-                return undo(setErr(AVDSP_B200_ERR_UNSUPPORTED, "this change moves FIR tap words the FIR table holds (tap block length)"));
+            for (auto tab : tables) {
+                const StreamTable& t = h->*tab;
+                if (t.d && id > 0 && h->variants[id - 1]->L.*t.words != h->L.*t.words)
+                    return undo(setErr(AVDSP_B200_ERR_UNSUPPORTED, std::string("this change moves ") + t.noun + " words the table holds"));
+            }
             moved.emplace(old, id);
         }
     }
-    if (h->dCoef) {
-        std::vector<int32_t> col((size_t)nStreams);
-        for (int k = 0; k < nWords; k++) {
-            if (colOf[k] < 0) continue;
-            std::fill(col.begin(), col.end(), values[k]);
-            CU(cudaMemcpyAsync(h->dCoef + (size_t)colOf[k] * h->nStreams + firstStream, col.data(), col.size() * 4,
-                               cudaMemcpyHostToDevice, h->stream));
-            CU(cudaStreamSynchronize(h->stream));
-        }
-        CU(cudaEventRecord(h->evLast, h->stream));
-    }
-    if (h->dFirTab) {
+    for (int t = 0; t < 2; t++) {
+        StreamTable& tab = h->*tables[t];
+        if (!tab.d) continue;
+        const size_t ss = tab.streamStride((h->L.*tab.words).size()), cs = tab.colStride(h->nStreams);
         bool any = false;
         std::vector<int32_t> col((size_t)nStreams);
         for (int k = 0; k < nWords; k++) {
-            if (tapColOf[k] < 0) continue;
-            std::fill(col.begin(), col.end(), values[k]);       // one word of every row of the range: a strided copy
-            CU(cudaMemcpy2DAsync(h->dFirTab + (size_t)firstStream * tw.size() + tapColOf[k], tw.size() * 4, col.data(), 4, 4, (size_t)nStreams,
+            if (colOf[t][k] < 0) continue;
+            std::fill(col.begin(), col.end(), values[k]);       // one word of every row of the range
+            CU(cudaMemcpy2DAsync(tab.d + firstStream * ss + colOf[t][k] * cs, ss * 4, col.data(), 4, 4, (size_t)nStreams,
                                  cudaMemcpyHostToDevice, h->stream));
             CU(cudaStreamSynchronize(h->stream));
             any = true;
         }
-        if (any) { const int r = firTapFlags(h, firstStream, nStreams, h->stream); if (r < 0) return r; h->firTcPerValid = false; }
+        if (any) { const int r = rowsChanged(h, tables[t], firstStream, nStreams, h->stream); if (r < 0) return r; }
         CU(cudaEventRecord(h->evLast, h->stream));
     }
     if (!anyVariantWord) return 0;
@@ -1209,168 +1314,21 @@ int avdsp_b200_set_param(avdsp_b200_t* h, int firstStream, int nStreams, int wor
 }
 
 int avdsp_b200_coef_words(const int32_t* prog, int progWords, int format, int32_t* wordIndex, int maxOut) {
-    if (maxOut < 0 || (maxOut > 0 && !wordIndex)) return setErr(AVDSP_B200_ERR_ARG, "bad output buffer");
-    // the column list does not depend on the rate: lower at the lowest one the header admits (decodeProgram validates it)
-    const int fi = (prog && progWords > H_FREQMIN) ? prog[H_FREQMIN] : 0;
-    const int fs = (fi >= 0 && fi < kNumFreq) ? kFreqTable[fi] : 0;
-    std::unique_ptr<Lowered> L(new Lowered);
-    std::string err;
-    const int rc = decodeProgram(prog, progWords, 0x7FFFFFFF, format, fs, 31, L.get(), &err);
-    if (rc < 0) return setErr(rc, err);
-    const int n = (int)L->coefWords.size();
-    for (int k = 0; k < n && k < maxOut; k++) wordIndex[k] = L->coefWords[k];
-    return n;
-}
-
-// The instance's coefficient table, created on first use: every stream's row holds the words it runs with now (the program's, or
-// its variant's).  Synchronous: the table is not in use yet.
-static int ensureCoefTable(avdsp_b200* h) {
-    if (h->dCoef) return 0;
-    const std::vector<int32_t>& cw = h->L.coefWords;
-    const size_t N = (size_t)h->nStreams, nc = cw.size();
-    std::vector<int32_t> init(nc * N);
-    for (size_t s = 0; s < N; s++) {
-        const int v = h->variantOf.empty() ? 0 : h->variantOf[s];
-        const std::vector<int32_t>& w = v ? h->variants[v - 1]->L.words : h->L.words;
-        for (size_t c = 0; c < nc; c++) init[c * N + s] = w[cw[c]];
-    }
-    int* d = nullptr;
-    CU(cudaMalloc(&d, init.size() * 4));
-    const cudaError_t e = cudaMemcpyAsync(d, init.data(), init.size() * 4, cudaMemcpyHostToDevice, h->stream);
-    const cudaError_t e2 = e == cudaSuccess ? cudaStreamSynchronize(h->stream) : e;
-    if (e2 != cudaSuccess) { cudaFree(d); return cudaErr(e2, "coefficient table upload"); }
-    h->dCoef = d;
-    return 0;
+    return tableWords(&Lowered::coefWords, false, prog, progWords, format, wordIndex, maxOut);
 }
 
 int avdsp_b200_set_coefs(avdsp_b200_t* h, int firstStream, int nStreams, const int32_t* values, int memspace, void* cudaStream) {
-    if (!h || !values) return setErr(AVDSP_B200_ERR_ARG, "NULL argument");
-    if (firstStream < 0 || nStreams < 0 || (long long)firstStream + nStreams > h->nStreams) return setErr(AVDSP_B200_ERR_ARG, "bad stream range");
-    if (memspace != AVDSP_B200_HOST && memspace != AVDSP_B200_DEVICE) return setErr(AVDSP_B200_ERR_ARG, "unknown memspace");
-    const int nCoef = (int)h->L.coefWords.size();
-    if (nCoef == 0) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "the program has no biquad coefficients");
-    if (!h->L.coefTableOk) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "biquad parameter blocks of this program overlap: no coefficient table");
-    if (!h->shards.empty()) {
-        if (memspace != AVDSP_B200_HOST) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a multi-device instance takes HOST coefficient rows (device buffers belong to one GPU)");
-        for (const avdsp_b200* sh : h->shards)
-            for (const avdsp_b200* v : sh->variants)
-                if (v->L.coefWords != h->L.coefWords) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a parameter variant moved the biquad coefficient words (section count)");
-        return forShards(h, [&](int k, avdsp_b200* sh) {
-            const int a = std::max(firstStream, h->shardFirst[k]), b = std::min(firstStream + nStreams, h->shardFirst[k + 1]);
-            if (b <= a) return 0;
-            return avdsp_b200_set_coefs(sh, a - h->shardFirst[k], b - a, values + (size_t)(a - firstStream) * nCoef, AVDSP_B200_HOST, nullptr);
-        });
-    }
-    for (const avdsp_b200* v : h->variants)
-        if (v->L.coefWords != h->L.coefWords) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a parameter variant moved the biquad coefficient words (section count)");
-    if (nStreams == 0) return 0;
-    CU(cudaSetDevice(h->device));
-    { const int r = ensureCoefTable(h); if (r < 0) return r; }
-    const cudaStream_t s = memspace == AVDSP_B200_DEVICE ? (cudaStream_t)cudaStream : h->stream;
-    const size_t words = (size_t)nStreams * nCoef;
-    CU(cudaStreamWaitEvent(s, h->evLast, 0));                 // after every launch enqueued on the instance before this call
-    const int* rows = values;
-    if (memspace == AVDSP_B200_HOST) {
-        if (words > h->coefStageWords) {
-            CU(cudaStreamSynchronize(s));
-            if (h->dCoefStage) cudaFree(h->dCoefStage);
-            h->dCoefStage = nullptr; h->coefStageWords = 0;
-            CU(cudaMalloc(&h->dCoefStage, words * 4));
-            h->coefStageWords = words;
-        }
-        CU(cudaMemcpyAsync(h->dCoefStage, values, words * 4, cudaMemcpyHostToDevice, s));
-        rows = h->dCoefStage;
-    }
-    k_coef_scatter<<<dim3((unsigned)((nStreams + 31) / 32), (unsigned)((nCoef + 31) / 32)), dim3(32, 8), 0, s>>>(h->dCoef, h->nStreams, firstStream, nStreams, nCoef, rows);
-    CU(cudaGetLastError());
-    h->launches++;
-    CU(cudaEventRecord(h->evLast, s));
-    if (memspace == AVDSP_B200_HOST) CU(cudaStreamSynchronize(s));    // the caller's buffer (and the staging rows) are free again
-    return 0;
+    const char* overlap = h && !h->L.coefTableOk ? "biquad parameter blocks of this program overlap: no coefficient table" : nullptr;
+    return setRows(h, &avdsp_b200::coefTab, overlap, firstStream, nStreams, values, memspace, cudaStream);
 }
 
+// validated at every rate the program admits, as the header states (avdsp_b200_coef_words: at the lowest one)
 int avdsp_b200_fir_tap_words(const int32_t* prog, int progWords, int format, int32_t* wordIndex, int maxOut) {
-    if (maxOut < 0 || (maxOut > 0 && !wordIndex)) return setErr(AVDSP_B200_ERR_ARG, "bad output buffer");
-    // the column list does not depend on the rate: lower at the lowest one the header admits (decodeProgram validates it)
-    const int fi = (prog && progWords > H_FREQMIN) ? prog[H_FREQMIN] : 0;
-    const int fs = (fi >= 0 && fi < kNumFreq) ? kFreqTable[fi] : 0;
-    std::unique_ptr<Lowered> L(new Lowered);
-    std::string err;
-    int rc = decodeProgram(prog, progWords, 0x7FFFFFFF, format, fs, 31, L.get(), &err);
-    if (rc < 0) return setErr(rc, err);
-    // the list covers every fs column: the program must lower at every rate it admits, as describe would check each of them
-    std::unique_ptr<Lowered> Lr(new Lowered);
-    for (int f = fi + 1; f <= prog[H_FREQMAX] && f < kNumFreq; f++) {
-        rc = decodeProgram(prog, progWords, 0x7FFFFFFF, format, kFreqTable[f], 31, Lr.get(), &err);
-        if (rc < 0) return setErr(rc, err);
-    }
-    const int n = (int)L->firTapWords.size();
-    for (int k = 0; k < n && k < maxOut; k++) wordIndex[k] = L->firTapWords[k];
-    return n;
-}
-
-// The instance's FIR table, created on first use: every stream's row holds the tap words it runs with now (the program's, or
-// its variant's).  Float programs get the exactness flags with it.  Synchronous: the table is not in use yet.
-static int ensureFirTable(avdsp_b200* h) {
-    if (h->dFirTab) return 0;
-    const std::vector<int32_t>& tw = h->L.firTapWords;
-    const size_t N = (size_t)h->nStreams, nt = tw.size();
-    std::vector<int32_t> init(nt * N);
-    for (size_t s = 0; s < N; s++) {
-        const int v = h->variantOf.empty() ? 0 : h->variantOf[s];
-        const std::vector<int32_t>& w = v ? h->variants[v - 1]->L.words : h->L.words;
-        for (size_t c = 0; c < nt; c++) init[s * nt + c] = w[tw[c]];
-    }
-    int* d = nullptr;
-    int* f = nullptr;
-    auto fail = [&](cudaError_t e) { if (d) cudaFree(d); if (f) cudaFree(f); return cudaErr(e, "FIR table upload"); };
-    cudaError_t e = cudaMalloc(&d, init.size() * 4);
-    if (e != cudaSuccess) { d = nullptr; return fail(e); }
-    if (h->L.gen.h.aluClass == ALU_F32) {
-        e = cudaMalloc(&f, N * 4);
-        if (e != cudaSuccess) { f = nullptr; return fail(e); }
-    }
-    e = cudaMemcpyAsync(d, init.data(), init.size() * 4, cudaMemcpyHostToDevice, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    if (e != cudaSuccess) return fail(e);
-    h->dFirTab = d; h->dFirFlags = f;
-    { const int r = firTapFlags(h, 0, h->nStreams, h->stream); if (r < 0) return r; }
-    CU(cudaStreamSynchronize(h->stream));
-    return 0;
+    return tableWords(&Lowered::firTapWords, true, prog, progWords, format, wordIndex, maxOut);
 }
 
 int avdsp_b200_set_fir_taps(avdsp_b200_t* h, int firstStream, int nStreams, const int32_t* values, int memspace, void* cudaStream) {
-    if (!h || !values) return setErr(AVDSP_B200_ERR_ARG, "NULL argument");
-    if (firstStream < 0 || nStreams < 0 || (long long)firstStream + nStreams > h->nStreams) return setErr(AVDSP_B200_ERR_ARG, "bad stream range");
-    if (memspace != AVDSP_B200_HOST && memspace != AVDSP_B200_DEVICE) return setErr(AVDSP_B200_ERR_ARG, "unknown memspace");
-    const int nTaps = (int)h->L.firTapWords.size();
-    if (nTaps == 0) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "the program has no FIR taps");
-    if (!h->shards.empty()) {
-        if (memspace != AVDSP_B200_HOST) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a multi-device instance takes HOST FIR rows (device buffers belong to one GPU)");
-        for (const avdsp_b200* sh : h->shards)
-            for (const avdsp_b200* v : sh->variants)
-                if (v->L.firTapWords != h->L.firTapWords) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a parameter variant moved the FIR tap words (tap block length)");
-        return forShards(h, [&](int k, avdsp_b200* sh) {
-            const int a = std::max(firstStream, h->shardFirst[k]), b = std::min(firstStream + nStreams, h->shardFirst[k + 1]);
-            if (b <= a) return 0;
-            return avdsp_b200_set_fir_taps(sh, a - h->shardFirst[k], b - a, values + (size_t)(a - firstStream) * nTaps, AVDSP_B200_HOST, nullptr);
-        });
-    }
-    for (const avdsp_b200* v : h->variants)
-        if (v->L.firTapWords != h->L.firTapWords) return setErr(AVDSP_B200_ERR_UNSUPPORTED, "a parameter variant moved the FIR tap words (tap block length)");
-    if (nStreams == 0) return 0;
-    CU(cudaSetDevice(h->device));
-    { const int r = ensureFirTable(h); if (r < 0) return r; }
-    const cudaStream_t s = memspace == AVDSP_B200_DEVICE ? (cudaStream_t)cudaStream : h->stream;
-    CU(cudaStreamWaitEvent(s, h->evLast, 0));                 // after every launch enqueued on the instance before this call
-    // rows arrive [stream][column], the table's own layout: one copy
-    CU(cudaMemcpyAsync(h->dFirTab + (size_t)firstStream * nTaps, values, (size_t)nStreams * nTaps * 4,
-                       memspace == AVDSP_B200_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, s));
-    { const int r = firTapFlags(h, firstStream, nStreams, s); if (r < 0) return r; }
-    h->firTcPerValid = false;
-    CU(cudaEventRecord(h->evLast, s));
-    if (memspace == AVDSP_B200_HOST) CU(cudaStreamSynchronize(s));    // the caller's buffer is free again
-    return 0;
+    return setRows(h, &avdsp_b200::firTab, nullptr, firstStream, nStreams, values, memspace, cudaStream);
 }
 
 int avdsp_b200_num_variants(const avdsp_b200_t* h) {
@@ -1391,8 +1349,8 @@ int avdsp_b200_reload_params(avdsp_b200_t* h, const int32_t* prog, int progWords
     }
     { const int q = quiesce(h); if (q < 0) return q; }
     dropVariants(h);                                          // a new program for everybody: per-stream overrides start over
-    if (h->dCoef) { cudaFree(h->dCoef); h->dCoef = nullptr; }   // ... the coefficient table too
-    if (h->dFirTab) { cudaFree(h->dFirTab); h->dFirTab = nullptr; }      // ... and the FIR table
+    freeTable(h->coefTab);                                    // ... the tables too
+    freeTable(h->firTab);
     if (h->dFirFlags) { cudaFree(h->dFirFlags); h->dFirFlags = nullptr; }
     if (h->dFirTcPer) { cudaFree(h->dFirTcPer); h->dFirTcPer = nullptr; }
     h->firTcPerValid = h->firTcPerFailed = false;

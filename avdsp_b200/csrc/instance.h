@@ -8,6 +8,19 @@
 #include "decoder.h"
 #include "kernels.h"
 
+// A per-stream table of program words (avdsp_b200_set_coefs, avdsp_b200_set_fir_taps): one row per stream, column c holds
+// word (L.*words)[c]; d == nullptr: none.  Variants (set_param on other words) keep their own plans and read the same table.
+struct StreamTable {
+    decltype(&avdsp::Lowered::coefWords) words;     // the column list: &Lowered::coefWords or &Lowered::firTapWords
+    bool streamMajor;           // [stream][column] (rows arrive in this layout: one copy), else [column][stream]
+    const char* noun;           // what a column holds, for messages
+    int* d = nullptr;
+    int* dStage = nullptr; size_t stageWords = 0;   // [column][stream]: HOST rows on their way to the table
+    // word (stream s, column c) lives at d[s * streamStride + c * colStride]
+    size_t streamStride(size_t nCols) const { return streamMajor ? nCols : 1; }
+    size_t colStride(size_t nStreams) const { return streamMajor ? 1 : nStreams; }
+};
+
 struct avdsp_b200 {
     int device = 0, numSMs = 148;
     int nStreams = 0;
@@ -66,14 +79,12 @@ struct avdsp_b200 {
     cudaStream_t varStream[kVarStreams] = {};
     cudaEvent_t varEv[kVarStreams] = {};
     cudaEvent_t evFork = nullptr;
-    // per-stream coefficient table (avdsp_b200_set_coefs): [column][stream] int32, column = index into L.coefWords; nullptr: none.
-    // Variants (set_param on other words) keep their own plans and read the same table.
-    int* dCoef = nullptr;
-    int* dCoefStage = nullptr; size_t coefStageWords = 0;     // HOST rows on their way to the table
-    // per-stream FIR table (avdsp_b200_set_fir_taps): [stream][column] int32, column = index into L.firTapWords, so that a k_fir CTA
-    // stages its stream's taps as one coalesced run; nullptr: none.  Float programs (ALU_F32) also keep one flag word per stream:
-    // set when the stream's row holds a non-zero tap below 2^-60, which the FIR kernels cannot multiply exactly (launchRun).
-    int* dFirTab = nullptr;
+    // per-stream coefficient table: [column][stream], so that the chain, DAG and generic kernels' lane = stream loads coalesce
+    StreamTable coefTab{&avdsp::Lowered::coefWords, false, "biquad coefficient"};
+    // per-stream FIR table: [stream][column], so that a k_fir CTA stages its stream's taps as one coalesced run.  Float programs
+    // (ALU_F32) also keep one flag word per stream: set when the stream's row holds a non-zero tap below 2^-60, which the FIR
+    // kernels cannot multiply exactly (launchRun).
+    StreamTable firTab{&avdsp::Lowered::firTapWords, true, "FIR tap"};
     int* dFirFlags = nullptr;
     // DSP_FORMAT 2 with a FIR table: every stream's Toeplitz limb planes for the per-stream tensor-core form (kernel_fir_tc.cu),
     // built on the device before the first such launch after the rows changed (valid = false)

@@ -72,7 +72,6 @@ class Executor:
         self.num_mem = L.avdsp_b200_num_mem(self._h)
         self.mem_words = [L.avdsp_b200_mem_word(self._h, k) for k in range(self.num_mem)]
         self.num_cores = L.avdsp_b200_num_cores(self._h)
-        self.n_coef = len(coef_words(self.words, fmt))   # columns of a set_coefs row
 
     def shards(self):
         """[(device, first_stream, n_streams, numa_node)] per GPU of the instance"""
@@ -125,7 +124,6 @@ class Executor:
         w = np.ascontiguousarray(words, dtype=np.int32)
         _check(self._L.avdsp_b200_reload_params(self._h, w.ctypes.data, len(w)))
         self.words = w
-        self.n_coef = len(coef_words(w, self.fmt))
 
     def param_index(self, offset: int, param_num: int = 0) -> int:
         """dump-file entry (offset, PARAM_NUM number) -> word index in the program (avdsp_b200_param_index)"""
@@ -147,6 +145,11 @@ class Executor:
         """Per-stream FIR taps (avdsp_b200_set_fir_taps): row s of `values` ([n, nTaps], columns in the order of
         fir_tap_words(words, fmt)) holds the tap words of stream first + s.  Host and device rows as for set_coefs."""
         self._set_rows(self._L.avdsp_b200_set_fir_taps, first, values, self.n_taps, "FIR tap")
+
+    @property
+    def n_coef(self) -> int:
+        """columns of a set_coefs row"""
+        return len(coef_words(self.words, self.fmt))
 
     @property
     def n_taps(self) -> int:
@@ -295,28 +298,24 @@ def describe(words, fs: int, fmt: int = 2, n_streams: int = 1, dither: int = 31,
     return buf.value.decode()
 
 
+def _table_words(fn, words, fmt: int) -> np.ndarray:
+    w = np.ascontiguousarray(words, dtype=np.int32)
+    out = np.zeros(_check(fn(w.ctypes.data, len(w), fmt, None, 0)), dtype=np.int32)
+    if out.size:
+        _check(fn(w.ctypes.data, len(w), fmt, out.ctypes.data, out.size))
+    return out
+
+
 def coef_words(words, fmt: int = 2) -> np.ndarray:
     """Word indices of the program's biquad coefficients (every section, every fs column, bypassed blocks too), ascending: the
     column order of Executor.set_coefs.  Host-only (no CUDA device needed)."""
-    w = np.ascontiguousarray(words, dtype=np.int32)
-    L = _lib.lib()
-    n = _check(L.avdsp_b200_coef_words(w.ctypes.data, len(w), fmt, None, 0))
-    out = np.zeros(n, dtype=np.int32)
-    if n:
-        _check(L.avdsp_b200_coef_words(w.ctypes.data, len(w), fmt, out.ctypes.data, n))
-    return out
+    return _table_words(_lib.lib().avdsp_b200_coef_words, words, fmt)
 
 
 def fir_tap_words(words, fmt: int = 2) -> np.ndarray:
     """Word indices of the program's FIR taps (every convolution entry of every DSP_FIR, every fs column), ascending, each
     word once: the column order of Executor.set_fir_taps.  Host-only (no CUDA device needed)."""
-    w = np.ascontiguousarray(words, dtype=np.int32)
-    L = _lib.lib()
-    n = _check(L.avdsp_b200_fir_tap_words(w.ctypes.data, len(w), fmt, None, 0))
-    out = np.zeros(n, dtype=np.int32)
-    if n:
-        _check(L.avdsp_b200_fir_tap_words(w.ctypes.data, len(w), fmt, out.ctypes.data, n))
-    return out
+    return _table_words(_lib.lib().avdsp_b200_fir_tap_words, words, fmt)
 
 
 def measure_int_peak(device: int = 0, iters: int = 4096) -> float:

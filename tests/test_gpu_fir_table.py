@@ -9,6 +9,7 @@ import pytest
 from conftest import load_program
 from avdsp_b200 import (Executor, AvdspError, synth, coef_words, fir_tap_words, KERNEL_AUTO, KERNEL_FIR, KERNEL_FIR_TC,
                         KERNEL_GENERIC)
+from oracle import wire
 from test_fir_table import fir_program, taps
 
 pytestmark = pytest.mark.gpu
@@ -203,10 +204,8 @@ def test_host_and_device_rows(oracle_lib):
         assert np.array_equal(ex.get_state(s)[: ex.data_size], o.data), s
 
 
-@pytest.mark.parametrize("fmt", [2, 3, 4, 6])
-def test_fir_and_biquad_tables_on_generic(oracle_lib, fmt):
-    """a program mixing FIR and biquads runs on k_generic: both tables meet there"""
-    fs, S, T = 48000, 24, 300
+def fir_and_biquad_tables(fmt, S, fs):
+    """a program mixing FIR and biquads, with a FIR table and a coefficient table whose rows all differ"""
     base = fir_program(fmt, [[taps(40, fmt, 1)], [taps(33, fmt, 2)]], biquad=True)
     tw, cw = fir_tap_words(base, fmt), coef_words(base, fmt)
     rows = impulse_rows(base, tw, S, 2 if fmt == 2 else 3, seed=15)     # taps are float bit patterns in every float format
@@ -220,15 +219,50 @@ def test_fir_and_biquad_tables_on_generic(oracle_lib, fmt):
     ex = make(base, fs, fmt, S, dither=24)
     ex.set_fir_taps(0, rows)
     ex.set_coefs(0, np.ascontiguousarray(crow))
-    x = (synth.pcm_float if fmt >= 5 else synth.pcm)("noise", S, T, ex.n_in, fs)
-    y = ex.process(x)
-    assert ex.last_kernel == "generic"
 
     def prog(s):
         p = own_program(base, tw, rows[s])
         p[cw] = crow[s]
         return p
+    return ex, base, tw, cw, prog
+
+
+@pytest.mark.parametrize("fmt", [2, 3, 4, 6])
+def test_fir_and_biquad_tables_on_generic(oracle_lib, fmt):
+    """a program mixing FIR and biquads runs on k_generic: both tables meet there"""
+    fs, S, T = 48000, 24, 300
+    ex, _, _, _, prog = fir_and_biquad_tables(fmt, S, fs)
+    x = (synth.pcm_float if fmt >= 5 else synth.pcm)("noise", S, T, ex.n_in, fs)
+    y = ex.process(x)
+    assert ex.last_kernel == "generic"
     check_streams(oracle_lib, y, ex, prog, x, fmt, fs, range(S), dither=24)
+
+
+@pytest.mark.parametrize("fmt", [2, 3])
+def test_one_set_param_spans_both_tables_and_a_variant_word(oracle_lib, fmt):
+    """one set_param over core 0's last tap, the words of the BIQUADS block before its first coefficient, and that coefficient:
+    the tap goes into the FIR rows, the coefficient into the coefficient rows, and the informational type word makes one
+    variant for the range"""
+    fs, S, T, first, n = 48000, 24, 300, 5, 11
+    ex, base, tw, cw, prog = fir_and_biquad_tables(fmt, S, fs)
+    a, b = int(tw[tw < cw[0]][-1]), int(cw[0])
+    hdr = a + 1 + int(np.flatnonzero((base[a + 1: b] >> 16) == wire.OP["BIQUADS"])[0])
+    vals = base[a: b + 1].copy()
+    vals[0] = np.float32(0.03125).view(np.int32) if fmt != 2 else 1 << 24                # the tap
+    vals[hdr + 2 - a] = 0x00020000 | 1000                                                 # section type << 16 | freq
+    vals[-1] = np.float32(0.09375).view(np.int32) if fmt != 2 else int(base[b]) + 99      # b0
+    assert sum(w in tw for w in range(a, b + 1)) == 1 and sum(w in cw for w in range(a, b + 1)) == 1
+    ex.set_param(first, n, a, vals)
+    assert ex.num_variants == 2
+    x = synth.pcm("noise", S, T, ex.n_in, fs)
+    y = ex.process(x)
+
+    def prog2(s):
+        p = prog(s)
+        if first <= s < first + n:
+            p[a: b + 1] = vals
+        return p
+    check_streams(oracle_lib, y, ex, prog2, x, fmt, fs, range(S), dither=24)
 
 
 def test_refusals_change_nothing(oracle_lib):
