@@ -168,92 +168,109 @@ static int quiesce(avdsp_b200* h);
 static int resetShards(avdsp_b200* h, int fs, const int32_t* seeds, int defaultDither);
 
 // Host-only half of plan preparation: which kernels can take the program, their CTA geometries, the lowering trace.
-static void planGeometries(avdsp_b200* h, std::vector<ChainLane>* lanes2) {
-    const Lowered& L = h->L;
-    h->chain2Usable = false;
+static void planGeometries(Plans& p, int nStreams, int numSMs, std::vector<ChainLane>* lanes2) {
+    const Lowered& L = p.L;
+    p.chain2Usable = false;
     lanes2->assign(1024, ChainLane{});
-    if (L.chainOk && chain2Supports(L.chain)) h->chain2Usable = planChain2Geometry(L.chain, h->nStreams, h->numSMs, &h->geom2, lanes2->data());
-    h->chain3Usable = h->chain2Usable && planChain3Geometry(L.chain, h->nStreams, h->numSMs, &h->geom3);
-    h->mixUsable = false;
-    if (L.chainOk) { std::string why; h->mixUsable = buildMixPlan(L.chain, &h->mix, &why); }
-    h->firUsable = L.firOk;
-    h->dagUsable = L.dagOk && L.dag && planDagGeometry(*L.dag, h->nStreams, h->numSMs, &h->geomDag);
+    if (L.chainOk && chain2Supports(L.chain)) p.chain2Usable = planChain2Geometry(L.chain, nStreams, numSMs, &p.geom2, lanes2->data());
+    p.chain3Usable = p.chain2Usable && planChain3Geometry(L.chain, nStreams, numSMs, &p.geom3);
+    p.mixUsable = false;
+    if (L.chainOk) { std::string why; p.mixUsable = buildMixPlan(L.chain, &p.mix, &why); }
+    p.firUsable = L.firOk;
+    p.dagUsable = L.dagOk && L.dag && planDagGeometry(*L.dag, nStreams, numSMs, &p.geomDag);
     char line[512];
-    h->trace = L.trace;
-    if (h->firUsable) {
+    p.trace = L.trace;
+    if (p.firUsable) {
         snprintf(line, sizeof line, "time-parallel FIR kernel: usable (%d paths, longest impulse %d taps)\n", L.fir.nPaths, L.fir.maxLen);
-        h->trace += line;
-    } else if (!L.firs.empty()) h->trace += "FIR kernel not used: " + L.firWhyNot + "\n";
-    if (h->mixUsable) h->trace += "time-parallel mix kernel: usable (no biquad in any path)\n";
-    if (h->chain2Usable) {
+        p.trace += line;
+    } else if (!L.firs.empty()) p.trace += "FIR kernel not used: " + L.firWhyNot + "\n";
+    if (p.mixUsable) p.trace += "time-parallel mix kernel: usable (no biquad in any path)\n";
+    if (p.chain2Usable) {
         snprintf(line, sizeof line, "chain kernel v2 geometry: %d streams/CTA, %d sections/lane, tile %d frames, gmax %d, %d section threads + %d helper threads, %d sources, %zu B smem\n",
-                 h->geom2.streamsPerCta, h->geom2.secPerLane, h->geom2.tileFrames, h->geom2.gmax, h->geom2.secThreads, h->geom2.helpThreads, L.chain.h.nSrc, h->geom2.smemBytes);
-        h->trace += line;
+                 p.geom2.streamsPerCta, p.geom2.secPerLane, p.geom2.tileFrames, p.geom2.gmax, p.geom2.secThreads, p.geom2.helpThreads, L.chain.h.nSrc, p.geom2.smemBytes);
+        p.trace += line;
     }
-    if (h->chain3Usable) {
+    if (p.chain3Usable) {
         snprintf(line, sizeof line, "chain kernel v3 geometry: %d streams/CTA (lane = one cascade part of one stream), %d cascade warps of <= %d sections + 1 dither warp + %d store warps, largest lag %d frames, row ring %d steps, %zu B smem; parts (chain:first+n@base):",
-                 h->geom3.streamsPerCta, h->geom3.nCascade, h->geom3.maxSec, h->geom3.nStore, h->geom3.gmax, h->geom3.postRing, h->geom3.smemBytes);
-        h->trace += line;
-        for (int w = 0; w < h->geom3.nCascade; w++) {
-            snprintf(line, sizeof line, " %d:%d+%d@%d", h->geom3.warpChain[w], h->geom3.warpFirstSec[w], h->geom3.warpNsec[w], h->geom3.warpBase[w]);
-            h->trace += line;
+                 p.geom3.streamsPerCta, p.geom3.nCascade, p.geom3.maxSec, p.geom3.nStore, p.geom3.gmax, p.geom3.postRing, p.geom3.smemBytes);
+        p.trace += line;
+        for (int w = 0; w < p.geom3.nCascade; w++) {
+            snprintf(line, sizeof line, " %d:%d+%d@%d", p.geom3.warpChain[w], p.geom3.warpFirstSec[w], p.geom3.warpNsec[w], p.geom3.warpBase[w]);
+            p.trace += line;
         }
-        h->trace += "; sub-partitions (sections of the cascade warps on hardware warps q, q+4, ..; d = dither warp, s = store warp):";
+        p.trace += "; sub-partitions (sections of the cascade warps on hardware warps q, q+4, ..; d = dither warp, s = store warp):";
         for (int q = 0; q < 4; q++) {
-            h->trace += q ? " |" : " ";
-            for (int id = q; id < h->geom3.threads / 32; id += 4) {
-                const int role = h->geom3.warpRole[id];
-                if (role >= 0) snprintf(line, sizeof line, " %d", h->geom3.warpNsec[role]);
+            p.trace += q ? " |" : " ";
+            for (int id = q; id < p.geom3.threads / 32; id += 4) {
+                const int role = p.geom3.warpRole[id];
+                if (role >= 0) snprintf(line, sizeof line, " %d", p.geom3.warpNsec[role]);
                 else snprintf(line, sizeof line, " %s", role == -1 ? "d" : "s");
-                h->trace += line;
+                p.trace += line;
             }
         }
-        h->trace += "\n";
+        p.trace += "\n";
     }
-    if (h->dagUsable) {
+    if (p.dagUsable) {
         snprintf(line, sizeof line, "DAG kernel geometry: %d nodes (depth %d, longest cascade %d sections), %d streams/CTA, %d threads, tiles of %d frames, input rows of %d frames, %d words/stream, %zu B smem%s\n",
-                 L.dag->nNodes, L.dag->maxDepth, L.dag->maxSec, h->geomDag.streamsPerCta, h->geomDag.threads, h->geomDag.tileFrames, h->geomDag.rawMask + 1, h->geomDag.perStreamWords,
-                 h->geomDag.smemBytes, (h->chain2Usable || h->mixUsable || h->firUsable) ? " (another fused kernel takes this program first)" : "");
-        h->trace += line;
-    } else if (!L.dagOk && !h->chain2Usable && !h->mixUsable && !h->firUsable) h->trace += "DAG kernel not used: " + L.dagWhyNot + "\n";
-    if (!h->chain2Usable && !h->mixUsable) {
+                 L.dag->nNodes, L.dag->maxDepth, L.dag->maxSec, p.geomDag.streamsPerCta, p.geomDag.threads, p.geomDag.tileFrames, p.geomDag.rawMask + 1, p.geomDag.perStreamWords,
+                 p.geomDag.smemBytes, (p.chain2Usable || p.mixUsable || p.firUsable) ? " (another fused kernel takes this program first)" : "");
+        p.trace += line;
+    } else if (!L.dagOk && !p.chain2Usable && !p.mixUsable && !p.firUsable) p.trace += "DAG kernel not used: " + L.dagWhyNot + "\n";
+    if (!p.chain2Usable && !p.mixUsable) {
         const bool coefRange = L.chainOk && L.chain.h.aluClass == ALU_F32 && !chainFloatCoefsInRange(L.chain);
         snprintf(line, sizeof line, "chain kernels not used: %s\n",
                  coefRange ? "a biquad coefficient lies outside [2^-60, 2^7): the float class could not bound its products (exactness guard), the interpreter runs this program"
                            : L.chainOk ? "geometry does not fit" : L.chainWhyNot.c_str());
-        h->trace += line;
+        p.trace += line;
     }
 }
 
-static int uploadPlanData(avdsp_b200* h) {
-    cudaSetDevice(h->device);
-    const Lowered& L = h->L;
+static int uploadPlanData(Plans& p, int device, int nStreams, int numSMs) {
+    cudaSetDevice(device);
+    p.planDevice = device;
+    const Lowered& L = p.L;
     // big pool (FIR taps, data tables)
-    if (h->dBig) { cudaFree(h->dBig); h->dBig = nullptr; }
-    h->bigWords = L.bigPool.size();
-    if (h->bigWords) {
-        CU(cudaMalloc(&h->dBig, h->bigWords * 4));
-        CU(cudaMemcpy(h->dBig, L.bigPool.data(), h->bigWords * 4, cudaMemcpyHostToDevice));
+    if (p.dBig) { cudaFree(p.dBig); p.dBig = nullptr; }
+    p.bigWords = L.bigPool.size();
+    if (p.bigWords) {
+        CU(cudaMalloc(&p.dBig, p.bigWords * 4));
+        CU(cudaMemcpy(p.dBig, L.bigPool.data(), p.bigWords * 4, cudaMemcpyHostToDevice));
     }
-    if (h->dFirCol) { cudaFree(h->dFirCol); h->dFirCol = nullptr; }
+    if (p.dFirCol) { cudaFree(p.dFirCol); p.dFirCol = nullptr; }
     if (!L.firColOfOp.empty()) {
-        CU(cudaMalloc(&h->dFirCol, L.firColOfOp.size() * 4));
-        CU(cudaMemcpy(h->dFirCol, L.firColOfOp.data(), L.firColOfOp.size() * 4, cudaMemcpyHostToDevice));
+        CU(cudaMalloc(&p.dFirCol, L.firColOfOp.size() * 4));
+        CU(cudaMemcpy(p.dFirCol, L.firColOfOp.data(), L.firColOfOp.size() * 4, cudaMemcpyHostToDevice));
     }
     std::vector<ChainLane> lanes2;
-    planGeometries(h, &lanes2);
-    if (h->chain2Usable) {
-        if (!h->dLanes2) CU(cudaMalloc(&h->dLanes2, 1024 * sizeof(ChainLane)));
-        CU(cudaMemcpy(h->dLanes2, lanes2.data(), 1024 * sizeof(ChainLane), cudaMemcpyHostToDevice));
+    planGeometries(p, nStreams, numSMs, &lanes2);
+    if (p.chain2Usable) {
+        if (!p.dLanes2) CU(cudaMalloc(&p.dLanes2, 1024 * sizeof(ChainLane)));
+        CU(cudaMemcpy(p.dLanes2, lanes2.data(), 1024 * sizeof(ChainLane), cudaMemcpyHostToDevice));
     }
-    if (h->dFirTaps) { cudaFree(h->dFirTaps); h->dFirTaps = nullptr; }
-    if (h->firUsable) {
+    if (p.dFirTaps) { cudaFree(p.dFirTaps); p.dFirTaps = nullptr; }
+    if (p.firUsable) {
         std::vector<unsigned char> blobs;
         firTcBuildTaps(L.fir, L.fir.aluClass == ALU_INT64 ? FIRTC_I8 : FIRTC_TF32, L.bigPool.data(), &blobs);
-        CU(cudaMalloc(&h->dFirTaps, blobs.size()));
-        CU(cudaMemcpy(h->dFirTaps, blobs.data(), blobs.size(), cudaMemcpyHostToDevice));
+        CU(cudaMalloc(&p.dFirTaps, blobs.size()));
+        CU(cudaMemcpy(p.dFirTaps, blobs.data(), blobs.size(), cudaMemcpyHostToDevice));
     }
     return 0;
+}
+
+// p's own words lowered at another rate / default dither into *nl (the multi-device parent takes only this half)
+static int decodeAt(const Plans& p, int fs, int defaultDither, Lowered* nl) {
+    std::string err;
+    const int rc = decodeProgram(p.L.words.data(), (int)p.L.words.size(), 0x7FFFFFFF, p.L.format, fs, defaultDither, nl, &err);
+    return rc < 0 ? setErr(rc, err) : rc;
+}
+
+// p re-planned at another rate / default dither for instance h's device and batch; its state layout may not change
+static int replanAt(Plans& p, int fs, int defaultDither, const avdsp_b200* h) {
+    Lowered nl;
+    const int rc = decodeAt(p, fs, defaultDither, &nl); if (rc < 0) return rc;
+    if (nl.gen.h.stateWords != p.L.gen.h.stateWords) return setErr(AVDSP_B200_ERR_ARG, "state layout changed on reset");
+    p.L = std::move(nl);
+    return uploadPlanData(p, h->device, h->nStreams, h->numSMs);
 }
 
 static int initState(avdsp_b200* h) {
@@ -297,22 +314,16 @@ static void freeAll(avdsp_b200* h) {
         return;
     }
     if (h->evLast) cudaEventSynchronize(h->evLast);
-    for (avdsp_b200* v : h->variants) freeAll(v);
-    h->variants.clear();
     cudaSetDevice(h->device);
     if (h->dState) cudaFree(h->dState);
-    if (h->dBig) cudaFree(h->dBig);
-    if (h->dFirCol) cudaFree(h->dFirCol);
     if (h->dMemInit) cudaFree(h->dMemInit);
     if (h->dSeeds) cudaFree(h->dSeeds);
-    if (h->dLanes2) cudaFree(h->dLanes2);
     if (h->dJump) cudaFree(h->dJump);
     if (h->dTpdf) cudaFree(h->dTpdf);
     if (h->dRedo) cudaFree(h->dRedo);
     if (h->dSnap) cudaFree(h->dSnap);
     if (h->dRedoList) cudaFree(h->dRedoList);
     if (h->dRedoCount) cudaFree(h->dRedoCount);
-    if (h->dFirTaps) cudaFree(h->dFirTaps);
     if (h->dFirWs) cudaFree(h->dFirWs);
     freeTable(h->coefTab);
     freeTable(h->firTab);
@@ -370,7 +381,7 @@ int avdsp_b200_create(avdsp_b200_t** out, const int32_t* prog, int progWords, in
     CU(cudaEventCreateWithFlags(&h->evLast, cudaEventDisableTiming));
     const size_t words = (size_t)nStreams * h->L.gen.h.stateWords;
     CU(cudaMalloc(&h->dState, std::max<size_t>(words, 1) * 4));
-    int r = uploadPlanData(h.get()); if (r < 0) return r;
+    int r = uploadPlanData(*h, device, nStreams, h->numSMs); if (r < 0) return r;
     r = initState(h.get()); if (r < 0) return r;
     g_lastError.clear();
     *out = h.release();
@@ -382,14 +393,13 @@ void avdsp_b200_destroy(avdsp_b200_t* h) { freeAll(h); }
 int avdsp_b200_describe(const int32_t* prog, int progWords, int fs, int format, int defaultDither, int nStreams, int numSMs,
                         char* out, int outLen) {
     if (!out || outLen < 1 || nStreams < 1 || numSMs < 1) return setErr(AVDSP_B200_ERR_ARG, "bad argument");
-    avdsp_b200 h;                                            // host-only: decode + lower + plan, nothing touches CUDA
+    Plans p;                                                 // host-only: decode + lower + plan, nothing touches CUDA
     std::string err;
-    const int rc = decodeProgram(prog, progWords, 0x7FFFFFFF, format, fs, defaultDither, &h.L, &err);
+    const int rc = decodeProgram(prog, progWords, 0x7FFFFFFF, format, fs, defaultDither, &p.L, &err);
     if (rc < 0) return setErr(rc, err);
-    h.nStreams = nStreams; h.numSMs = numSMs;
     std::vector<ChainLane> lanes2;
-    planGeometries(&h, &lanes2);
-    snprintf(out, (size_t)outLen, "%s", h.trace.c_str());
+    planGeometries(p, nStreams, numSMs, &lanes2);
+    snprintf(out, (size_t)outLen, "%s", p.trace.c_str());
     return rc;
 }
 
@@ -398,25 +408,12 @@ int avdsp_b200_reset(avdsp_b200_t* h, int fs, const int32_t* seeds, int defaultD
     if (!h->shards.empty()) return resetShards(h, fs, seeds, defaultDither);
     { const int q = quiesce(h); if (q < 0) return q; }
     if (fs != h->L.fs || defaultDither != h->L.defaultDither) {
-        Lowered nl;
-        std::string err;
-        const std::vector<int32_t> words = h->L.words;
-        const int rc = decodeProgram(words.data(), (int)words.size(), 0x7FFFFFFF, h->L.format, fs, defaultDither, &nl, &err);
-        if (rc < 0) return setErr(rc, err);
-        if (nl.gen.h.stateWords != h->L.gen.h.stateWords) return setErr(AVDSP_B200_ERR_ARG, "state layout changed on reset");
-        h->L = nl;
-        const int r = uploadPlanData(h); if (r < 0) return r;
+        const int r = replanAt(*h, fs, defaultDither, h); if (r < 0) return r;
         // the per-stream Toeplitz planes follow this rate's tap blocks (and their size its longest impulse)
         if (h->dFirTcPer) { cudaFree(h->dFirTcPer); h->dFirTcPer = nullptr; }
         h->firTcPerValid = h->firTcPerFailed = false;
-        for (avdsp_b200* v : h->variants) {                   // the overrides stay; their plans follow the new rate / dither
-            Lowered vl;
-            const std::vector<int32_t> vw = v->L.words;
-            const int vr = decodeProgram(vw.data(), (int)vw.size(), 0x7FFFFFFF, h->L.format, fs, defaultDither, &vl, &err);
-            if (vr < 0) return setErr(vr, err);
-            v->L = vl;
-            const int ur = uploadPlanData(v); if (ur < 0) return ur;
-        }
+        for (auto& v : h->variants)                           // the overrides stay; their plans follow the new rate / dither
+            { const int vr = replanAt(*v, fs, defaultDither, h); if (vr < 0) return vr; }
     }
     if (seeds) h->seeds.assign(seeds, seeds + h->nStreams); else h->seeds.clear();
     return initState(h);
@@ -467,13 +464,13 @@ const char* avdsp_b200_trace(const avdsp_b200_t* h) { return h ? h->trace.c_str(
 
 // One launch over streams [first, first+n) with device buffers.  coreSel/plan override serve the
 // dspRuntime_<fmt> compatibility path.
-// `pl` carries the plans (the instance itself, or the variant a per-stream parameter override created, see avdsp_b200_set_param);
-// state, scratch and bookkeeping are the instance's.
+// `pl`: the plans the streams run (the instance's own, or a variant a per-stream parameter override created, see
+// avdsp_b200_set_param); state, scratch, tables and bookkeeping are the instance's.
 // ordered = false: the caller (launchRange, runs of variants on forked streams) has done the instance's stream ordering itself.
-static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int nFrames, int layout, int first, int n,
+static int launchRun(avdsp_b200* h, const Plans& pl, const int* in, int* out, int nFrames, int layout, int first, int n,
                      cudaStream_t stream, int coreSel, const GenericPlan* planOverride, int cap, bool ordered = true) {
     if (nFrames == 0 || n == 0) return 0;
-    const GenericPlan& G = planOverride ? *planOverride : pl->L.gen;
+    const GenericPlan& G = planOverride ? *planOverride : pl.L.gen;
     const PlanHeader& P = G.h;
     const int nIn = P.nIn, nOut = P.nOut;
     if (cap <= 0) cap = nFrames;            // frames the buffers are laid out for (>= nFrames: staging slots are reused for a shorter last chunk)
@@ -491,28 +488,28 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
     const int* firTaps = h->firTab.d ? h->firTab.d + (size_t)first * nTapCols : nullptr;      // ... and the FIR table
     if (ordered) CU(cudaStreamWaitEvent(stream, h->evLast, 0));          // stream-ordered after the instance's previous launch (see evLast)
     // the fused kernels run the canonical order; a plugin-order request may use them when the two orders provably agree
-    const bool chainOrder = (h->period == 0 || pl->L.orderIndependent) && coreSel < 0 && !planOverride;
+    const bool chainOrder = (h->period == 0 || pl.L.orderIndependent) && coreSel < 0 && !planOverride;
     int use = AVDSP_B200_KERNEL_GENERIC;
     if (chainOrder && h->kernelSel != AVDSP_B200_KERNEL_GENERIC) {
         if (h->kernelSel == AVDSP_B200_KERNEL_CHAIN_V1)
             return setErr(AVDSP_B200_ERR_UNSUPPORTED, "the first, tile-synchronous chain kernel was removed; use AVDSP_B200_KERNEL_CHAIN");
-        if (pl->chain2Usable) use = AVDSP_B200_KERNEL_CHAIN;
+        if (pl.chain2Usable) use = AVDSP_B200_KERNEL_CHAIN;
     }
     // X/Y dataflow programs: the DAG kernel when no other fused kernel takes the program (or on request)
-    if (chainOrder && pl->dagUsable && ((h->kernelSel == AVDSP_B200_KERNEL_AUTO && use == AVDSP_B200_KERNEL_GENERIC && !pl->mixUsable && !pl->firUsable) ||
+    if (chainOrder && pl.dagUsable && ((h->kernelSel == AVDSP_B200_KERNEL_AUTO && use == AVDSP_B200_KERNEL_GENERIC && !pl.mixUsable && !pl.firUsable) ||
                                         h->kernelSel == AVDSP_B200_KERNEL_DAG)) use = AVDSP_B200_KERNEL_DAG;
     if (h->kernelSel == AVDSP_B200_KERNEL_DAG && use != AVDSP_B200_KERNEL_DAG)
-        return setErr(AVDSP_B200_ERR_UNSUPPORTED, "DAG kernel requested but this program/order does not map to it: " + pl->L.dagWhyNot);
-    if (chainOrder && pl->mixUsable && (h->kernelSel == AVDSP_B200_KERNEL_AUTO || h->kernelSel == AVDSP_B200_KERNEL_MIX)) use = AVDSP_B200_KERNEL_MIX;
-    if (chainOrder && pl->firUsable && (h->kernelSel == AVDSP_B200_KERNEL_AUTO || h->kernelSel == AVDSP_B200_KERNEL_FIR)) use = AVDSP_B200_KERNEL_FIR;
+        return setErr(AVDSP_B200_ERR_UNSUPPORTED, "DAG kernel requested but this program/order does not map to it: " + pl.L.dagWhyNot);
+    if (chainOrder && pl.mixUsable && (h->kernelSel == AVDSP_B200_KERNEL_AUTO || h->kernelSel == AVDSP_B200_KERNEL_MIX)) use = AVDSP_B200_KERNEL_MIX;
+    if (chainOrder && pl.firUsable && (h->kernelSel == AVDSP_B200_KERNEL_AUTO || h->kernelSel == AVDSP_B200_KERNEL_FIR)) use = AVDSP_B200_KERNEL_FIR;
     // tensor-core Toeplitz GEMM: the bit-exact int8-limb form is the default for fixed-point batches that fill a tile;
     // the 3xTF32 form (stated tolerance) only on request.  With a per-stream FIR table the int8-limb form runs per stream (a
     // CTA = 128 outputs x 64 output blocks of one stream), which AUTO takes when a call fills those 64 blocks (8192 frames);
     // the 3xTF32 form takes shared taps only
-    const bool fixedTc = pl->L.fir.aluClass == ALU_INT64 && pl->L.fir.maxLen >= 256;
-    if (h->kernelSel == AVDSP_B200_KERNEL_FIR_TC && firTaps && pl->L.fir.aluClass != ALU_INT64)
+    const bool fixedTc = pl.L.fir.aluClass == ALU_INT64 && pl.L.fir.maxLen >= 256;
+    if (h->kernelSel == AVDSP_B200_KERNEL_FIR_TC && firTaps && pl.L.fir.aluClass != ALU_INT64)
         return setErr(AVDSP_B200_ERR_UNSUPPORTED, "the 3xTF32 tensor-core FIR kernel takes taps every stream shares; this instance has a per-stream FIR table");
-    if (chainOrder && pl->firUsable && (h->kernelSel == AVDSP_B200_KERNEL_FIR_TC ||
+    if (chainOrder && pl.firUsable && (h->kernelSel == AVDSP_B200_KERNEL_FIR_TC ||
         (h->kernelSel == AVDSP_B200_KERNEL_AUTO && fixedTc && (firTaps ? nFrames >= 8192 && !h->firTcPerFailed : n >= 32 && nFrames >= 128))))
         use = AVDSP_B200_KERNEL_FIR_TC;
     if (use == AVDSP_B200_KERNEL_FIR_TC && firTaps && !h->dFirTcPer && !h->firTcPerFailed) {
@@ -529,18 +526,18 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
     }
     if (use == AVDSP_B200_KERNEL_FIR_TC && firTaps && h->firTcPerFailed) use = AVDSP_B200_KERNEL_FIR;
     if (h->kernelSel == AVDSP_B200_KERNEL_FIR_TC && use != AVDSP_B200_KERNEL_FIR_TC && !(firTaps && h->firTcPerFailed))
-        return setErr(AVDSP_B200_ERR_UNSUPPORTED, "tensor-core FIR kernel requested but this program/order does not map to it: " + pl->L.firWhyNot);
+        return setErr(AVDSP_B200_ERR_UNSUPPORTED, "tensor-core FIR kernel requested but this program/order does not map to it: " + pl.L.firWhyNot);
     if (h->kernelSel == AVDSP_B200_KERNEL_FIR && use != AVDSP_B200_KERNEL_FIR)
-        return setErr(AVDSP_B200_ERR_UNSUPPORTED, "FIR kernel requested but this program/order does not map to it: " + pl->L.firWhyNot);
+        return setErr(AVDSP_B200_ERR_UNSUPPORTED, "FIR kernel requested but this program/order does not map to it: " + pl.L.firWhyNot);
     if (h->kernelSel == AVDSP_B200_KERNEL_MIX && use != AVDSP_B200_KERNEL_MIX)
         return setErr(AVDSP_B200_ERR_UNSUPPORTED, "mix kernel requested but the program has biquads or does not map to independent paths");
     if ((h->kernelSel == AVDSP_B200_KERNEL_CHAIN || h->kernelSel == AVDSP_B200_KERNEL_CHAIN_V1 || h->kernelSel == AVDSP_B200_KERNEL_CHAIN_V2 ||
          h->kernelSel == AVDSP_B200_KERNEL_CHAIN_V3) && use == AVDSP_B200_KERNEL_GENERIC)
-        return setErr(AVDSP_B200_ERR_UNSUPPORTED, "chain kernel requested but this program/order does not map to it: " + pl->L.chainWhyNot);
+        return setErr(AVDSP_B200_ERR_UNSUPPORTED, "chain kernel requested but this program/order does not map to it: " + pl.L.chainWhyNot);
     cudaError_t e;
     if (use == AVDSP_B200_KERNEL_FIR || use == AVDSP_B200_KERNEL_FIR_TC) {
         FirArgs A{};
-        A.in = in; A.out = out; A.state = st; A.bigPool = pl->dBig;
+        A.in = in; A.out = out; A.state = st; A.bigPool = pl.dBig;
         A.nStreams = n; A.nFrames = nFrames;
         A.inStreamStride = inSS; A.outStreamStride = outSS;
         A.inFrameStride = inFS; A.inChStride = inCS; A.outFrameStride = outFS; A.outChStride = outCS;
@@ -552,7 +549,7 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
                 h->firTcPerValid = true;
                 h->launches++;
             }
-            const size_t need = firTcPerWorkspaceBytes(pl->L.fir, n, nFrames);
+            const size_t need = firTcPerWorkspaceBytes(pl.L.fir, n, nFrames);
             if (need > h->firWsBytes) {
                 CU(cudaStreamSynchronize(stream));
                 if (h->dFirWs) cudaFree(h->dFirWs);
@@ -561,10 +558,10 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
                 h->firWsBytes = need;
             }
             A.taps = firTaps; A.tapPitch = nTapCols;
-            e = launchFirTcPer(pl->L.fir, A, h->dFirTcPer + (size_t)first * (firTcPerTapsBytes(h->L.fir, 1)), h->dFirWs, stream, &nl);
+            e = launchFirTcPer(pl.L.fir, A, h->dFirTcPer + (size_t)first * (firTcPerTapsBytes(h->L.fir, 1)), h->dFirWs, stream, &nl);
         } else if (use == AVDSP_B200_KERNEL_FIR_TC) {
-            const int kind = pl->L.fir.aluClass == ALU_INT64 ? FIRTC_I8 : FIRTC_TF32;
-            const size_t need = firTcWorkspaceBytes(pl->L.fir, kind, n, nFrames);
+            const int kind = pl.L.fir.aluClass == ALU_INT64 ? FIRTC_I8 : FIRTC_TF32;
+            const size_t need = firTcWorkspaceBytes(pl.L.fir, kind, n, nFrames);
             if (need > h->firWsBytes) {
                 CU(cudaStreamSynchronize(stream));
                 if (h->dFirWs) cudaFree(h->dFirWs);
@@ -572,24 +569,24 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
                 CU(cudaMalloc(&h->dFirWs, need));
                 h->firWsBytes = need;
             }
-            e = launchFirTc(pl->L.fir, kind, A, pl->dFirTaps, h->dFirWs, stream, &nl);
+            e = launchFirTc(pl.L.fir, kind, A, pl.dFirTaps, h->dFirWs, stream, &nl);
         } else {
             A.taps = firTaps; A.tapPitch = nTapCols;
-            A.skip = firTaps && pl->L.fir.aluClass == ALU_F32 ? h->dFirFlags + first : nullptr;
-            e = launchFir(pl->L.fir, A, h->numSMs, stream, &nl);
+            A.skip = firTaps && pl.L.fir.aluClass == ALU_F32 ? h->dFirFlags + first : nullptr;
+            e = launchFir(pl.L.fir, A, h->numSMs, stream, &nl);
             if (e == cudaSuccess && A.skip) {
                 // float rows with a tap the FIR kernels cannot multiply exactly: their CTAs did nothing, and the interpreter
                 // runs those streams now from their untouched state blocks (one launch; streams without the flag return at once)
                 GenericArgs X{};
-                X.in = in; X.out = out; X.state = st; X.bigPool = pl->dBig;
+                X.in = in; X.out = out; X.state = st; X.bigPool = pl.dBig;
                 X.nStreams = n; X.nFrames = nFrames;
                 X.inStreamStride = inSS; X.outStreamStride = outSS;
                 X.inFrameStride = inFS; X.inChStride = inCS; X.outFrameStride = outFS; X.outChStride = outCS;
                 X.coreSel = -1; X.period = 0;
                 X.redo = A.skip; X.snapshot = st;
-                X.coefs = coefs; X.coefPitch = h->nStreams; X.coefStep = 5 * pl->L.nFreq;
-                X.firTaps = firTaps; X.firPitch = nTapCols; X.firCol = pl->dFirCol;
-                for (int c = 0; c < P.nCores && c < kMaxCores; c++) { X.coreInMask[c] = pl->L.cores[c].usedIn; X.coreOutMask[c] = pl->L.cores[c].usedOut; }
+                X.coefs = coefs; X.coefPitch = h->nStreams; X.coefStep = 5 * pl.L.nFreq;
+                X.firTaps = firTaps; X.firPitch = nTapCols; X.firCol = pl.dFirCol;
+                for (int c = 0; c < P.nCores && c < kMaxCores; c++) { X.coreInMask[c] = pl.L.cores[c].usedIn; X.coreOutMask[c] = pl.L.cores[c].usedOut; }
                 e = launchGeneric(G, X, stream);
                 nl++;
             }
@@ -605,8 +602,8 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         A.vecIn = inCS == 1 && inFS == nIn && (inSS & 3) == 0 && ((size_t)in & 15) == 0;
         A.vecOut = outCS == 1 && (nOut & 3) == 0 && (outFS & 3) == 0 && (outSS & 3) == 0 && ((size_t)out & 15) == 0;
         int J = 1, Lseg = nFrames;
-        mixPrngSegments(pl->mix, A, h->numSMs, &J, &Lseg);
-        if (pl->mix.hasCalc || pl->mix.anyTpdf) {
+        mixPrngSegments(pl.mix, A, h->numSMs, &J, &Lseg);
+        if (pl.mix.hasCalc || pl.mix.anyTpdf) {
             const size_t need = (size_t)n * nFrames;
             if (need > h->tpdfWords) { if (h->dTpdf) cudaFree(h->dTpdf); h->dTpdf = nullptr; CU(cudaMalloc(&h->dTpdf, need * 4)); h->tpdfWords = need; }
             constexpr int kJumpLevels = kMixJumpLevels;       // thread j applies M^(2L * 2^b) for the bits b set in j
@@ -621,7 +618,7 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         }
         A.tpdfBuf = h->dTpdf;
         int nl = 1;
-        e = launchMix(pl->mix, A, h->dJump, J, Lseg, h->numSMs, stream, &nl);
+        e = launchMix(pl.mix, A, h->dJump, J, Lseg, h->numSMs, stream, &nl);
         h->lastKernel = AVDSP_B200_KERNEL_MIX;
         h->launches += nl - 1;                               // one is counted below
     } else if (use == AVDSP_B200_KERNEL_DAG) {
@@ -631,11 +628,11 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         A.inStreamStride = inSS; A.outStreamStride = outSS;
         A.inFrameStride = inFS; A.inChStride = inCS; A.outFrameStride = outFS; A.outChStride = outCS;
         A.coefs = coefs; A.coefPitch = h->nStreams;
-        e = launchDag(*pl->L.dag, pl->geomDag, A, stream);
+        e = launchDag(*pl.L.dag, pl.geomDag, A, stream);
         h->lastKernel = AVDSP_B200_KERNEL_DAG;
     } else if (use == AVDSP_B200_KERNEL_CHAIN) {
         Chain2Args A{};
-        A.in = in; A.out = out; A.state = st; A.lanes = pl->dLanes2;
+        A.in = in; A.out = out; A.state = st; A.lanes = pl.dLanes2;
         A.nStreams = n; A.nFrames = nFrames;
         A.inStreamStride = inSS; A.outStreamStride = outSS;
         A.inFrameStride = inFS; A.inChStride = inCS; A.outFrameStride = outFS; A.outChStride = outCS;
@@ -645,14 +642,14 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         // against v2's 9.50; with whole 6- and 8-section cascades per warp v3 is the slower one) and the call is long enough to
         // pay for v3's pipeline fill and drain (parts run a tile behind each other: C2 breaks even near 1500 frames per call --
         // 128 frames: v2 0.083 ms / v3 0.117, 1024: 0.262 / 0.267, 4096: 0.864 / 0.816); everything else runs on v2
-        const bool v3Ok = pl->chain3Usable && use == AVDSP_B200_KERNEL_CHAIN;
+        const bool v3Ok = pl.chain3Usable && use == AVDSP_B200_KERNEL_CHAIN;
         static const int envChain3 = [] { const char* v = getenv("AVDSP_B200_CHAIN3"); return (v && *v) ? atoi(v) : -1; }();
         bool v3 = v3Ok && h->kernelSel != AVDSP_B200_KERNEL_CHAIN_V2 &&
                   (h->kernelSel == AVDSP_B200_KERNEL_CHAIN_V3 || envChain3 == 1 ||
-                   (envChain3 != 0 && pl->geom3.maxSec <= 4 && pl->geom3.streamsPerCta >= 16 && nFrames >= std::max(1536, 32 * pl->geom3.gmax)));
+                   (envChain3 != 0 && pl.geom3.maxSec <= 4 && pl.geom3.streamsPerCta >= 16 && nFrames >= std::max(1536, 32 * pl.geom3.gmax)));
         if (h->kernelSel == AVDSP_B200_KERNEL_CHAIN_V3 && !v3)
             return setErr(AVDSP_B200_ERR_UNSUPPORTED, "chain kernel v3 requested but the program shape does not map to it");
-        const bool flt = pl->L.chain.h.aluClass == ALU_F32;
+        const bool flt = pl.L.chain.h.aluClass == ALU_F32;
         if (flt) {
             // the float class is the reference's arithmetic except next to the underflow threshold and beyond the binary32 range
             // (avdsp_dev.cuh, fltGuard): snapshot the state, let the cascades flag the streams that came near either, then list
@@ -668,17 +665,17 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
             if (e != cudaSuccess) return cudaErr(e, "kernel launch");
             A.redo = h->dRedo + first;
         }
-        if (v3) e = launchChain3(pl->L.chain, pl->geom3, A, stream);
-        else e = launchChain2(pl->L.chain, pl->geom2, A, stream);
+        if (v3) e = launchChain3(pl.L.chain, pl.geom3, A, stream);
+        else e = launchChain2(pl.L.chain, pl.geom2, A, stream);
         if (flt && e == cudaSuccess) {
             e = launchRedoCompact(h->dRedo + first, n, h->dRedoList + first, h->dRedoCount + first, st, h->dSnap + (size_t)first * P.stateWords, P.stateWords, stream);
             if (e == cudaSuccess) {
                 Chain2Args X = A;
-                X.lanes = pl->dLanes2; X.redo = nullptr;
+                X.lanes = pl.dLanes2; X.redo = nullptr;
                 X.map = h->dRedoList + first; X.countPtr = h->dRedoCount + first; X.exact = 1;
-                Chain2Geom gx = pl->geom2;
+                Chain2Geom gx = pl.geom2;
                 gx.floatFast = 0;                                // sources through the restatement as well
-                e = launchChain2(pl->L.chain, gx, X, stream);
+                e = launchChain2(pl.L.chain, gx, X, stream);
             }
             h->launches += 3;
         }
@@ -686,14 +683,14 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
         h->lastKernel = AVDSP_B200_KERNEL_CHAIN;
     } else {
         GenericArgs A{};
-        A.in = in; A.out = out; A.state = st; A.bigPool = pl->dBig;
+        A.in = in; A.out = out; A.state = st; A.bigPool = pl.dBig;
         A.nStreams = n; A.nFrames = nFrames;
         A.inStreamStride = inSS; A.outStreamStride = outSS;
         A.inFrameStride = inFS; A.inChStride = inCS; A.outFrameStride = outFS; A.outChStride = outCS;
         A.coreSel = coreSel; A.period = coreSel >= 0 ? 0 : h->period;
-        A.coefs = planOverride ? nullptr : coefs; A.coefPitch = h->nStreams; A.coefStep = 5 * pl->L.nFreq;
-        A.firTaps = planOverride ? nullptr : firTaps; A.firPitch = nTapCols; A.firCol = pl->dFirCol;
-        for (int c = 0; c < P.nCores && c < kMaxCores; c++) { A.coreInMask[c] = pl->L.cores[c].usedIn; A.coreOutMask[c] = pl->L.cores[c].usedOut; }
+        A.coefs = planOverride ? nullptr : coefs; A.coefPitch = h->nStreams; A.coefStep = 5 * pl.L.nFreq;
+        A.firTaps = planOverride ? nullptr : firTaps; A.firPitch = nTapCols; A.firCol = pl.dFirCol;
+        for (int c = 0; c < P.nCores && c < kMaxCores; c++) { A.coreInMask[c] = pl.L.cores[c].usedIn; A.coreOutMask[c] = pl.L.cores[c].usedOut; }
         e = launchGeneric(G, A, stream);
         h->lastKernel = AVDSP_B200_KERNEL_GENERIC;
     }
@@ -710,11 +707,11 @@ static int launchRun(avdsp_b200* h, avdsp_b200* pl, const int* in, int* out, int
 // launch's time.  Variants whose kernels share per-instance scratch (dither rows of the mix kernel, FIR workspace) stay in order.
 static int launchRange(avdsp_b200* h, const int* in, int* out, int nFrames, int layout, int first, int n,
                        cudaStream_t stream, int coreSel = -1, const GenericPlan* planOverride = nullptr, int cap = 0) {
-    if (h->variantOf.empty() || planOverride) return launchRun(h, h, in, out, nFrames, layout, first, n, stream, coreSel, planOverride, cap);
+    if (h->variantOf.empty() || planOverride) return launchRun(h, *h, in, out, nFrames, layout, first, n, stream, coreSel, planOverride, cap);
     const PlanHeader& P = h->L.gen.h;
     const size_t c = (size_t)(cap > 0 ? cap : nFrames);
     bool fork = !(h->mixUsable || h->firUsable);
-    for (const avdsp_b200* v : h->variants) fork = fork && !(v->mixUsable || v->firUsable);
+    for (const auto& v : h->variants) fork = fork && !(v->mixUsable || v->firUsable);
     int nRuns = 0;
     for (int a = first; a < first + n; nRuns++) { const int v = h->variantOf[a]; while (a < first + n && h->variantOf[a] == v) a++; }
     fork = fork && nRuns > 1;
@@ -740,7 +737,7 @@ static int launchRange(avdsp_b200* h, const int* in, int* out, int nFrames, int 
             s = h->varStream[run % avdsp_b200::kVarStreams];
             if (run < avdsp_b200::kVarStreams) CU(cudaStreamWaitEvent(s, h->evFork, 0));
         }
-        const int r = launchRun(h, v ? h->variants[v - 1] : h, in ? in + off * P.nIn : in, out ? out + off * P.nOut : out, nFrames, layout,
+        const int r = launchRun(h, v ? *h->variants[v - 1] : *h, in ? in + off * P.nIn : in, out ? out + off * P.nOut : out, nFrames, layout,
                                 a, b - a, s, coreSel, nullptr, cap, !fork);
         if (r < 0) return r;
         a = b;
@@ -896,11 +893,9 @@ static int shardOf(const avdsp_b200* h, int stream) {
 }
 static int resetShards(avdsp_b200* h, int fs, const int32_t* seeds, int defaultDither) {
     if (fs != h->L.fs || defaultDither != h->L.defaultDither) {
-        Lowered nl; std::string err;
-        const std::vector<int32_t> words = h->L.words;
-        const int rc = decodeProgram(words.data(), (int)words.size(), 0x7FFFFFFF, h->L.format, fs, defaultDither, &nl, &err);
-        if (rc < 0) return setErr(rc, err);
-        h->L = nl;
+        Lowered nl;
+        const int rc = decodeAt(*h, fs, defaultDither, &nl); if (rc < 0) return rc;
+        h->L = std::move(nl);
     }
     if (seeds) h->seeds.assign(seeds, seeds + h->nStreams); else h->seeds.clear();
     return forShards(h, [&](int k, avdsp_b200* sh) { return avdsp_b200_reset(sh, fs, seeds ? seeds + h->shardFirst[k] : nullptr, defaultDither); });
@@ -1077,24 +1072,18 @@ int avdsp_b200_process_pcm(avdsp_b200_t* h, const void* in, int pcmFormat, void*
 } // extern "C"
 
 // ---- per-stream parameter overrides (SURVEY.md 8f-3; the dump-file workflow per stream) -------------------------------
-static void dropVariants(avdsp_b200* h) {
-    for (avdsp_b200* v : h->variants) freeAll(v);
-    h->variants.clear();
-    h->variantOf.clear();
-}
 // plans for `words` (the loaded program with some PARAM words replaced): an existing variant with exactly these words, or a new one
 static int variantFor(avdsp_b200* h, const std::vector<int32_t>& words, int* id) {
     if (words == h->L.words) { *id = 0; return 0; }
     for (size_t k = 0; k < h->variants.size(); k++) if (h->variants[k]->L.words == words) { *id = (int)k + 1; return 0; }
-    std::unique_ptr<avdsp_b200, void (*)(avdsp_b200*)> v(new avdsp_b200, freeAll);
-    v->device = h->device; v->numSMs = h->numSMs; v->nStreams = h->nStreams;
+    std::unique_ptr<Plans> v(new Plans);
     v->L = h->L;
     std::string err;
     const int rc = relowerProgram(words.data(), (int)words.size(), &v->L, &err);       // same opcode structure, same state layout, else an error
     if (rc < 0) return setErr(rc, err);
-    const int r = uploadPlanData(v.get());
+    const int r = uploadPlanData(*v, h->device, h->nStreams, h->numSMs);
     if (r < 0) return r;
-    h->variants.push_back(v.release());
+    h->variants.push_back(std::move(v));
     *id = (int)h->variants.size();
     return 0;
 }
@@ -1163,7 +1152,7 @@ static int setRows(avdsp_b200* h, StreamTable avdsp_b200::* tab, const char* ref
     if (!h->shards.empty() && memspace != AVDSP_B200_HOST)
         return setErr(AVDSP_B200_ERR_UNSUPPORTED, std::string("a multi-device instance takes HOST ") + t.noun + " rows (device buffers belong to one GPU)");
     for (const avdsp_b200* o : h->shards.empty() ? std::vector<avdsp_b200*>{h} : h->shards)
-        for (const avdsp_b200* v : o->variants)
+        for (const auto& v : o->variants)
             if (v->L.*t.words != cols) return setErr(AVDSP_B200_ERR_UNSUPPORTED, std::string("a parameter variant moved the ") + t.noun + " words");
     if (!h->shards.empty())
         return forShards(h, [&](int k, avdsp_b200* sh) {
@@ -1257,10 +1246,7 @@ int avdsp_b200_set_param(avdsp_b200_t* h, int firstStream, int nStreams, int wor
     std::map<int, int> moved;                 // old variant -> new variant
     if (anyVariantWord) {
         const size_t nBefore = h->variants.size();
-        auto undo = [&](int rc) {             // release the variants this call created; nothing else has changed yet
-            while (h->variants.size() > nBefore) { freeAll(h->variants.back()); h->variants.pop_back(); }
-            return rc;
-        };
+        auto undo = [&](int rc) { h->variants.resize(nBefore); return rc; };    // release the variants this call created; nothing else has changed yet
         for (int s = firstStream; s < firstStream + nStreams; s++) {
             const int old = h->variantOf.empty() ? 0 : h->variantOf[s];
             if (moved.count(old)) continue;
@@ -1301,11 +1287,9 @@ int avdsp_b200_set_param(avdsp_b200_t* h, int firstStream, int nStreams, int wor
     std::vector<int> used(h->variants.size() + 1, 0);
     for (int v : h->variantOf) used[v] = 1;
     std::vector<int> remap(h->variants.size() + 1, 0);
-    std::vector<avdsp_b200*> keep;
-    for (size_t k = 0; k < h->variants.size(); k++) {
-        if (used[k + 1]) { keep.push_back(h->variants[k]); remap[k + 1] = (int)keep.size(); }
-        else freeAll(h->variants[k]);
-    }
+    std::vector<std::unique_ptr<Plans>> keep;
+    for (size_t k = 0; k < h->variants.size(); k++)
+        if (used[k + 1]) { keep.push_back(std::move(h->variants[k])); remap[k + 1] = (int)keep.size(); }
     h->variants.swap(keep);
     bool any = false;
     for (int& v : h->variantOf) { v = remap[v]; any = any || v != 0; }
@@ -1348,13 +1332,14 @@ int avdsp_b200_reload_params(avdsp_b200_t* h, const int32_t* prog, int progWords
         return r < 0 ? r : rc;
     }
     { const int q = quiesce(h); if (q < 0) return q; }
-    dropVariants(h);                                          // a new program for everybody: per-stream overrides start over
+    h->variants.clear();                                      // a new program for everybody: per-stream overrides start over
+    h->variantOf.clear();
     freeTable(h->coefTab);                                    // ... the tables too
     freeTable(h->firTab);
     if (h->dFirFlags) { cudaFree(h->dFirFlags); h->dFirFlags = nullptr; }
     if (h->dFirTcPer) { cudaFree(h->dFirTcPer); h->dFirTcPer = nullptr; }
     h->firTcPerValid = h->firTcPerFailed = false;
-    const int r = uploadPlanData(h);
+    const int r = uploadPlanData(*h, h->device, h->nStreams, h->numSMs);
     return r < 0 ? r : rc;
 }
 

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <map>
+#include <memory>
 #include <string>
 #include <vector>
 #include "../../include/avdsp_b200.h"
@@ -21,16 +22,12 @@ struct StreamTable {
     size_t colStride(size_t nStreams) const { return streamMajor ? 1 : nStreams; }
 };
 
-struct avdsp_b200 {
-    int device = 0, numSMs = 148;
-    int nStreams = 0;
+// What one program word list needs on one device: its lowering, the kernels that can take it and their plan data there.  Owns
+// its buffers (no copies), freed on the device uploadPlanData put them on; one that never uploaded makes no CUDA call (describe).
+struct Plans {
     avdsp::Lowered L;
-    std::vector<int32_t> seeds;
-    int* dState = nullptr;
     int* dBig = nullptr; size_t bigWords = 0;
     int* dFirCol = nullptr;         // L.firColOfOp on the device: the FIR-table column of each micro-op (k_generic with a FIR table)
-    int* dMemInit = nullptr;
-    int* dSeeds = nullptr;
     avdsp::ChainLane* dLanes2 = nullptr;
     avdsp::Chain2Geom geom2{};
     bool chain2Usable = false;      // kernel_chain2.cu (v2: warp-specialised, the default)
@@ -38,12 +35,31 @@ struct avdsp_b200 {
     bool chain3Usable = false;      // kernel_chain3.cu (v3: one cascade per lane; the common crossover / EQ shape at batch width)
     avdsp::DagGeom geomDag{};
     bool dagUsable = false;         // kernel_dag.cu (X/Y dataflow programs: a DAG of cascades, node per warp)
-    int lastChainVariant = 0;       // 2 / 3: which chain kernel the last AVDSP_B200_KERNEL_CHAIN launch used
     avdsp::MixPlan mix{};
     bool mixUsable = false;         // kernel_mix.cu (time-parallel: programs without biquads)
     bool firUsable = false;         // kernel_fir.cu (time-parallel FIR paths)
     unsigned char* dFirTaps = nullptr;              // kernel_fir_tc.cu: pre-swizzled Toeplitz taps blobs
-    unsigned char* dFirWs = nullptr; size_t firWsBytes = 0;     // ... and the packed-sample workspace
+    std::string trace;
+    int planDevice = -1;            // where the buffers above live (-1: nothing uploaded)
+    Plans() = default;
+    Plans(const Plans&) = delete; Plans& operator=(const Plans&) = delete;
+    ~Plans() {
+        if (planDevice < 0) return;
+        cudaSetDevice(planDevice);
+        cudaFree(dBig); cudaFree(dFirCol); cudaFree(dLanes2); cudaFree(dFirTaps);       // cudaFree(nullptr) does nothing
+    }
+};
+
+// An instance is its program's plans plus the streams that run them.
+struct avdsp_b200 : Plans {
+    int device = 0, numSMs = 148;
+    int nStreams = 0;
+    std::vector<int32_t> seeds;
+    int* dState = nullptr;
+    int* dMemInit = nullptr;
+    int* dSeeds = nullptr;
+    int lastChainVariant = 0;       // 2 / 3: which chain kernel the last AVDSP_B200_KERNEL_CHAIN launch used
+    unsigned char* dFirWs = nullptr; size_t firWsBytes = 0;     // kernel_fir_tc.cu: the packed-sample workspace
     unsigned* dJump = nullptr; int jumpL = -1;      // PRNG jump matrix for segments of jumpL draws
     int* dTpdf = nullptr; size_t tpdfWords = 0;     // scratch dither values of a launch
     // float class of the chain kernels: per-stream "re-execute me exactly" flags and the state snapshot the interpreter's second
@@ -64,16 +80,15 @@ struct avdsp_b200 {
     size_t slotInWords = 0, slotOutWords = 0;
     cudaEvent_t evIn[kSlots] = {nullptr, nullptr, nullptr}, evKernel[kSlots] = {nullptr, nullptr, nullptr}, evOut[kSlots] = {nullptr, nullptr, nullptr};
     void* pcmRaw = nullptr; int* pcmIn = nullptr; int* pcmOut = nullptr; size_t pcmRawBytes = 0, pcmInWords = 0, pcmOutWords = 0;
-    std::string trace;
     // multi-device instance (avdsp_b200_create_multi): this object only carries the decoded program; the streams live in
     // one single-device instance per GPU, contiguous balanced ranges (stream s of the whole = stream s - shardFirst[k] of shard k)
     std::vector<avdsp_b200*> shards;
     std::vector<int> shardFirst;       // [nShards + 1]
-    // per-stream parameter overrides (avdsp_b200_set_param): variantOf[s] == 0: the program as loaded, v > 0: variants[v - 1],
-    // an object of this type that only carries plans (own L, dBig, dLanes2, dFirTaps, geometries) for the patched words.
-    // Empty variantOf: no override anywhere.  Streams keep their state blocks whatever variant they run.
+    // per-stream parameter overrides (avdsp_b200_set_param): variantOf[s] == 0: the program as loaded, v > 0: the plans of the
+    // patched words in variants[v - 1].  Empty variantOf: no override anywhere.  Streams keep their state blocks whatever variant
+    // they run.  A variant is released only once the instance is quiesced (quiesce, freeAll): launches read its plan data.
     std::vector<int> variantOf;
-    std::vector<avdsp_b200*> variants;
+    std::vector<std::unique_ptr<Plans>> variants;
     // runs of streams on different variants are independent launches: they go out on a few forked streams and join the caller's
     static constexpr int kVarStreams = 32;
     cudaStream_t varStream[kVarStreams] = {};

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN, load_program
-from avdsp_b200 import Executor, AvdspError, synth, params, KERNEL_GENERIC, KERNEL_AUTO
+from avdsp_b200 import Executor, AvdspError, synth, params, coef_words, KERNEL_GENERIC, KERNEL_AUTO
 from oracle import wire
 
 pytestmark = pytest.mark.gpu
@@ -139,3 +139,34 @@ def test_dump_file_symbols_on_c1(oracle_lib):
         o = oracle_lib.Oracle(mine if s == 3 else w, 2, fs, seed=s, dither=24)
         assert np.array_equal(y[s], o.process(x[s])), s
     assert not np.array_equal(y[3], oracle_lib.Oracle(w, 2, fs, seed=3, dither=24).process(x[3]))
+
+
+def test_reset_to_another_rate_replans_every_variant(oracle_lib):
+    """three blocks of streams on three parameter sets (the loaded program and two variants), reset through the lowest, the
+    highest and again the lowest rate of a multi-rate program: every variant's plans follow the rate"""
+    base = load_program("c2_testrpi_xover_f2_multifs")
+    hd = wire.header(base.view(np.uint32))
+    lo, hi = wire.FREQS[hd["freqMin"]], wire.FREQS[hd["freqMax"]]
+    S, T, blk = 24, 400, 8
+    cw = coef_words(base, 2)
+    ff = cw[(np.arange(len(cw)) % 5 < 3) & (base[cw] != 0)]         # b0 b1 b2 of every section, every fs column
+    rng = np.random.default_rng(29)
+    progs = [base]
+    for _ in range(2):
+        p = base.copy()
+        p[ff] += rng.integers(-64, 65, len(ff)).astype(np.int32)
+        progs.append(p)
+    seeds = np.arange(S, dtype=np.int32)
+    ex = Executor(base, hi, 2, S, seeds=seeds, dither=24)
+    for b in (1, 2):
+        apply_diff(ex, b * blk, blk, base, progs[b])
+    assert ex.num_variants == 3
+    for fs in (lo, hi, lo):
+        ex.reset(fs, seeds=seeds, dither=24)
+        assert ex.num_variants == 3
+        x = synth.pcm("noise", S, T, ex.n_in, fs)
+        y = ex.process(x)
+        for s in range(S):
+            o = oracle_lib.Oracle(progs[s // blk], 2, fs, seed=s, dither=24)
+            assert np.array_equal(y[s], o.process(x[s])), (fs, s)
+            assert np.array_equal(ex.get_state(s)[: ex.data_size], o.data), (fs, s)
