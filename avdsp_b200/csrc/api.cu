@@ -194,10 +194,17 @@ static void planGeometries(Plans& p, int nStreams, int numSMs, std::vector<Chain
         snprintf(line, sizeof line, "chain kernel v3 geometry: %d streams/CTA (lane = one cascade part of one stream), %d cascade warps of <= %d sections + 1 dither warp + %d store warps, largest lag %d frames, row ring %d steps, %zu B smem; parts (chain:first+n@base):",
                  p.geom3.streamsPerCta, p.geom3.nCascade, p.geom3.maxSec, p.geom3.nStore, p.geom3.gmax, p.geom3.postRing, p.geom3.smemBytes);
         p.trace += line;
+        int macs = 0, algMacs = 0, unitSecs = 0;
         for (int w = 0; w < p.geom3.nCascade; w++) {
-            snprintf(line, sizeof line, " %d:%d+%d@%d", p.geom3.warpChain[w], p.geom3.warpFirstSec[w], p.geom3.warpNsec[w], p.geom3.warpBase[w]);
+            snprintf(line, sizeof line, " %d:%d+%d@%d%s", p.geom3.warpChain[w], p.geom3.warpFirstSec[w], p.geom3.warpNsec[w], p.geom3.warpBase[w],
+                     p.geom3.warpUnit[w] ? "u" : "");
             p.trace += line;
+            algMacs += 5 * p.geom3.warpNsec[w];
+            macs += (p.geom3.warpUnit[w] ? 2 : 5) * p.geom3.warpNsec[w];
+            if (p.geom3.warpUnit[w]) unitSecs += p.geom3.warpNsec[w];
         }
+        snprintf(line, sizeof line, "; unit-gain form (u) on %d sections: %d IMAD.WIDE per frame executed, %d algorithmic", unitSecs, macs, algMacs);
+        p.trace += line;
         p.trace += "; sub-partitions (sections of the cascade warps on hardware warps q, q+4, ..; d = dither warp, s = store warp):";
         for (int q = 0; q < 4; q++) {
             p.trace += q ? " |" : " ";

@@ -156,6 +156,55 @@ __device__ __forceinline__ long long cascStepExact(Casc<NSEC>& L, int xin, int t
     return last;
 }
 
+// Unit-gain form (DESIGN.md 4.2a).  A section with b0 = 2^28, b1 + a1 = -2^28, b2 + a2 = 0 (as integers: the 0 dB peaking slots of a
+// crossover) satisfies, exactly over the integers and so in Z/2^64,
+//     b0 x + b1 x1 + b2 x2 + a1 y1 + a2 y2 = 2^28 (x - x1) + a1 (y1 - x1) + a2 (y2 - x2).
+// The part carries z = acc - 2^28 x (x = the section's input of that frame): the 2^28 term telescopes away and
+//     z_n = z_{n-1} + a1 d_{n-1} + a2 d_{n-2},   d = y - x = z >> 28,   y_n = x_n + (int)(z_n >> 28)
+// (2^28 x has no low bits, so acc >> 28 = x + (z >> 28)): 2 MACs instead of 5, no shift of x, no 33-bit difference.
+// That is the reference's arithmetic as long as (a) d fits 32 bits, so that the MAC operand is d itself, and (b) no section saturates,
+// so that acc >> 28 is y.  Tiles run optimistically on two sticky records and are replayed exactly when either fires:
+//   * hi32(z) in [-2^20, 2^20)  =>  |d| < 2^24;
+//   * the part's input x0 in [-(2^31 - 2^27), 2^31 - 2^27].  Section k's input is x0 plus the d of the k sections before it, so every
+//     input and output of the part lies within 2^31 - 2^27 + 4 * 2^24 < 2^31 - 32: x + d cannot wrap, and acc >> 28 = y stays inside
+//     [-2^31 + 32, 2^31 - 1], the range in which checkbiquadsat (hi32(acc) = (acc >> 28) >> 4 in [-2^27 + 2, 2^27 - 1]) never clamps.
+// Both tests are stricter than the reference's clamp: a false alarm costs a replay, never a wrong sample.  A unit section is a
+// pass-through plus a rounding residue, so on any but near-full-scale input neither record fires.
+constexpr unsigned kUnitZBias = 1u << 20, kUnitZLimit = (1u << 21) - 1u;           // (unsigned)(hi32(z) + bias) <= limit
+constexpr unsigned kUnitXBias = 0x78000000u, kUnitXLimit = 2u * 0x78000000u;        // (unsigned)(x0 + bias) <= limit
+
+__device__ __forceinline__ bool unitSection(int b0, int b1, int b2, int a1, int a2) {
+    return b0 == (1 << kMantBQ) && (long long)b1 + a1 == -(1ll << kMantBQ) && (long long)b2 + a2 == 0;
+}
+template <int NSEC>
+struct CascU { long long z[NSEC]; int d1[NSEC], d2[NSEC]; };
+
+// one step of a unit-gain part, every section active, optimistic (records only).  Keeps the y / X histories of Casc as they are, so
+// that the part leaves the tile in the general layout; returns the accumulator of the last section (frame t - (NSEC-1)).
+template <int NSEC>
+__device__ __forceinline__ long long unitStep(Casc<NSEC>& L, CascU<NSEC>& U, int xin, unsigned& w0, unsigned& w1, unsigned& wx) {
+    long long z[NSEC];
+#pragma unroll
+    for (int k = 0; k < NSEC; k++) z[k] = mac32(U.z[k], U.d1[k], L.a1[k]);
+#pragma unroll
+    for (int k = 0; k < NSEC; k++) z[k] = mac32(z[k], U.d2[k], L.a2[k]);
+    int y[NSEC];
+#pragma unroll
+    for (int k = 0; k < NSEC; k++) {
+        const int s = q59ToS31(z[k]);
+        if (k & 1) w1 = max(w1, (unsigned)hi32(z[k]) + kUnitZBias);
+        else       w0 = max(w0, (unsigned)hi32(z[k]) + kUnitZBias);
+        y[k] = (k ? L.y1[k - 1] : xin) + s;
+        U.z[k] = z[k]; U.d2[k] = U.d1[k]; U.d1[k] = s;
+    }
+    const int inLast = NSEC > 1 ? L.y1[NSEC - 2] : xin;
+    wx = max(wx, (unsigned)xin + kUnitXBias);
+#pragma unroll
+    for (int k = 0; k < NSEC; k++) { L.y3[k] = L.y2[k]; L.y2[k] = L.y1[k]; L.y1[k] = y[k]; }
+    L.X2 = L.X1; L.X1 = xin;
+    return z[NSEC - 1] + (long long)((unsigned long long)(long long)inLast << kMantBQ);
+}
+
 // SAT0DB_TPDF on the cascade's accumulator (dsp_runtime.c:478-491, dspTpdfApply runtime/dsp_tpdf.h:141-145)
 __device__ __forceinline__ int finishTpdf3(long long acc, int tv, bool up, int sh) {
     const long long t = tv;
@@ -214,6 +263,16 @@ __device__ __forceinline__ void cascadeWarp(const ChainPlan& P, const Chain2Args
             if (k == 0) { L.X1 = q[2]; L.X2 = q[3]; }
         }
     }
+    // the unit-gain form needs every section of every lane's stream to satisfy the identity (a per-stream coefficient table may
+    // break it for some streams: then the whole warp runs the general form).  Parts of 3 and 4 sections only.
+    constexpr bool kUnitForm = CKREG && NSEC >= 3;
+    bool unit = false;
+    if constexpr (kUnitForm) {
+        bool ok = true;
+#pragma unroll
+        for (int k = 0; k < NSEC; k++) ok = ok && unitSection(L.b0[k], L.b1[k], L.b2[k], L.a1[k], L.a2[k]);
+        unit = __all_sync(0xffffffffu, ok);
+    }
     // delay line (dsp_runtime.c:769-794): ring of n samples, frame f swaps with position (idx0+f) mod n, so the output of frame
     // f is the post value of frame f-n.  The post ring IS the delay line: the n samples the reference ring holds are preloaded
     // as "virtual frames" -n..-1.  A stale index idx0 >= n (delay shortened by reload_params) is used once by the reference
@@ -266,32 +325,72 @@ __device__ __forceinline__ void cascadeWarp(const ChainPlan& P, const Chain2Args
                 }
                 ck[(5 * NSEC) * CKP] = L.X1; ck[(5 * NSEC + 1) * CKP] = L.X2;
             }
-            unsigned w0 = 0, w1 = 0;
+            unsigned w0 = 0, w1 = 0, wx = 0;
             unsigned rj = ra;
             unsigned pj = postRow + (fin ? ((unsigned)(t0 & RM) << 2) : (unsigned)((i % 3) * F3) * 4u);
             unsigned tj = (unsigned)((t0 - LAGA) << 2);
-            // one step; jj is a compile-time offset inside the unrolled group
-            auto step = [&](int jj) {
-                const int smp = lds3(rj); rj += rstep;
-                const int x = (MODE & 1) ? smp : q59ToS31(mul32(smp, gain));
-                const long long acc = cascStep<NSEC>(L, x, w0, w1);
-                int v;
-                if (MODE & 2) v = finishTpdf3(acc, lds3(tpdfRow + ((tj + 4u * jj) & TM4)), tpdfUp, tpdfSh);
-                else v = q59ToS31(acc);        // SAT0DB of a clamped accumulator is its own >> 28 (replayed exactly if a clamp fired)
-                if (live) sts3(pj + 4u * jj, v);
-            };
-            // groups of AVDSP_UNR3 steps: 6 = lcm of the history depths (y1..y3, X1..X2), so the register rotation closes on itself
-            // and the loop needs no moves (they would be IMAD.MOVs on the very pipe the MACs saturate); the tile's last steps follow
-            constexpr int kMain = (F3 / AVDSP_UNR3) * AVDSP_UNR3;
+            // groups of AVDSP_UNR3 steps: 6 = lcm of the history depths (y1..y3, X1..X2, d1..d2), so the register rotation closes on
+            // itself and the loop needs no moves (they would be IMAD.MOVs on the very pipe the MACs saturate); the tile's last steps
+            // follow.  step(jj, x) runs one step on input x and returns the value the part writes; jj is a compile-time offset.
+            auto runTile = [&](auto&& step) {
+                auto one = [&](int jj) {
+                    const int smp = lds3(rj); rj += rstep;
+                    const int v = step(jj, (MODE & 1) ? smp : q59ToS31(mul32(smp, gain)));
+                    if (live) sts3(pj + 4u * jj, v);
+                };
+                constexpr int kMain = (F3 / AVDSP_UNR3) * AVDSP_UNR3;
 #pragma unroll 1
-            for (int j0 = 0; j0 < kMain; j0 += AVDSP_UNR3) {
+                for (int j0 = 0; j0 < kMain; j0 += AVDSP_UNR3) {
 #pragma unroll
-                for (int jj = 0; jj < AVDSP_UNR3; jj++) step(jj);
-                pj += 4u * AVDSP_UNR3; tj += 4u * AVDSP_UNR3;
+                    for (int jj = 0; jj < AVDSP_UNR3; jj++) one(jj);
+                    pj += 4u * AVDSP_UNR3; tj += 4u * AVDSP_UNR3;
+                }
+#pragma unroll
+                for (int jj = 0; jj < F3 - kMain; jj++) one(jj);
+            };
+            bool fired;
+            if constexpr (kUnitForm) {
+                // unit-gain part: enter the z form from the checkpointed state.  The first step needs d1 = y1 - x1 and d2 = y2 - x2
+                // exactly in 32 bits, and the inputs already inside the skewed pipeline within the x0 bound; else this tile runs exact.
+                CascU<NSEC> U;
+                bool entry = true;
+                if (unit) {
+#pragma unroll
+                    for (int k = 0; k < NSEC; k++) {
+                        const int xp1 = k ? L.y2[k - 1] : L.X1, xp2 = k ? L.y3[k - 1] : L.X2;
+                        const long long e1 = (long long)L.y1[k] - xp1, e2 = (long long)L.y2[k] - xp2;
+                        U.z[k] = L.acc[k] - (long long)((unsigned long long)(long long)xp1 << kMantBQ);
+                        U.d1[k] = (int)e1; U.d2[k] = (int)e2;
+                        entry = entry && e1 == (long long)(int)e1 && e2 == (long long)(int)e2;
+                        if (k < NSEC - 1) entry = entry && (unsigned)L.y1[k] + kUnitXBias <= kUnitXLimit;
+                    }
+                    entry = __all_sync(0xffffffffu, entry);
+                }
+                if (unit && !entry) {
+                    fired = true;
+                } else if (unit) {
+                    runTile([&](int jj, int x) {
+                        const long long acc = unitStep<NSEC>(L, U, x, w0, w1, wx);
+                        if (MODE & 2) return finishTpdf3(acc, lds3(tpdfRow + ((tj + 4u * jj) & TM4)), tpdfUp, tpdfSh);
+                        return L.y1[NSEC - 1];
+                    });
+                    fired = __any_sync(0xffffffffu, max(w0, w1) > kUnitZLimit || wx > kUnitXLimit);
+                    if (!fired) {                           // back to the general layout: acc = z + 2^28 * (the section's last input)
+#pragma unroll
+                        for (int k = 0; k < NSEC; k++)
+                            L.acc[k] = U.z[k] + (long long)((unsigned long long)(long long)(k ? L.y2[k - 1] : L.X1) << kMantBQ);
+                    }
+                }
             }
-#pragma unroll
-            for (int jj = 0; jj < F3 - kMain; jj++) step(jj);
-            if (__any_sync(0xffffffffu, max(w0, w1) > kSatLimit3)) {
+            if (!kUnitForm || !unit) {
+                runTile([&](int jj, int x) {
+                    const long long acc = cascStep<NSEC>(L, x, w0, w1);
+                    if (MODE & 2) return finishTpdf3(acc, lds3(tpdfRow + ((tj + 4u * jj) & TM4)), tpdfUp, tpdfSh);
+                    return q59ToS31(acc);      // SAT0DB of a clamped accumulator is its own >> 28 (replayed exactly if a clamp fired)
+                });
+                fired = __any_sync(0xffffffffu, max(w0, w1) > kSatLimit3);
+            }
+            if (fired) {
                 if (CKREG) {
 #pragma unroll
                     for (int k = 0; k < NSEC; k++) { L.acc[k] = cAcc[CKREG ? k : 0]; L.y1[k] = cY1[CKREG ? k : 0]; L.y2[k] = cY2[CKREG ? k : 0]; L.y3[k] = cY3[CKREG ? k : 0]; }
@@ -953,7 +1052,7 @@ bool planChain3Geometry(const ChainPlan& plan, int nStreams, int numSMs, Chain3G
     for (int partMax : {envInt3("AVDSP_B200_PART3", 4), 8}) {
         if (partMax < 1 || partMax > 8) continue;
         if (plan.h.aluClass == ALU_F32 && partMax > 4) continue;      // the float form exists for parts of <= 4 sections
-        struct Part { int chain, first, nsec, base, src, fin; };
+        struct Part { int chain, first, nsec, base, src, fin, unit; };
         Part parts[kChain3MaxWarps];
         int nParts = 0, gmax = 0, maxSec = 0;
         bool fits = true;
@@ -967,7 +1066,13 @@ bool planChain3Geometry(const ChainPlan& plan, int nStreams, int numSMs, Chain3G
             for (int p = 0; p < np; p++) {
                 if (nParts >= kChain3MaxWarps) { fits = false; break; }
                 const int n = nsec / np + (p < nsec % np ? 1 : 0);          // near-equal parts, the longer ones first
-                parts[nParts] = {c, first, n, base, prev, p == np - 1};
+                // the unit-gain form exists for the fixed-point parts of 3 and 4 sections (register checkpoint: partMax <= 4)
+                bool unit = plan.h.aluClass == ALU_INT64 && partMax <= 4 && n >= 3;
+                for (int k = first; k < first + n && unit; k++) {
+                    const int32_t* cf = plan.pool + plan.chains[c].coefOff + 5 * k;
+                    unit = cf[0] == (1 << kMantBQ) && (long long)cf[1] + cf[3] == -(1ll << kMantBQ) && (long long)cf[2] + cf[4] == 0;
+                }
+                parts[nParts] = {c, first, n, base, prev, p == np - 1, unit ? 1 : 0};
                 prev = nParts++;
                 first += n;
                 maxSec = std::max(maxSec, n);
@@ -1014,7 +1119,7 @@ bool planChain3Geometry(const ChainPlan& plan, int nStreams, int numSMs, Chain3G
                 order[k] = k;
                 if (k >= nParts) { itemCost[k] = 8; continue; }              // helper warps: k == nParts dither, then store
                 const ChainDesc& d = plan.chains[parts[k].chain];
-                itemCost[k] = 5 * parts[k].nsec + 2;
+                itemCost[k] = (parts[k].unit ? 4 : 5) * parts[k].nsec + 2;
                 if (parts[k].fin && (d.satKind & 1)) itemCost[k] += 6;
                 if (parts[k].src < 0 && !(d.srcKind == SRC_LOAD_GAIN && d.srcArg == (1 << kMant))) itemCost[k] += 2;
             }
@@ -1060,6 +1165,7 @@ bool planChain3Geometry(const ChainPlan& plan, int nStreams, int numSMs, Chain3G
                 const int w = slotOf[k];
                 g.warpChain[w] = parts[k].chain; g.warpFirstSec[w] = parts[k].first; g.warpNsec[w] = parts[k].nsec;
                 g.warpBase[w] = parts[k].base; g.warpSrc[w] = parts[k].src >= 0 ? slotOf[parts[k].src] : -1; g.warpFinal[w] = parts[k].fin;
+                g.warpUnit[w] = parts[k].unit;
                 if (parts[k].fin) g.chainRow[parts[k].chain] = w;
             }
         }

@@ -147,6 +147,9 @@ struct Chain3Geom {
     int warpBase[kChain3MaxWarps];        // step offset of the part: its section k works on frame t - base - k at step t
     int warpSrc[kChain3MaxWarps];         // -1: the PCM tile; else the warp whose row feeds this part
     int warpFinal[kChain3MaxWarps];       // last part of its chain
+    // the program's coefficients put every section of the part in the unit-gain form (kernel_chain3.cu unitStep: 2 MACs per section
+    // instead of 5).  Placement and the trace use it; the warp itself decides from the words it loads (a per-stream table may differ)
+    int warpUnit[kChain3MaxWarps];
     int warpRowOff[kChain3MaxWarps];      // byte offset of the warp's rows [stream][pitch] in shared memory
     int warpPitch[kChain3MaxWarps];       // words per row: R + 1 (final parts: the post ring) or 3 tiles + 1 (hand-over rows)
     int warpRole[32];                     // hardware warp id -> cascade warp index (>= 0), -1 dither warp, -2-k store warp k

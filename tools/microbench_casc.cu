@@ -3,6 +3,8 @@
 // chain of a warp is only known at run time -- but see MODE 2: with a block-uniform address ptxas keeps them in UNIFORM registers);
 // MODE 2: 5*CH coefficient VECTOR registers (lane-dependent address), k_chain3's real situation; MODE 1: constant-bank operands with compile-time offsets (c[bank][imm]
 // operands: two register sources per IMAD.WIDE instead of three).  W warps per sub-partition, one CTA per SM.
+// MODE 3: the unit-gain form of kernel_chain3.cu (unitStep: z += a1 d1 + a2 d2, y = x + (z >> 28), two sticky records), vector-register
+// coefficients as in MODE 2.  Rates count 5 MACs per section in every mode, so cycles per MAC compare the cost of a section.
 #include <cstdio>
 #include <cuda_runtime.h>
 
@@ -28,12 +30,34 @@ __global__ void __launch_bounds__(512) k(long long* out, const int* __restrict__
         const int* cf = coefG + 5 * c + (MODE == 2 ? (int)(threadIdx.x & 1) : (int)(blockIdx.x & 1));
         b0[c] = cf[0]; b1[c] = cf[1]; b2[c] = cf[2]; a1[c] = cf[3]; a2[c] = cf[4];
     }
-    unsigned w0 = 0, w1 = 0;
+    unsigned w0 = 0, w1 = 0, wx = 0;
     int xin = threadIdx.x * 77;
+    long long z[CH]; int d1[CH], d2[CH];
+#pragma unroll
+    for (int c = 0; c < CH; c++) { z[c] = acc[c]; d1[c] = c; d2[c] = c + 1; }
     for (int i = 0; i < iters; i++) {
 #pragma unroll
         for (int u = 0; u < 4; u++) {
             long long a[CH];
+            if (MODE == 3) {
+#pragma unroll
+                for (int c = 0; c < CH; c++) a[c] = mac32(z[c], d1[c], a1[c]);
+#pragma unroll
+                for (int c = 0; c < CH; c++) a[c] = mac32(a[c], d2[c], a2[c]);
+                int y[CH];
+#pragma unroll
+                for (int c = 0; c < CH; c++) {
+                    const int s = q59(a[c]);
+                    if (c & 1) w1 = max(w1, (unsigned)hi32(a[c]) + 0x100000u); else w0 = max(w0, (unsigned)hi32(a[c]) + 0x100000u);
+                    y[c] = (c ? y1[c - 1] : xin) + s;
+                    z[c] = a[c]; d2[c] = d1[c]; d1[c] = s;
+                }
+                wx = max(wx, (unsigned)xin + 0x78000000u);
+#pragma unroll
+                for (int c = 0; c < CH; c++) { y3[c] = y2[c]; y2[c] = y1[c]; y1[c] = y[c]; }
+                X2 = X1; X1 = xin; xin = xin * 5 + 1;
+                continue;
+            }
             if (MODE == 0 || MODE == 2) {
 #pragma unroll
                 for (int c = 0; c < CH; c++) a[c] = mac32(acc[c], c ? y2[c - 1] : X1, b1[c]);
@@ -65,9 +89,9 @@ __global__ void __launch_bounds__(512) k(long long* out, const int* __restrict__
             X2 = X1; X1 = xin; xin = xin * 5 + 1;
         }
     }
-    long long s = w0 ^ w1;
+    long long s = w0 ^ w1 ^ wx;
 #pragma unroll
-    for (int c = 0; c < CH; c++) s ^= acc[c] + y1[c] + y3[c];
+    for (int c = 0; c < CH; c++) s ^= acc[c] + z[c] + y1[c] + y3[c];
     if (s == 0x123456789abcdefll) out[0] = s;
 }
 
@@ -87,14 +111,18 @@ template <int CH, int MODE> void run(int W, int iters, const int* dCoef) {
     int clk; cudaDeviceGetAttribute(&clk, cudaDevAttrClockRate, dev);
     const double perClkSM = best / (p.multiProcessorCount * (double)clk * 1e3);
     printf("{\"sections\": %d, \"coefficients\": \"%s\", \"warps_per_subpartition\": %d, \"T_mac_per_s\": %.3f, \"mac_per_clk_per_SM\": %.2f, "
-           "\"cycles_per_warp_mac_per_subpartition\": %.2f}\n", CH, MODE == 1 ? "constant bank" : MODE == 2 ? "vector registers" : "uniform registers", W, best / 1e12, perClkSM, 128.0 / perClkSM);
+           "\"cycles_per_warp_mac_per_subpartition\": %.2f}\n", CH, MODE == 1 ? "constant bank" : MODE == 2 ? "vector registers" : MODE == 3 ? "vector registers, unit-gain form" : "uniform registers", W, best / 1e12, perClkSM, 128.0 / perClkSM);
     cudaFree(d);
 }
 
-int main() {
+int main(int argc, char**) {
     int h[48]; for (int i = 0; i < 48; i++) h[i] = 0x0123457 * (i + 3);
     int* dCoef; cudaMalloc(&dCoef, sizeof h); cudaMemcpy(dCoef, h, sizeof h, cudaMemcpyHostToDevice);
     cudaMemcpyToSymbol(cCoef, h, 40 * sizeof(int));
+    if (argc > 1) {          // "unitgain": the general and the unit-gain part side by side, parts of 3 and 4 sections
+        for (int W : {2, 3}) { run<4, 2>(W, 2048, dCoef); run<4, 3>(W, 2048, dCoef); run<3, 2>(W, 2048, dCoef); run<3, 3>(W, 2048, dCoef); }
+        return 0;
+    }
     for (int W : {1, 2, 3, 4}) run<8, 0>(W, 2048, dCoef);
     for (int W : {1, 2, 3, 4}) run<8, 1>(W, 2048, dCoef);
     for (int W : {1, 2, 3, 4}) run<4, 0>(W, 2048, dCoef);
