@@ -216,6 +216,7 @@ static void planGeometries(Plans& p, int nStreams, int numSMs, std::vector<Chain
             }
         }
         p.trace += "\n";
+        p.trace += chain3PlacementTrace(L.chain, p.geom3);
     }
     if (p.dagUsable) {
         snprintf(line, sizeof line, "DAG kernel geometry: %d nodes (depth %d, longest cascade %d sections), %d streams/CTA, %d threads, tiles of %d frames, input rows of %d frames, %d words/stream, %zu B smem%s\n",

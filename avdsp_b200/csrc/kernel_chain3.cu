@@ -21,7 +21,7 @@
 //     IMAD.WIDE every ~6.7 cycles at best, two per sub-partition reach 4.8, three or more ~4.5 (tools/microbench_warps.cu),
 //     and a warp that finishes its tile early leaves its neighbour alone with the pipe -- so long cascades are cut into
 //     parts of <= 4 sections that run as separate warps (C2: 14 warps of 3 or 4 sections, placed on the sub-partitions
-//     by issue cost, planChain3Geometry).  A part hands its output to the next part through a shared-memory row (three
+//     by price per frame, placeChain3Warps).  A part hands its output to the next part through a shared-memory row (three
 //     tiles deep), one tile later (the consumer part runs F + lag frames behind and waits on a per-part tile counter),
 //     so parts never synchronise inside a tile;
 //   * the lane reads its input sample straight from the staged PCM tile (cp.async.bulk + mbarrier, issued two tiles
@@ -44,6 +44,7 @@
 #include "avdsp_dev.cuh"
 #include "kernels.h"
 #include <algorithm>
+#include <climits>
 #include <cstdlib>
 
 namespace avdsp {
@@ -1040,6 +1041,134 @@ bool chain3Supports(const ChainPlan& plan) {
     return true;
 }
 
+// What one warp costs per frame on its sub-partition: IMAD.WIDE on the MAC pipe (the planned form, and the general form a CTA
+// falls back to when a per-stream coefficient row breaks the unit-gain identity), and the rest in issue cycles beside them.
+// Item k < nCascade is cascade warp k; then the dither warp, then the store warps.  A section issues a shift and a saturation
+// record beside its MACs (unit-gain form: one add more), a part 4 instructions of bookkeeping.  The TPDF finish, the source
+// gain and the helper warps are priced from tools/chain3_placement_sweep.py (profiles/r7_chain3_placement_sweep.jsonl): on
+// the tile barrier's critical path they cost more than their instruction counts, and these prices rank the timed C2, C3 and
+// C3-float placements (Spearman 0.92-0.98 against the measured times).
+struct Chain3Price { int macs, other, macsGeneral, otherGeneral; };
+
+static Chain3Price chain3Price(const ChainPlan& plan, const Chain3Geom& g, int k) {
+    if (k == g.nCascade) return {0, 20, 0, 20};
+    if (k > g.nCascade) {                                    // 4 cycles per 32 output words, shared by the store warps
+        const int words = plan.h.nOut * g.streamsPerCta;
+        const int o = (4 * words + 16 * g.nStore) / (32 * g.nStore);
+        return {0, o, 0, o};
+    }
+    const ChainDesc& d = plan.chains[g.warpChain[k]];
+    const int n = g.warpNsec[k];
+    int extra = 4;
+    if (g.warpFinal[k] && (d.satKind & 1)) extra += 30;
+    if (g.warpSrc[k] < 0 && !(d.srcKind == SRC_LOAD_GAIN && d.srcArg == (1 << kMant))) extra += 24;
+    return {(g.warpUnit[k] ? 2 : 5) * n, (g.warpUnit[k] ? 3 : 2) * n + extra, 5 * n, 2 * n + extra};
+}
+
+// Price of a sub-partition per frame in issue cycles: the MAC pipe takes about 4 cycles per IMAD.WIDE (tools/microbench_warps.cu:
+// 4.05 at best), the other instructions are added on top (they share the issue slots and the tile barrier waits for all of them)
+static int chain3BinCost(int macs, int other) { return 4 * macs + other; }
+
+std::string chain3PlacementTrace(const ChainPlan& plan, const Chain3Geom& g) {
+    const int total = g.threads / 32;
+    int itemOf[32];                                          // hardware warp id -> item
+    for (int id = 0; id < total; id++) itemOf[id] = g.warpRole[id] >= 0 ? g.warpRole[id] : g.nCascade - 1 - g.warpRole[id];
+    int bin[32];
+    for (int id = 0; id < total; id++) bin[itemOf[id]] = id & 3;
+    std::string s = "chain kernel v3 placement: items (cascade warps, sections + u = unit-gain form + T = TPDF finish + g = "
+                    "source gain; d = dither warp, s = store warp) : IMAD.WIDE + other issue per frame:";
+    char b[64];
+    int macs[4] = {0, 0, 0, 0}, gen[4] = {0, 0, 0, 0}, other[4] = {0, 0, 0, 0};
+    for (int k = 0; k < total; k++) {
+        const Chain3Price p = chain3Price(plan, g, k);
+        if (k < g.nCascade) {
+            const ChainDesc& d = plan.chains[g.warpChain[k]];
+            snprintf(b, sizeof b, " %d%s%s%s:%d+%d", g.warpNsec[k], g.warpUnit[k] ? "u" : "", g.warpFinal[k] && (d.satKind & 1) ? "T" : "",
+                     g.warpSrc[k] < 0 && !(d.srcKind == SRC_LOAD_GAIN && d.srcArg == (1 << kMant)) ? "g" : "", p.macs, p.other);
+        } else snprintf(b, sizeof b, " %s:%d+%d", k == g.nCascade ? "d" : "s", p.macs, p.other);
+        s += b;
+        macs[bin[k]] += p.macs; gen[bin[k]] += p.macsGeneral; other[bin[k]] += p.other;
+    }
+    s += "; sub-partition of each item ";
+    for (int k = 0; k < total; k++) { snprintf(b, sizeof b, "%s%d", k ? "," : "", bin[k]); s += b; }
+    snprintf(b, sizeof b, "; IMAD.WIDE per frame on sub-partitions 0-3: %d %d %d %d", macs[0], macs[1], macs[2], macs[3]);
+    s += b;
+    snprintf(b, sizeof b, ", every part general: %d %d %d %d", gen[0], gen[1], gen[2], gen[3]);
+    s += b;
+    snprintf(b, sizeof b, "; model cost (issue cycles per frame): %d %d %d %d\n", chain3BinCost(macs[0], other[0]), chain3BinCost(macs[1], other[1]),
+             chain3BinCost(macs[2], other[2]), chain3BinCost(macs[3], other[3]));
+    return s + b;
+}
+
+// Exact placement search.  Items with equal prices are one class; a bin is a count vector over the classes, and bins of
+// equal size are filled in non-increasing order of their vectors, so every placement distinct up to interchangeable items and
+// sub-partition relabelling is visited once (C2: 4229), pruned by the best placement so far.
+struct Chain3Search {
+    int nClass, nBin, slots[4];
+    int macs[32], other[32], gen[32], otherGen[32], avail[32];   // per class: prices (planned, general form), items left
+    int cur[4][32], best[4][32];                           // per bin: items of each class
+    bool general;                                          // price every part in its general form
+    int genBound;                                          // largest all-general bin cost a placement may have
+    long long bestKey[2];                                  // largest bin cost, then the sum of squared bin costs
+
+    int binCost(int q, bool gen_) const {
+        int m = 0, o = 0;
+        for (int c = 0; c < nClass; c++) { m += cur[q][c] * (gen_ ? gen[c] : macs[c]); o += cur[q][c] * (gen_ ? otherGen[c] : other[c]); }
+        return chain3BinCost(m, o);
+    }
+    void fill(int q, int c, int room, long long maxCost, long long sumSq) {
+        if (c == nClass) {
+            if (room) return;
+            if (q > 0 && slots[q] == slots[q - 1] &&
+                std::lexicographical_compare(cur[q - 1], cur[q - 1] + nClass, cur[q], cur[q] + nClass)) return;
+            if (binCost(q, true) > genBound) return;
+            const long long cost = binCost(q, general);
+            const long long k0 = std::max(maxCost, cost), k1 = sumSq + cost * cost;
+            if (k0 > bestKey[0] || (q == nBin - 1 && k0 == bestKey[0] && k1 >= bestKey[1])) return;
+            if (q == nBin - 1) {
+                bestKey[0] = k0; bestKey[1] = k1;
+                std::copy(&cur[0][0], &cur[0][0] + 4 * 32, &best[0][0]);
+            } else fill(q + 1, 0, slots[q + 1], k0, k1);
+            return;
+        }
+        for (int n = std::min(avail[c], room); n >= 0; n--) {
+            cur[q][c] = n; avail[c] -= n;
+            fill(q, c + 1, room - n, maxCost, sumSq);
+            avail[c] += n; cur[q][c] = 0;
+        }
+    }
+    long long run(bool general_, int genBound_) {
+        general = general_; genBound = genBound_;
+        bestKey[0] = bestKey[1] = LLONG_MAX;
+        fill(0, 0, slots[0], 0, 0);
+        return bestKey[0];
+    }
+};
+
+// warps -> sub-partitions (hardware warp id % 4, tools/microbench_smsp.cu).  Item k is cascade warp k, then the dither warp,
+// then the store warps; itemBin[k] = its sub-partition.  The placement minimises the largest sub-partition price in the
+// planned forms, among the placements whose largest all-general price is the least any placement
+// reaches: a CTA that a per-stream coefficient row sends back to the general form runs on the best all-general placement the
+// prices know (C2: 55 55 65 65 IMAD.WIDE, no more than before the unit-gain form).
+static void placeChain3Warps(const ChainPlan& plan, const Chain3Geom& g, int total, int* itemBin) {
+    Chain3Search s{};
+    s.nBin = std::min(total, 4);
+    for (int q = 0; q < s.nBin; q++) s.slots[q] = (total - q + 3) / 4;
+    int cls[32];
+    for (int k = 0; k < total; k++) {
+        const Chain3Price p = chain3Price(plan, g, k);
+        int c = 0;
+        while (c < s.nClass && !(s.macs[c] == p.macs && s.other[c] == p.other && s.gen[c] == p.macsGeneral && s.otherGen[c] == p.otherGeneral)) c++;
+        if (c == s.nClass) { s.macs[c] = p.macs; s.other[c] = p.other; s.gen[c] = p.macsGeneral; s.otherGen[c] = p.otherGeneral; s.nClass++; }
+        s.avail[c]++;
+        cls[k] = c;
+    }
+    s.run(false, (int)s.run(true, INT_MAX));
+    for (int k = 0; k < total; k++)
+        for (int q = 0; q < s.nBin; q++)
+            if (s.best[q][cls[k]] > 0) { s.best[q][cls[k]]--; itemBin[k] = q; break; }
+}
+
 bool planChain3Geometry(const ChainPlan& plan, int nStreams, int numSMs, Chain3Geom* geom) {
     if (!chain3Supports(plan)) return false;
     const int C = plan.h.nChains;
@@ -1109,7 +1238,15 @@ bool planChain3Geometry(const ChainPlan& plan, int nStreams, int numSMs, Chain3G
         // warps count too); longest-processing-time first, then pairwise swaps while they flatten the four sums.  C2 ends up
         // as (4T,4,3,helper) x 2 + (4,3,3,3) x 2: 8.66 ms per step against 9.08 with equal section counts per sub-partition
         // (both TPDF parts on one of them) -- the heaviest single warp sets the pace of its sub-partition.
+        // Programs with unit-gain parts (C2) are placed by the exact search on measured prices instead (placeChain3Warps):
+        // that search picks slower placements for C3 and C3-float (profiles/r7_chain3_ab.jsonl).
         // Cascade warp index w (rows, tables) is independent of the hardware warp id.
+        for (int w = 0; w < nParts; w++) {
+            g.warpChain[w] = parts[w].chain; g.warpFirstSec[w] = parts[w].first; g.warpNsec[w] = parts[w].nsec;
+            g.warpBase[w] = parts[w].base; g.warpSrc[w] = parts[w].src; g.warpFinal[w] = parts[w].fin;
+            g.warpUnit[w] = parts[w].unit;
+            if (parts[w].fin) g.chainRow[parts[w].chain] = w;
+        }
         {
             const int total = nParts + 1 + g.nStore;
             int slots[4];
@@ -1119,7 +1256,7 @@ bool planChain3Geometry(const ChainPlan& plan, int nStreams, int numSMs, Chain3G
                 order[k] = k;
                 if (k >= nParts) { itemCost[k] = 8; continue; }              // helper warps: k == nParts dither, then store
                 const ChainDesc& d = plan.chains[parts[k].chain];
-                itemCost[k] = (parts[k].unit ? 4 : 5) * parts[k].nsec + 2;
+                itemCost[k] = 5 * parts[k].nsec + 2;
                 if (parts[k].fin && (d.satKind & 1)) itemCost[k] += 6;
                 if (parts[k].src < 0 && !(d.srcKind == SRC_LOAD_GAIN && d.srcArg == (1 << kMant))) itemCost[k] += 2;
             }
@@ -1146,6 +1283,9 @@ bool planChain3Geometry(const ChainPlan& plan, int nStreams, int numSMs, Chain3G
                 binCost[qa] -= dlt; binCost[qb] += dlt;
                 itemBin[ba] = qb; itemBin[bb] = qa;
             }
+            bool anyUnit = false;
+            for (int k = 0; k < nParts; k++) anyUnit |= parts[k].unit != 0;
+            if (anyUnit) placeChain3Warps(plan, g, total, itemBin);
             if (const char* ov = getenv("AVDSP_B200_BINS3")) {          // experiments: "b0,b1,..." = sub-partition of item k (parts, dither, stores)
                 int k = 0;
                 for (const char* q = ov; *q && k < total; q++) if (*q >= '0' && *q <= '3') itemBin[k++] = *q - '0';
@@ -1155,18 +1295,10 @@ bool planChain3Geometry(const ChainPlan& plan, int nStreams, int numSMs, Chain3G
             }
             int next[4] = {0, 0, 0, 0};
             for (int k = 0; k < 32; k++) g.warpRole[k] = -1;
-            int slotOf[kChain3MaxWarps];
             // cascade index = part index k (rows follow the part order); hardware warp id = bin + 4 * position in the bin
             for (int k = 0; k < total; k++) {
                 const int id = itemBin[k] + 4 * next[itemBin[k]]++;
-                if (k < nParts) { slotOf[k] = k; g.warpRole[id] = k; } else g.warpRole[id] = -1 - (k - nParts);
-            }
-            for (int k = 0; k < nParts; k++) {
-                const int w = slotOf[k];
-                g.warpChain[w] = parts[k].chain; g.warpFirstSec[w] = parts[k].first; g.warpNsec[w] = parts[k].nsec;
-                g.warpBase[w] = parts[k].base; g.warpSrc[w] = parts[k].src >= 0 ? slotOf[parts[k].src] : -1; g.warpFinal[w] = parts[k].fin;
-                g.warpUnit[w] = parts[k].unit;
-                if (parts[k].fin) g.chainRow[parts[k].chain] = w;
+                if (k < nParts) g.warpRole[id] = k; else g.warpRole[id] = -1 - (k - nParts);
             }
         }
         size_t bytes = 0;

@@ -142,7 +142,7 @@ struct Chain3Geom {
     int postOff, tpdfOff, ckOff, doneOff, mbarOff, rawOff;   // shared-memory map (bytes)
     int tma;               // filled per launch: the caller's input buffer allows bulk copies (else plain staged copies)
     int floatFast;         // float class: the source may use the hardware convert + mul.rz.ftz (gains checked on the host)
-    // cascade warp -> what it runs (dealt so that the four sub-partitions carry equal section counts)
+    // cascade warp -> what it runs (placed on the sub-partitions through warpRole, kernel_chain3.cu placeChain3Warps)
     int warpChain[kChain3MaxWarps], warpFirstSec[kChain3MaxWarps], warpNsec[kChain3MaxWarps];
     int warpBase[kChain3MaxWarps];        // step offset of the part: its section k works on frame t - base - k at step t
     int warpSrc[kChain3MaxWarps];         // -1: the PCM tile; else the warp whose row feeds this part
@@ -159,6 +159,7 @@ struct Chain3Geom {
 };
 bool chain3Supports(const ChainPlan& plan);
 bool planChain3Geometry(const ChainPlan& plan, int nStreams, int numSMs, Chain3Geom* geom);
+std::string chain3PlacementTrace(const ChainPlan& plan, const Chain3Geom& geom);   // the trace line of the warp placement
 cudaError_t launchChain3(const ChainPlan& plan, const Chain3Geom& geom, const Chain2Args& args, cudaStream_t stream);
 
 // ---- time-parallel mixer / delay / dither kernel (kernel_mix.cu) -----------------------------------
